@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: streamed audio-seconds per second of the 2-layer GRU-128 KWS path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2], the configuration the metric is quoted on): streaming serve of
 S = 131,072 concurrent streams PER GPU with carried GRU state and VAD reset, 300 ms chunks of
@@ -83,7 +83,15 @@ def parse_args():
     ap.add_argument("--no-bind", action="store_true", help="do not pin the rank to its GPU's NUMA-local cores")
     ap.add_argument("--cpu-streams", type=int, default=0, help="CPU sample: streams (default 64 per host core)")
     ap.add_argument("--cpu-chunks", type=int, default=0, help="CPU sample: chunks per step (default: calibrated)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (rank 0) as DIR/<name>.npy, "
+                         "float32 / float64, at most 64 MB: streaming = the trigger flags of every stream and, for a fixed "
+                         "seeded sample of streams, the carried GRU state and the window labels; attention = the softmax "
+                         "of a fixed seeded sample of utterances (all of them up to 4096)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference has none")
+    return args
 
 
 # ----------------------------------------------------------------------------- CPU port (oracle)
@@ -271,6 +279,42 @@ def timed_loop(torch, fn, steps, stream, barrier):
     barrier()
     per_step = [ev[i].elapsed_time(ev[i + 1]) for i in range(steps)]
     return ev[0].elapsed_time(ev[steps]), per_step
+
+
+# ----------------------------------------------------------------------------- --dump-outputs
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE_STREAMS = 8192        # state 8 MB + labels 2 MB; the trigger flags of 6.9 M streams (the HBM limit) add 28 MB
+DUMP_SAMPLE_UTTERANCES = 4096     # softmax [4096, 400, 6] fp32 = 39 MB
+
+
+def dump_sample(n, limit, seed=2024):
+    """Sorted indices of a fixed, seeded sample of min(n, limit) out of n items (all of them when n <= limit)."""
+    import numpy as np
+    if n <= limit:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, limit, replace=False))
+
+
+def stream_outputs(torch, det, trig):
+    """What the last kws_stream_step left for its caller: the trigger flags of every stream and, for a fixed seeded
+    sample of streams, the carried GRU state and the labels of the decode window (max 64 entries, -1 padded)."""
+    import numpy as np
+    sample = dump_sample(det.n_streams, DUMP_SAMPLE_STREAMS)
+    idx = torch.from_numpy(sample).to(trig.device)
+    labels, counts = det.window_labels(max_labels=64)
+    return dict(triggers=trig.cpu().numpy().astype(np.float32), sample_streams=sample.astype(np.float64),
+                state=det.state()[:, idx].cpu().numpy(), window_labels=labels[sample].astype(np.float32),
+                window_label_counts=counts[sample].astype(np.float32))
+
+
+def write_outputs(out_dir, arrays):
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def boosted_weights(cfg, gain, seed=1234):
@@ -588,6 +632,8 @@ def run_ours(args, rank, world, local_rank):
         trig_total.add_(trig.sum())                  # result consumption on the device (no host sync)
 
     total_ms, per_step = timed_loop(torch, step_counted, args.steps, stream, barrier)
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, stream_outputs(torch, det, trig))
     total_ms_max = sharding.reduce_max_scalar(total_ms, device)
     ms_per_step = total_ms_max / args.steps
     value = world * S * AUDIO_S_PER_CHUNK * args.steps / (total_ms_max * 1e-3)
@@ -820,6 +866,10 @@ def run_attention(args, rank, world, local_rank):
     if rank == 0:
         sampler.start()
     total_ms, _ = timed_loop(torch, step_dev, args.steps, stream, barrier)
+    if args.dump_outputs and rank == 0:
+        sample = dump_sample(B, DUMP_SAMPLE_UTTERANCES)
+        write_outputs(args.dump_outputs, dict(softmax=out[0][torch.from_numpy(sample).to(device)].cpu().numpy(),
+                                              sample_utterances=sample.astype("float64")))
     total_ms = sharding.reduce_max_scalar(total_ms, device)
     for i in range(2):
         step_e2e(i)
