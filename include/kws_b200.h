@@ -357,9 +357,11 @@ typedef struct kws_attention_weights {
 int kws_attention_create(const kws_attention_config* cfg, const kws_attention_weights* host_weights, int device,
                          kws_attention** out);
 int kws_attention_destroy(kws_attention* m);
-/* T' = T / combine_frame + 1 (models/attention_ctc.py:88-90). */
+/* T' = T / combine_frame + 1 for combine_frame > 1 (models/attention_ctc.py:88-90), T' = T for combine_frame == 1. */
 int32_t kws_attention_frames(const kws_attention* m, int32_t T);
-/* mel [B, T, n_mel] (DEVICE, e.g. from kws_frontend_mel) -> probs_out [B, T', C]; logits_out may be NULL. */
+/* mel [B, T, n_mel] (DEVICE, e.g. from kws_frontend_mel) -> probs_out [B, T', C]; logits_out may be NULL.
+ * Precondition: |mel| and every activation stay below 65520, the largest value the fp16 `hi` part of the tensor-core
+ * operand splits holds; larger values give inf / NaN.  Front-end mel output stays far below that.              */
 int kws_attention_forward(kws_attention* m, const float* mel, int64_t B, int32_t T, float* probs_out,
                           float* logits_out, void* stream);
 
@@ -370,6 +372,20 @@ int kws_attention_forward(kws_attention* m, const float* mel, int64_t B, int32_t
  * Synchronises `stream`.                                                                       */
 int kws_debug_tc_gemm(const float* A, const float* B_host, float* D, int N, int K, int ss_mode,
                       void* stream);
+
+/* Debug / test: the kernels of kws_attention_forward one at a time, on caller DEVICE buffers (W_host is HOST).  Each
+ * call synchronises `stream` and returns KWS_ERR_UNSUPPORTED for a shape the chosen kernel does not take.
+ *   att_linear:  Y [rows, N] = act(A [rows, K] W [K, N] + bias [N]) (+ pe [r % Tp, N] when add_pe), act = relu or none;
+ *                path 0 = tcgen05 (N % 128 == 0, K % 4 == 0; W packed for this call), 1 = the fp32 FFMA kernel.
+ *   att_core:    qkv [B, Tp, 3 * 16 * heads] (q | k | v, head-major inside each) -> out [B, Tp, 16 * heads],
+ *                softmax(q k^T / 4) v per (utterance, head); path 0 = tcgen05 (Tp <= 400), 1 = the FFMA kernel.
+ *   att_add_layernorm:  y = layer_norm(a + b) over each utterance's [Tp, N], per-channel gamma / beta (N % 4 == 0);
+ *                in_smem = 1 keeps a + b in shared memory (Tp * N <= 51,200), 0 reads a and b three times.       */
+int kws_debug_att_linear(const float* A, const float* W_host, const float* bias, const float* pe, int32_t Tp,
+                         int64_t rows, int32_t K, int32_t N, int relu, int add_pe, int path, float* Y, void* stream);
+int kws_debug_att_core(const float* qkv, int64_t B, int32_t Tp, int32_t heads, int path, float* out, void* stream);
+int kws_debug_att_add_layernorm(const float* a, const float* b, const float* gamma, const float* beta, int64_t B,
+                                int32_t Tp, int32_t N, int in_smem, float* y, void* stream);
 
 /* Debug: enable/disable and read the phase timeline (SM clock ticks) of the first tile of CTA 0 of the last
  * tensor-core GRU launch; see csrc/gru_tc.cu.  host_out may be NULL (only set the switch).               */

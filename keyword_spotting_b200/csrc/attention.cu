@@ -34,8 +34,8 @@ struct kws_attention {
   } p_in, p_qkv[8], p_ff1[8], p_ff2[8];
   float* pe = nullptr;          // [pe_rows, N] from the K6 kernel
   int pe_rows = 0;
-  float* scratch = nullptr;     // xin | x | y | att | big
-  size_t scratch_rows = 0;
+  float* scratch = nullptr;     // xin | x | y | att | big, each segment padded to 32 floats
+  size_t scratch_floats = 0;
 };
 
 namespace kws {
@@ -316,6 +316,15 @@ static int att_linear(const float* A, const float* W, const kws_attention::Packe
   return KWS_OK;
 }
 
+static int att_core_ffma(const float* qkv, long B, int Tp, int heads, float* out, cudaStream_t st) {
+  dim3 ga(static_cast<unsigned>(ceil_div(Tp, 128)), static_cast<unsigned>(heads), static_cast<unsigned>(B));
+  att_attention_kernel<<<ga, 128, 0, st>>>(qkv, Tp, heads, out);
+  KWS_LAUNCH_OK("att_attention_kernel");
+  return KWS_OK;
+}
+
+constexpr int kLnSmemBytes = 200 * 1024;       // the layer norm keeps a + b in shared memory up to this size
+
 }  // namespace kws
 
 using namespace kws;
@@ -415,27 +424,30 @@ extern "C" int kws_attention_forward(kws_attention* m, const float* mel, int64_t
     const int rc = kws_positional_encoding(Tp, N, m->pe, stream);
     if (rc != KWS_OK) return rc;
   }
-  const size_t per_row = static_cast<size_t>(Kin) + 3 * N + (F > 3 * N ? F : 3 * N);
-  if (static_cast<size_t>(rows) > m->scratch_rows) {
+  // every segment starts on a 128-byte boundary: the tensor-core dense layers and the layer norm move 16-byte pieces,
+  // and rows * Kin is odd for some accepted configs (n_mel = 41, combine_frame = 3 and an odd B * T')
+  const auto seg = [rows](int width) { return (static_cast<size_t>(rows) * width + 31) & ~static_cast<size_t>(31); };
+  const size_t scratch_floats = seg(Kin) + 3 * seg(N) + seg(F > 3 * N ? F : 3 * N);
+  if (scratch_floats > m->scratch_floats) {
     KWS_CUDA_OK(cudaDeviceSynchronize());
     cudaFree(m->scratch);
     m->scratch = nullptr;
-    m->scratch_rows = 0;
-    cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&m->scratch), sizeof(float) * per_row * rows);
+    m->scratch_floats = 0;
+    cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&m->scratch), sizeof(float) * scratch_floats);
     if (e != cudaSuccess) return fail(KWS_ERR_ALLOC, "scratch for %ld rows failed: %s", rows, cudaGetErrorString(e));
-    m->scratch_rows = rows;
+    m->scratch_floats = scratch_floats;
   }
   float* xin = m->scratch;
-  float* x = xin + static_cast<size_t>(rows) * Kin;
-  float* y = x + static_cast<size_t>(rows) * N;
-  float* att = y + static_cast<size_t>(rows) * N;
-  float* big = att + static_cast<size_t>(rows) * N;
+  float* x = xin + seg(Kin);
+  float* y = x + seg(N);
+  float* att = y + seg(N);
+  float* big = att + seg(N);
 
   // layer norm: the utterance's T' * N floats in shared memory when they fit
   const size_t ln_bytes = sizeof(float) * static_cast<size_t>(Tp) * N;
-  const int ln_in_smem = ln_bytes <= 200 * 1024 ? 1 : 0;
+  const int ln_in_smem = ln_bytes <= kLnSmemBytes ? 1 : 0;
   const size_t ln_smem = ln_in_smem ? ln_bytes : 0;
-  KWS_CUDA_OK(cudaFuncSetAttribute(att_add_layernorm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  KWS_CUDA_OK(cudaFuncSetAttribute(att_add_layernorm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnSmemBytes));
   const long total_in = rows * Kin;
   att_combine_kernel<<<static_cast<unsigned>(ceil_div(total_in, 256)), 256, 0, st>>>(mel, B, T, c.n_mel, c.combine_frame, Tp, xin);
   KWS_LAUNCH_OK("att_combine_kernel");
@@ -448,9 +460,8 @@ extern "C" int kws_attention_forward(kws_attention* m, const float* mel, int64_t
       rc = launch_att_core_tc(big, B, Tp, c.heads, att, st);
       if (rc != KWS_OK) break;
     } else {
-      dim3 ga(static_cast<unsigned>(ceil_div(Tp, 128)), static_cast<unsigned>(c.heads), static_cast<unsigned>(B));
-      att_attention_kernel<<<ga, 128, 0, st>>>(big, Tp, c.heads, att);
-      KWS_LAUNCH_OK("att_attention_kernel");
+      rc = att_core_ffma(big, B, Tp, c.heads, att, st);
+      if (rc != KWS_OK) break;
     }
     att_add_layernorm_kernel<<<static_cast<unsigned>(B), 1024, ln_smem, st>>>(att, x, L.ln1_g, L.ln1_b, Tp, N, ln_in_smem, y);
     KWS_LAUNCH_OK("att_add_layernorm_kernel");
@@ -464,5 +475,68 @@ extern "C" int kws_attention_forward(kws_attention* m, const float* mel, int64_t
   att_output_kernel<<<static_cast<unsigned>(ceil_div(rows, 128)), 128, sizeof(float) * (N * C + C), st>>>(
       x, m->w_out, m->b_out, rows, N, C, c.use_relu, probs_out, logits_out);
   KWS_LAUNCH_OK("att_output_kernel");
+  return KWS_OK;
+}
+
+// ---- single kernels of the forward pass on caller buffers, for tests that hold each one against a float64 reference
+extern "C" int kws_debug_att_linear(const float* A, const float* W_host, const float* bias, const float* pe, int32_t Tp,
+                                    int64_t rows, int32_t K, int32_t N, int relu, int add_pe, int path, float* Y,
+                                    void* stream) {
+  clear_error();
+  KWS_REQUIRE(A && W_host && bias && Y && (pe || !add_pe), "NULL pointer");
+  KWS_REQUIRE(rows >= 1 && K >= 1 && N >= 1 && Tp >= 1, "bad sizes");
+  KWS_REQUIRE(path == 0 || path == 1, "path must be 0 (tcgen05) or 1 (FFMA)");
+  if (path == 0 && !att_linear_tc_supported(K, N))
+    return fail(KWS_ERR_UNSUPPORTED, "the tensor-core dense layer needs N %% 128 == 0 and K %% 4 == 0 (K = %d, N = %d)", K, N);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  kws_attention::Packed pk;
+  float* dW = nullptr;
+  int rc = path == 0 ? att_pack_linear(W_host, K, N, &pk.w, &pk.nchunks) : att_upload(&dW, W_host, static_cast<size_t>(K) * N);
+  if (rc == KWS_OK) {
+    if (relu) rc = add_pe ? att_linear<true, true>(A, dW, pk, bias, pe, Tp, rows, K, N, Y, st)
+                          : att_linear<true, false>(A, dW, pk, bias, pe, Tp, rows, K, N, Y, st);
+    else rc = add_pe ? att_linear<false, true>(A, dW, pk, bias, pe, Tp, rows, K, N, Y, st)
+                     : att_linear<false, false>(A, dW, pk, bias, pe, Tp, rows, K, N, Y, st);
+  }
+  const cudaError_t e = cudaStreamSynchronize(st);
+  cudaFree(pk.w);
+  cudaFree(dW);
+  if (rc != KWS_OK) return rc;
+  if (e != cudaSuccess) return fail(KWS_ERR_CUDA, "att_linear (path %d) failed: %s", path, cudaGetErrorString(e));
+  return KWS_OK;
+}
+
+extern "C" int kws_debug_att_core(const float* qkv, int64_t B, int32_t Tp, int32_t heads, int path, float* out,
+                                  void* stream) {
+  clear_error();
+  KWS_REQUIRE(qkv && out, "NULL pointer");
+  KWS_REQUIRE(B >= 1 && B <= 65535 && Tp >= 1 && heads >= 1 && heads <= 64, "bad sizes");
+  KWS_REQUIRE(path == 0 || path == 1, "path must be 0 (tcgen05) or 1 (FFMA)");
+  if (path == 0 && !att_core_tc_supported(Tp, heads, heads * kAttHeadDim))
+    return fail(KWS_ERR_UNSUPPORTED, "the tensor-core attention core takes 1 <= T' <= 400 (T' = %d)", Tp);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int rc = path == 0 ? launch_att_core_tc(qkv, B, Tp, heads, out, st) : att_core_ffma(qkv, B, Tp, heads, out, st);
+  const cudaError_t e = cudaStreamSynchronize(st);
+  if (rc != KWS_OK) return rc;
+  if (e != cudaSuccess) return fail(KWS_ERR_CUDA, "attention core (path %d) failed: %s", path, cudaGetErrorString(e));
+  return KWS_OK;
+}
+
+extern "C" int kws_debug_att_add_layernorm(const float* a, const float* b, const float* gamma, const float* beta,
+                                           int64_t B, int32_t Tp, int32_t N, int in_smem, float* y, void* stream) {
+  clear_error();
+  KWS_REQUIRE(a && b && gamma && beta && y, "NULL pointer");
+  KWS_REQUIRE(B >= 1 && B <= (1L << 31) - 1 && Tp >= 1 && N >= 1 && static_cast<int64_t>(Tp) * N < (1L << 31), "bad sizes");
+  if (N % 4 != 0) return fail(KWS_ERR_UNSUPPORTED, "the layer norm needs N %% 4 == 0 (N = %d)", N);
+  const size_t bytes = sizeof(float) * static_cast<size_t>(Tp) * N;
+  if (in_smem && bytes > kLnSmemBytes)
+    return fail(KWS_ERR_UNSUPPORTED, "T' * N = %d floats do not fit the layer norm's shared memory", Tp * N);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  KWS_CUDA_OK(cudaFuncSetAttribute(att_add_layernorm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnSmemBytes));
+  att_add_layernorm_kernel<<<static_cast<unsigned>(B), 1024, in_smem ? bytes : 0, st>>>(a, b, gamma, beta, Tp, N,
+                                                                                       in_smem ? 1 : 0, y);
+  KWS_LAUNCH_OK("att_add_layernorm_kernel");
+  const cudaError_t e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) return fail(KWS_ERR_CUDA, "att_add_layernorm_kernel failed: %s", cudaGetErrorString(e));
   return KWS_OK;
 }

@@ -39,9 +39,11 @@ class AttentionWeights:
     b_out: np.ndarray = None
 
 
-def init_weights(seed=4321, n_mel=60, mel_basis=None) -> AttentionWeights:
+def init_weights(seed=4321, n_mel=60, mel_basis=None, combine=COMBINE, layers=LAYERS, ffn=FFN,
+                 classes=CLASSES) -> AttentionWeights:
     """Random weights: glorot-uniform kernels (tf.layers.conv2d default) with small random biases and
-    non-trivial layer-norm parameters so that every term of the graph is exercised."""
+    non-trivial layer-norm parameters so that every term of the graph is exercised.  The defaults are the
+    shipped config; other values give the weights of any config kws_attention_create accepts."""
     from .model import slaney_mel_basis
     rng = np.random.default_rng(seed)
 
@@ -51,21 +53,21 @@ def init_weights(seed=4321, n_mel=60, mel_basis=None) -> AttentionWeights:
 
     w = AttentionWeights()
     w.mel_basis = (slaney_mel_basis(n_mels=n_mel).T if mel_basis is None else mel_basis).astype(np.float32)
-    w.w_in = glorot(COMBINE * n_mel, HIDDEN)
+    w.w_in = glorot(combine * n_mel, HIDDEN)
     w.b_in = (rng.standard_normal(HIDDEN) * 0.05).astype(np.float32)
-    for _ in range(LAYERS):
+    for _ in range(layers):
         w.w_qkv.append(glorot(HIDDEN, 3 * HIDDEN))
         w.b_qkv.append((rng.standard_normal(3 * HIDDEN) * 0.05).astype(np.float32))
         w.ln1_g.append((1 + 0.1 * rng.standard_normal(HIDDEN)).astype(np.float32))
         w.ln1_b.append((0.1 * rng.standard_normal(HIDDEN)).astype(np.float32))
-        w.w_ff1.append(glorot(HIDDEN, FFN))
-        w.b_ff1.append((rng.standard_normal(FFN) * 0.05).astype(np.float32))
-        w.w_ff2.append(glorot(FFN, HIDDEN))
+        w.w_ff1.append(glorot(HIDDEN, ffn))
+        w.b_ff1.append((rng.standard_normal(ffn) * 0.05).astype(np.float32))
+        w.w_ff2.append(glorot(ffn, HIDDEN))
         w.b_ff2.append((rng.standard_normal(HIDDEN) * 0.05).astype(np.float32))
         w.ln2_g.append((1 + 0.1 * rng.standard_normal(HIDDEN)).astype(np.float32))
         w.ln2_b.append((0.1 * rng.standard_normal(HIDDEN)).astype(np.float32))
-    w.w_out = glorot(HIDDEN, CLASSES)
-    w.b_out = (rng.standard_normal(CLASSES) * 0.05).astype(np.float32)
+    w.w_out = glorot(HIDDEN, classes)
+    w.b_out = (rng.standard_normal(classes) * 0.05).astype(np.float32)
     return w
 
 
@@ -102,10 +104,11 @@ def self_attention(x, w_qkv, b_qkv, heads=HEADS):
     return o.transpose(0, 2, 1, 3).reshape(B, T, N)
 
 
-def mel_forward(mel, w: AttentionWeights, dtype=np.float32, use_relu=True):
-    """inference() + softmax: mel [B, T, M] -> (softmax [B, T', C], logits)."""
+def mel_forward(mel, w: AttentionWeights, dtype=np.float32, use_relu=True, combine=COMBINE):
+    """inference() + softmax: mel [B, T, M] -> (softmax [B, T', C], logits).  Layers, FFN width and classes
+    follow the weights."""
     f = lambda a: np.asarray(a).astype(dtype)
-    x = combine_frames(f(mel))
+    x = combine_frames(f(mel), combine)
     x = x @ f(w.w_in) + f(w.b_in)                      # input_linear_trans (:92-95)
     Tp = x.shape[1]
     x = x + f(posenc.positional_encoding(Tp, HIDDEN))  # :96-98

@@ -334,3 +334,47 @@ def test_stream_oracle_decide_on_hook_only_changes_the_decision_window():
         fired += int(r["trigger"].sum())
         assert r["softmax"].max() > 0.1                              # the returned softmax stays the oracle's own
     assert fired == 0
+
+
+# ---------------------------------------------------------------- attention_ctc oracle (oracle/attention.py)
+_ATTENTION_DEFAULT_WEIGHTS_SHA256 = "5eb546514f69998ad00afa584478e85b367fbf16f5212b50f905e1e72032603d"
+
+
+def test_attention_oracle_defaults_are_the_shipped_config_unchanged():
+    """init_weights / mel_forward take the config as parameters; their defaults must keep giving the weights and outputs
+    that the shipped-config tests were written against.  The weights are pinned bit for bit (sha256 of every array, in
+    field order); the outputs of a fixed mel batch (default_rng(77), [2, 9, 60]) are pinned in float64 to 1e-12, which
+    only leaves room for a BLAS that orders its sums differently."""
+    import hashlib
+    from oracle import attention as oa
+    w = oa.init_weights()
+    h = hashlib.sha256()
+    for name in ("mel_basis", "w_in", "b_in", "w_qkv", "b_qkv", "ln1_g", "ln1_b", "w_ff1", "b_ff1", "w_ff2", "b_ff2",
+                 "ln2_g", "ln2_b", "w_out", "b_out"):
+        v = getattr(w, name)
+        for a in (v if isinstance(v, list) else [v]):
+            h.update(np.ascontiguousarray(a).tobytes())
+    assert h.hexdigest() == _ATTENTION_DEFAULT_WEIGHTS_SHA256
+    explicit = oa.init_weights(seed=4321, n_mel=60, combine=2, layers=3, ffn=512, classes=6)
+    for name in ("w_in", "w_qkv", "w_ff1", "w_ff2", "b_ff2", "w_out", "b_out"):
+        np.testing.assert_array_equal(np.asarray(getattr(w, name)), np.asarray(getattr(explicit, name)))
+    mel = np.abs(np.random.default_rng(77).standard_normal((2, 9, 60))).astype(np.float32)
+    g = golden("attention_oracle_golden.npz")
+    probs, logits = oa.mel_forward(mel, w, np.float64)
+    np.testing.assert_allclose(probs, g["probs"], rtol=1e-12, atol=0)
+    np.testing.assert_allclose(logits, g["logits"], rtol=1e-12, atol=1e-15)
+    p2, l2 = oa.mel_forward(mel, w, np.float64, use_relu=True, combine=2)
+    np.testing.assert_array_equal(p2, probs)
+    np.testing.assert_array_equal(l2, logits)
+
+
+def test_attention_oracle_other_configs_have_their_shapes():
+    from oracle import attention as oa
+    w = oa.init_weights(seed=1, n_mel=41, combine=3, layers=2, ffn=200, classes=16)
+    assert w.w_in.shape == (123, 128) and len(w.w_qkv) == 2 and w.w_ff1[1].shape == (128, 200)
+    assert w.w_out.shape == (128, 16) and w.mel_basis.shape == (201, 41)
+    mel = np.ones((2, 10, 41), np.float32)
+    probs, logits = oa.mel_forward(mel, w, np.float64, use_relu=False, combine=3)
+    assert probs.shape == logits.shape == (2, 10 // 3 + 1, 16)
+    assert (logits < 0).any()                                   # no relu on the output layer
+    np.testing.assert_allclose(probs.sum(-1), 1, rtol=1e-12)
