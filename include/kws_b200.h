@@ -320,7 +320,8 @@ int kws_positional_encoding(int32_t max_position, int32_t encoding_size, float* 
  * The attention_ctc deployment forward pass (models/attention_ctc.py:73-128, :215-274; BASELINE config 5), the
  * consumer of the positional_encoding op: combine_frame folding, input dense + positional encoding, num_layers x
  * {8-head self-attention over all T' positions, add + layer_norm over (T', N), relu FFN, add + layer_norm},
- * output dense (+relu) and softmax.  Utterances of one call have the same length (the graph has no padding mask). */
+ * output dense (+relu) and softmax.  The graph has no padding mask: kws_attention_forward takes utterances of one
+ * length, kws_attention_forward_lens utterances of different lengths, each computed as the graph computes it alone. */
 typedef struct kws_attention kws_attention;
 
 typedef struct kws_attention_config {
@@ -364,6 +365,12 @@ int32_t kws_attention_frames(const kws_attention* m, int32_t T);
  * operand splits holds; larger values give inf / NaN.  Front-end mel output stays far below that.              */
 int kws_attention_forward(kws_attention* m, const float* mel, int64_t B, int32_t T, float* probs_out,
                           float* logits_out, void* stream);
+/* Variable-length batch: utterance b has lens[b] valid mel frames (DEVICE int32 [B]) in the first rows of mel [B, T, n_mel];
+ * the rest of its rows is never read.  Rows 0 .. kws_attention_frames(lens[b]) - 1 of probs_out / logits_out [B, T', C]
+ * (T' = kws_attention_frames(T)) are bit-identical to kws_attention_forward on that utterance alone with T = lens[b];
+ * the remaining rows are zero.  lens values are clamped to [1, T].  lens == NULL: every utterance has T frames.   */
+int kws_attention_forward_lens(kws_attention* m, const float* mel, int64_t B, int32_t T, const int32_t* lens,
+                               float* probs_out, float* logits_out, void* stream);
 
 /* ----------------------------------------------------------------- self-test
  * One 128 x N x K tensor-core product through the tcgen05 conventions the recurrent kernel builds on
@@ -380,12 +387,19 @@ int kws_debug_tc_gemm(const float* A, const float* B_host, float* D, int N, int 
  *   att_core:    qkv [B, Tp, 3 * 16 * heads] (q | k | v, head-major inside each) -> out [B, Tp, 16 * heads],
  *                softmax(q k^T / 4) v per (utterance, head); path 0 = tcgen05 (Tp <= 400), 1 = the FFMA kernel.
  *   att_add_layernorm:  y = layer_norm(a + b) over each utterance's [Tp, N], per-channel gamma / beta (N % 4 == 0);
- *                in_smem = 1 keeps a + b in shared memory (Tp * N <= 51,200), 0 reads a and b three times.       */
+ *                in_smem = 1 keeps a + b in shared memory (Tp * N <= 51,200), 0 reads a and b three times.
+ *   The _lens forms take per-utterance row counts lens (DEVICE int32 [B], in T' units, clamped to [1, Tp]; NULL = Tp)
+ *   with rows still at stride Tp, as kws_attention_forward_lens runs them: utterance b uses its first lens[b] rows (and
+ *   keys) only, and rows at or past lens[b] of `out` / `y` are not written.                                       */
 int kws_debug_att_linear(const float* A, const float* W_host, const float* bias, const float* pe, int32_t Tp,
                          int64_t rows, int32_t K, int32_t N, int relu, int add_pe, int path, float* Y, void* stream);
 int kws_debug_att_core(const float* qkv, int64_t B, int32_t Tp, int32_t heads, int path, float* out, void* stream);
 int kws_debug_att_add_layernorm(const float* a, const float* b, const float* gamma, const float* beta, int64_t B,
                                 int32_t Tp, int32_t N, int in_smem, float* y, void* stream);
+int kws_debug_att_core_lens(const float* qkv, int64_t B, int32_t Tp, const int32_t* lens, int32_t heads, int path,
+                            float* out, void* stream);
+int kws_debug_att_add_layernorm_lens(const float* a, const float* b, const float* gamma, const float* beta, int64_t B,
+                                     int32_t Tp, const int32_t* lens, int32_t N, int in_smem, float* y, void* stream);
 
 /* Debug: enable/disable and read the phase timeline (SM clock ticks) of the first tile of CTA 0 of the last
  * tensor-core GRU launch; see csrc/gru_tc.cu.  host_out may be NULL (only set the switch).               */

@@ -133,12 +133,16 @@ _SIGNATURES = {
     "kws_attention_destroy": (c_int, [c_void_p]),
     "kws_attention_frames": (c_int32, [c_void_p, c_int32]),
     "kws_attention_forward": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p]),
+    "kws_attention_forward_lens": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]),
     "kws_debug_tc_gemm": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "kws_debug_att_linear": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int64, c_int32, c_int32, c_int,
                                      c_int, c_int, c_void_p, c_void_p]),
     "kws_debug_att_core": (c_int, [c_void_p, c_int64, c_int32, c_int32, c_int, c_void_p, c_void_p]),
+    "kws_debug_att_core_lens": (c_int, [c_void_p, c_int64, c_int32, c_void_p, c_int32, c_int, c_void_p, c_void_p]),
     "kws_debug_att_add_layernorm": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int,
                                             c_void_p, c_void_p]),
+    "kws_debug_att_add_layernorm_lens": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_int32,
+                                                 c_int, c_void_p, c_void_p]),
     "kws_debug_tc_timeline": (c_int, [c_int, c_void_p, c_int]),
     "kws_debug_step_timing": (c_int, [c_int, c_void_p, c_void_p]),
     "kws_debug_mel_quads": (c_int, [c_void_p, c_int, c_void_p, c_int]),

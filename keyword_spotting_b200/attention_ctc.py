@@ -3,7 +3,9 @@
 
 ``AttentionDeployModel.run(['model/softmax:0'], {'model/inputX:0': pcm})`` mirrors the reference's frozen-graph
 call; PCM goes through the same fused front end as the rnn_ctc model (K1, n_mel = 60) and then through
-``kws_attention_forward``.  Utterances of one call share a length (the reference graph has no padding mask).
+``kws_attention_forward_lens``.  The reference graph has no padding mask, so a batch of utterances of different
+lengths takes their lengths (``run_mel(..., lens=)``, ``forward(..., lengths=)``): each utterance is then computed
+exactly as the graph computes it alone, and its output rows past ``output_lengths(lens)`` are zero.
 """
 from __future__ import annotations
 
@@ -168,8 +170,38 @@ class AttentionDeployModel:
     def frames(self, T: int) -> int:
         return int(self._lib.kws_attention_frames(self._handle, int(T)))
 
-    def run_mel(self, mel, want_logits: bool = False):
-        """mel ``[B, T, n_mel]`` (or ``[T, n_mel]``) -> softmax ``[B, T', C]`` [, logits]."""
+    def output_lengths(self, lens):
+        """T'_b of utterances of ``lens`` valid mel frames, in the container type of ``lens`` (int, list, tuple, numpy
+        or torch): the ``lens`` to give ``prediction.decode_batch`` / ``kws_ctc_decode`` for the posteriors of
+        ``run_mel(mel, lens=lens)``."""
+        c = self.config.combine_frame
+        rule = (lambda t: t // c + 1) if c > 1 else (lambda t: t)       # kws_attention_frames
+        if isinstance(lens, (torch.Tensor, np.ndarray)):
+            return rule(lens)
+        if isinstance(lens, (list, tuple)):
+            return type(lens)(rule(int(t)) for t in lens)
+        return rule(int(lens))
+
+    def _check_lens(self, lens, B: int, T: int):
+        """lens -> int32 CUDA [B].  Host values are validated (1 <= lens <= T); CUDA values are left to the kernels,
+        which clamp them to [1, T] (reading them here would synchronise the stream)."""
+        if not _tensors.is_host(lens):
+            if tuple(lens.shape) != (B,) or lens.dtype.is_floating_point or lens.dtype == torch.bool:
+                raise _lib.InvalidArgumentError("lens must be integers [%d], got %s %r" % (B, lens.dtype, tuple(lens.shape)))
+            return _tensors.to_device(lens, torch.int32, self.device)
+        a = np.asarray(lens.numpy() if isinstance(lens, torch.Tensor) else lens)
+        if a.shape != (B,) or a.dtype.kind not in "iu":
+            raise _lib.InvalidArgumentError("lens must be integers [%d], got %s %r" % (B, a.dtype, a.shape))
+        if B and (a.min() < 1 or a.max() > T):
+            raise _lib.InvalidArgumentError("lens must lie in [1, T = %d], got [%d, %d]" % (T, a.min(), a.max()))
+        return _tensors.to_device(a.astype(np.int32), torch.int32, self.device)
+
+    def run_mel(self, mel, want_logits: bool = False, lens=None):
+        """mel ``[B, T, n_mel]`` (or ``[T, n_mel]``) -> softmax ``[B, T', C]`` [, logits].
+
+        ``lens [B]`` (host or CUDA integers): valid mel frames per utterance, in the first rows of ``mel``.  Utterance
+        b is computed exactly as a call on ``mel[b, :lens[b]]`` alone computes it, bit for bit; frames past lens[b] are
+        never read and its output rows from ``output_lengths(lens)[b]`` on are zero.  Host lens must lie in [1, T]."""
         host = _tensors.is_host(mel)
         x = _tensors.to_device(mel, torch.float32, self.device)
         if x.dim() == 2:
@@ -177,6 +209,7 @@ class AttentionDeployModel:
         if x.dim() != 3 or x.shape[2] != self.config.n_mel or x.shape[1] < 1:
             raise _lib.InvalidArgumentError("mel must be [B, T>=1, %d]" % self.config.n_mel)
         B, T, _ = x.shape
+        ln = None if lens is None else self._check_lens(lens, B, T)
         Tp, C = self.frames(T), self.config.num_classes
         probs = torch.empty((B, Tp, C), dtype=torch.float32, device=self.device)
         logits = torch.empty_like(probs) if want_logits else None
@@ -184,21 +217,40 @@ class AttentionDeployModel:
         with torch.cuda.device(self.device):
             for b0 in range(0, B, step):
                 b1 = min(B, b0 + step)
-                _lib.check(self._lib.kws_attention_forward(
-                    self._handle, _tensors.ptr(x[b0:b1]), b1 - b0, T, _tensors.ptr(probs[b0:b1]),
-                    _tensors.ptr(logits[b0:b1]) if want_logits else None, _tensors.stream_ptr(self.device)))
+                _lib.check(self._lib.kws_attention_forward_lens(
+                    self._handle, _tensors.ptr(x[b0:b1]), b1 - b0, T, _tensors.ptr(None if ln is None else ln[b0:b1]),
+                    _tensors.ptr(probs[b0:b1]), _tensors.ptr(logits[b0:b1]) if want_logits else None,
+                    _tensors.stream_ptr(self.device)))
         outs = [probs] + ([logits] if want_logits else [])
         if host:
             torch.cuda.current_stream(self.device).synchronize()
             outs = [_tensors.to_host(o) for o in outs]
         return tuple(outs) if want_logits else outs[0]
 
-    def forward(self, inputX, want_logits: bool = False):
-        """PCM ``[L]`` or ``[B, L]`` (float scaled by 2^-15, or int16) -> softmax ``[B, T', C]``."""
+    def forward(self, inputX, want_logits: bool = False, lengths=None):
+        """PCM ``[L]`` or ``[B, L]`` (float scaled by 2^-15, or int16) -> softmax ``[B, T', C]``.
+
+        ``lengths [B]``: valid samples per row (fft_size <= lengths <= L); row b is then computed as a call on
+        ``inputX[b, :lengths[b]]`` alone, on its ``1 + (lengths[b] - fft_size) // hop_size`` frames (``run_mel``'s
+        ``lens``).  Those frames read no sample past lengths[b], so one front-end call on the padded batch serves.  The
+        front end's mel frames of a padded row may differ from those of the row alone in the last bits, so the result
+        matches a call on the row alone to within 1e-5, not bit for bit (``run_mel`` with ``lens`` is bit for bit)."""
         host = _tensors.is_host(inputX)
+        lens = None
+        if lengths is not None:
+            shape = tuple(inputX.shape) if isinstance(inputX, torch.Tensor) else np.shape(inputX)
+            B, L = (1, shape[0]) if len(shape) == 1 else shape[:2]
+            a = np.asarray(lengths.cpu().numpy() if isinstance(lengths, torch.Tensor) else lengths)
+            c = self.config
+            if a.shape != (B,) or a.dtype.kind not in "iu":
+                raise _lib.InvalidArgumentError("lengths must be integers [%d], got %s %r" % (B, a.dtype, a.shape))
+            if B and (a.min() < c.fft_size or a.max() > L):
+                raise _lib.InvalidArgumentError("lengths must lie in [fft_size = %d, L = %d], got [%d, %d]"
+                                                % (c.fft_size, L, a.min(), a.max()))
+            lens = (1 + (a.astype(np.int64) - c.fft_size) // c.hop_size).astype(np.int32)
         mel = self._frontend.frontend(inputX if not host else np.asarray(inputX))
         mel_dev = _tensors.to_device(mel, torch.float32, self.device)
-        outs = self.run_mel(mel_dev, want_logits)
+        outs = self.run_mel(mel_dev, want_logits, lens=lens)
         if host:
             torch.cuda.current_stream(self.device).synchronize()
             outs = tuple(_tensors.to_host(o) for o in outs) if want_logits else _tensors.to_host(outs)

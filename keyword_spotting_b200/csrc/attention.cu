@@ -2,7 +2,7 @@
 // positional-encoding op.
 //
 // Reference: models/attention_ctc.py:73-128 (inference), :28-58 (self_attention), :61-70 (feed_forward),
-// :215-274 (DeployModel).  Per batch of equal-length utterances, on mel frames [B, T, M]:
+// :215-274 (DeployModel).  Per batch of utterances, on mel frames [B, T, M] of which utterance b has lens[b] valid:
 //   combine_frame=2 folding with the reference's padding rule (T' = T/2 + 1)       :77-90
 //   input_linear_trans (1x1 conv = dense + bias) + positional_encoding(T', N)       :92-98
 //   3 x { qkv dense, 8-head softmax(q k^T / sqrt(16)) v over ALL T' keys (no mask),
@@ -10,6 +10,14 @@
 //   output_linear_trans (+ relu when config.use_relu) and softmax                    :122-127, :272
 // tf.contrib.layers.layer_norm of that TensorFlow era normalises over all non-batch axes of [B, T', N]
 // (one mean/variance per utterance), gamma/beta per channel, epsilon 1e-12.
+//
+// Variable-length batches: every utterance is computed exactly as the graph computes it alone on its own lens[b] frames
+// (batch-1 sess.run): T'_b = att_frames(lens[b]) rows folded with zeros after frame lens[b], positions 0 .. T'_b - 1,
+// keys 0 .. T'_b - 1 only, layer-norm moments over T'_b x N; output rows T'_b .. T' - 1 are zero.  Rows keep the stride
+// T' of the longest utterance; each kernel reads its utterance's T'_b through AttLens (common.cuh) and never reads mel
+// frames at or past lens[b] or activation rows at or past T'_b.  Because every kernel does per utterance (attention
+// core, layer norm) or per row (dense, output) the same arithmetic as at T' = T'_b, the valid rows are bit-identical to
+// a call on that utterance alone.
 //
 // Dense layers: tcgen05 with fp16 hi/lo operand splits, fp32-grade (attention_tc.cu); the fp32 FFMA GEMM below remains for
 // shapes that kernel does not take.  Attention itself: one thread per query, online softmax, K/V blocks staged in shared
@@ -43,15 +51,16 @@ namespace kws {
 bool att_linear_tc_supported(int K, int N);                                                   // attention_tc.cu
 int att_pack_linear(const float* W, int K, int N, unsigned char** out, int* nchunks_out);
 int launch_att_linear_tc(const float* A, const unsigned char* wpack, int nchunks, const float* bias, const float* pe, int Tp,
-                         long rows, int K, int N, bool relu, bool add_pe, float* Y, cudaStream_t st);
+                         AttLens lens, long rows, int K, int N, bool relu, bool add_pe, float* Y, cudaStream_t st);
 bool att_core_tc_supported(int Tp, int heads, int hidden);
-int launch_att_core_tc(const float* qkv, long B, int Tp, int heads, float* out, cudaStream_t st);
+int launch_att_core_tc(const float* qkv, long B, int Tp, int heads, AttLens lens, float* out, cudaStream_t st);
 
 constexpr int kAttHidden = 128;
 constexpr int kAttHeadDim = 16;
 
-// ---- fold `combine` frames into one row with the reference's zero padding (:77-90)
-__global__ void att_combine_kernel(const float* __restrict__ mel, long B, int T, int M, int combine, int Tp,
+// ---- fold `combine` frames into one row with the reference's zero padding (:77-90) after the utterance's last frame
+// (rows at or past T'_b come out zero: their first frame lies past lens[b])
+__global__ void att_combine_kernel(const float* __restrict__ mel, long B, int T, int M, int combine, int Tp, AttLens lens,
                                    float* __restrict__ out) {
   const long idx = blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x;
   const int K = M * combine;
@@ -62,14 +71,16 @@ __global__ void att_combine_kernel(const float* __restrict__ mel, long B, int T,
   const int tp = static_cast<int>(row % Tp);
   const long b = row / Tp;
   const int f = tp * combine + j / M;
-  out[idx] = f < T ? mel[(b * T + f) * M + j % M] : 0.0f;
+  out[idx] = f < lens.frames_in(b) ? mel[(b * T + f) * M + j % M] : 0.0f;
 }
 
-// ---- Y[r, n] = act(sum_k A[r,k] W[k,n] + bias[n]) (+ pe[r % Tp, n]);  64x64 tile, 256 threads x (4x4)
+// ---- Y[r, n] = act(sum_k A[r,k] W[k,n] + bias[n]) (+ pe[r % Tp, n]);  64x64 tile, 256 threads x (4x4); a tile of
+// padding rows only (at or past their utterances' T'_b) does nothing
 template <bool kRelu, bool kAddPe>
 __global__ void __launch_bounds__(256)
 att_linear_kernel(const float* __restrict__ A, const float* __restrict__ W, const float* __restrict__ bias,
-                  const float* __restrict__ pe, int Tp, long rows, int K, int N, float* __restrict__ Y) {
+                  const float* __restrict__ pe, int Tp, AttLens lens, long rows, int K, int N, float* __restrict__ Y) {
+  if (!lens.tile_live(Tp, rows, blockIdx.x * 64L, 64)) return;
   __shared__ float sA[16][64 + 4];
   __shared__ float sW[16][64];
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;          // 16 x 16 threads
@@ -117,27 +128,31 @@ att_linear_kernel(const float* __restrict__ A, const float* __restrict__ W, cons
   }
 }
 
-// ---- multi-head attention: one thread per query row, K/V blocks of 128 keys in shared memory, online softmax
+// ---- multi-head attention: one thread per query row, K/V blocks of 128 keys in shared memory, online softmax over the
+// utterance's T'_b keys (Tp is the row stride); utterances with T'_b <= skip_upto are left to the tensor-core core
 __global__ void __launch_bounds__(128)
-att_attention_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __restrict__ out) {
+att_attention_kernel(const float* __restrict__ qkv, int Tp, int heads, AttLens lens, int skip_upto,
+                     float* __restrict__ out) {
   __shared__ float sK[128][kAttHeadDim];
   __shared__ float sV[128][kAttHeadDim];
   const int N = heads * kAttHeadDim;
   const int h = blockIdx.y;
   const long b = blockIdx.z;
+  const int Tb = lens.rows_of(b);
+  if (Tb <= skip_upto || blockIdx.x * 128 >= Tb) return;
   const int i = blockIdx.x * 128 + threadIdx.x;
   const float* base = qkv + b * Tp * 3L * N;
   const float scale = rsqrtf(static_cast<float>(kAttHeadDim)) * 1.4426950408889634f;   // 1/sqrt(d), in log2 units
   float q[kAttHeadDim], o[kAttHeadDim];
 #pragma unroll
   for (int d = 0; d < kAttHeadDim; ++d) {
-    q[d] = i < Tp ? base[static_cast<long>(i) * 3 * N + h * kAttHeadDim + d] * scale : 0.0f;
+    q[d] = i < Tb ? base[static_cast<long>(i) * 3 * N + h * kAttHeadDim + d] * scale : 0.0f;
     o[d] = 0.0f;
   }
   float m = -INFINITY, l = 0.0f;
-  for (int j0 = 0; j0 < Tp; j0 += 128) {
+  for (int j0 = 0; j0 < Tb; j0 += 128) {
     const int j = j0 + threadIdx.x;
-    if (j < Tp) {
+    if (j < Tb) {
       const float4* kp = reinterpret_cast<const float4*>(base + static_cast<long>(j) * 3 * N + N + h * kAttHeadDim);
       const float4* vp = reinterpret_cast<const float4*>(base + static_cast<long>(j) * 3 * N + 2 * N + h * kAttHeadDim);
 #pragma unroll
@@ -147,7 +162,7 @@ att_attention_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __
       }
     }
     __syncthreads();
-    const int nk = Tp - j0 < 128 ? Tp - j0 : 128;
+    const int nk = Tb - j0 < 128 ? Tb - j0 : 128;
     for (int jj = 0; jj < nk; ++jj) {
       float s = 0.0f;
 #pragma unroll
@@ -166,7 +181,7 @@ att_attention_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __
     }
     __syncthreads();
   }
-  if (i < Tp) {
+  if (i < Tb) {
     const float inv = 1.0f / l;
     float* dst = out + (b * Tp + i) * N + h * kAttHeadDim;
 #pragma unroll
@@ -174,7 +189,8 @@ att_attention_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __
   }
 }
 
-// ---- y = layer_norm(a + b) over all T'*N elements of one utterance, per-channel gamma/beta
+// ---- y = layer_norm(a + b) over all T'_b * N elements of one utterance, per-channel gamma/beta; rows at or past T'_b are
+// neither read nor written.  The reduction order depends on T'_b only, not on the row stride Tp nor on in_smem.
 __device__ __forceinline__ float block_sum(float v, float* red) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -194,13 +210,13 @@ __device__ __forceinline__ float block_sum(float v, float* red) {
 
 __global__ void __launch_bounds__(1024)
 att_add_layernorm_kernel(const float* __restrict__ a, const float* __restrict__ b, const float* __restrict__ gamma,
-                         const float* __restrict__ beta, int Tp, int N, int in_smem, float* __restrict__ y) {
+                         const float* __restrict__ beta, int Tp, AttLens lens, int N, int in_smem, float* __restrict__ y) {
   // the utterance's a + b is kept in shared memory when it fits (T' * N <= 51,200 floats: 8 s at config 5), so a and b
   // are read from HBM once and the mean / variance / output passes run out of shared memory; N % 4 == 0
   extern __shared__ __align__(16) float sx[];
   __shared__ float red[32];
   const long base = blockIdx.x * static_cast<long>(Tp) * N;
-  const int n = Tp * N, n4 = n >> 2;
+  const int n = lens.rows_of(blockIdx.x) * N, n4 = n >> 2;
   const float4* a4 = reinterpret_cast<const float4*>(a + base);
   const float4* b4 = reinterpret_cast<const float4*>(b + base);
   float4* s4 = reinterpret_cast<float4*>(sx);
@@ -243,16 +259,23 @@ att_add_layernorm_kernel(const float* __restrict__ a, const float* __restrict__ 
   }
 }
 
-// ---- output_linear_trans (+relu) + softmax: one thread per row
+// ---- output_linear_trans (+relu) + softmax: one thread per row; rows at or past T'_b are written as zeros
 __global__ void __launch_bounds__(128)
 att_output_kernel(const float* __restrict__ x, const float* __restrict__ w, const float* __restrict__ bias, long rows,
-                  int N, int C, int use_relu, float* __restrict__ probs, float* __restrict__ logits) {
+                  int Tp, AttLens lens, int N, int C, int use_relu, float* __restrict__ probs, float* __restrict__ logits) {
   extern __shared__ float sw[];                       // [N][C] + [C]
+  const long r = blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x;
+  const bool pad = lens.lens && r < rows && r % Tp >= lens.rows_of(r / Tp);   // a row at or past T'_b
+  if (pad) {
+    for (int c = 0; c < C; ++c) {
+      probs[r * C + c] = 0.0f;
+      if (logits) logits[r * C + c] = 0.0f;
+    }
+  }
   for (int i = threadIdx.x; i < N * C; i += blockDim.x) sw[i] = w[i];
   for (int i = threadIdx.x; i < C; i += blockDim.x) sw[N * C + i] = bias[i];
   __syncthreads();
-  const long r = blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x;
-  if (r >= rows) return;
+  if (r >= rows || pad) return;
   float acc[kMaxClasses];
   for (int c = 0; c < C; ++c) acc[c] = sw[N * C + c];
   const float4* xr = reinterpret_cast<const float4*>(x + r * N);
@@ -308,19 +331,32 @@ static void att_free(kws_attention* m) {
 
 template <bool R, bool P>
 static int att_linear(const float* A, const float* W, const kws_attention::Packed& pk, const float* bias, const float* pe, int Tp,
-                      long rows, int K, int N, float* Y, cudaStream_t st) {
-  if (pk.w) return launch_att_linear_tc(A, pk.w, pk.nchunks, bias, pe, Tp, rows, K, N, R, P, Y, st);   // tcgen05, fp32-grade
+                      AttLens lens, long rows, int K, int N, float* Y, cudaStream_t st) {
+  if (pk.w) return launch_att_linear_tc(A, pk.w, pk.nchunks, bias, pe, Tp, lens, rows, K, N, R, P, Y, st);   // tcgen05, fp32-grade
   dim3 grid(static_cast<unsigned>(ceil_div(rows, 64)), static_cast<unsigned>(ceil_div(N, 64)));
-  att_linear_kernel<R, P><<<grid, 256, 0, st>>>(A, W, bias, pe, Tp, rows, K, N, Y);
+  att_linear_kernel<R, P><<<grid, 256, 0, st>>>(A, W, bias, pe, Tp, lens, rows, K, N, Y);
   KWS_LAUNCH_OK("att_linear_kernel");
   return KWS_OK;
 }
 
-static int att_core_ffma(const float* qkv, long B, int Tp, int heads, float* out, cudaStream_t st) {
+static int att_core_ffma(const float* qkv, long B, int Tp, int heads, AttLens lens, int skip_upto, float* out, cudaStream_t st) {
   dim3 ga(static_cast<unsigned>(ceil_div(Tp, 128)), static_cast<unsigned>(heads), static_cast<unsigned>(B));
-  att_attention_kernel<<<ga, 128, 0, st>>>(qkv, Tp, heads, out);
+  att_attention_kernel<<<ga, 128, 0, st>>>(qkv, Tp, heads, lens, skip_upto, out);
   KWS_LAUNCH_OK("att_attention_kernel");
   return KWS_OK;
+}
+
+// the attention core of one layer.  Every utterance goes to the core a call on it alone would use: the tensor cores when
+// T'_b <= 400, the FFMA kernel otherwise.  With T' <= 400 that is the tcgen05 core alone; past it, with lengths, both
+// kernels run and each returns at once for the other's utterances.
+static int att_core(const float* qkv, long B, int Tp, int heads, AttLens lens, float* out, cudaStream_t st) {
+  if (att_core_tc_supported(Tp, heads, heads * kAttHeadDim)) return launch_att_core_tc(qkv, B, Tp, heads, lens, out, st);
+  if (lens.lens) {
+    const int rc = launch_att_core_tc(qkv, B, Tp, heads, lens, out, st);
+    if (rc != KWS_OK) return rc;
+    return att_core_ffma(qkv, B, Tp, heads, lens, kAttCoreTcMaxKeys, out, st);
+  }
+  return att_core_ffma(qkv, B, Tp, heads, lens, 0, out, st);
 }
 
 constexpr int kLnSmemBytes = 200 * 1024;       // the layer norm keeps a + b in shared memory up to this size
@@ -396,12 +432,16 @@ extern "C" int kws_attention_destroy(kws_attention* m) {
 }
 
 extern "C" int32_t kws_attention_frames(const kws_attention* m, int32_t T) {
-  const int c = m ? m->cfg.combine_frame : 2;
-  return c > 1 ? T / c + 1 : T;                      // models/attention_ctc.py:88-90
+  return att_frames(T, m ? m->cfg.combine_frame : 2);   // models/attention_ctc.py:88-90
 }
 
 extern "C" int kws_attention_forward(kws_attention* m, const float* mel, int64_t B, int32_t T, float* probs_out,
                                      float* logits_out, void* stream) {
+  return kws_attention_forward_lens(m, mel, B, T, nullptr, probs_out, logits_out, stream);
+}
+
+extern "C" int kws_attention_forward_lens(kws_attention* m, const float* mel, int64_t B, int32_t T, const int32_t* lens,
+                                          float* probs_out, float* logits_out, void* stream) {
   clear_error();
   KWS_REQUIRE(m != nullptr, "model is NULL");
   KWS_REQUIRE(B >= 0 && T >= 1, "need at least one frame");
@@ -448,32 +488,28 @@ extern "C" int kws_attention_forward(kws_attention* m, const float* mel, int64_t
   const int ln_in_smem = ln_bytes <= kLnSmemBytes ? 1 : 0;
   const size_t ln_smem = ln_in_smem ? ln_bytes : 0;
   KWS_CUDA_OK(cudaFuncSetAttribute(att_add_layernorm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnSmemBytes));
+  const AttLens L{lens, T, c.combine_frame};
   const long total_in = rows * Kin;
-  att_combine_kernel<<<static_cast<unsigned>(ceil_div(total_in, 256)), 256, 0, st>>>(mel, B, T, c.n_mel, c.combine_frame, Tp, xin);
+  att_combine_kernel<<<static_cast<unsigned>(ceil_div(total_in, 256)), 256, 0, st>>>(mel, B, T, c.n_mel, c.combine_frame, Tp,
+                                                                                     L, xin);
   KWS_LAUNCH_OK("att_combine_kernel");
-  int rc = att_linear<false, true>(xin, m->w_in, m->p_in, m->b_in, m->pe, Tp, rows, Kin, N, x, st);
+  int rc = att_linear<false, true>(xin, m->w_in, m->p_in, m->b_in, m->pe, Tp, L, rows, Kin, N, x, st);
   for (int l = 0; l < c.num_layers && rc == KWS_OK; ++l) {
-    const auto& L = m->layer[l];
-    rc = att_linear<false, false>(x, L.w_qkv, m->p_qkv[l], L.b_qkv, nullptr, Tp, rows, N, 3 * N, big, st);
+    const auto& W = m->layer[l];
+    rc = att_linear<false, false>(x, W.w_qkv, m->p_qkv[l], W.b_qkv, nullptr, Tp, L, rows, N, 3 * N, big, st);
+    if (rc == KWS_OK) rc = att_core(big, B, Tp, c.heads, L, att, st);
     if (rc != KWS_OK) break;
-    if (att_core_tc_supported(Tp, c.heads, N)) {                     // tcgen05: T' <= 400 keys
-      rc = launch_att_core_tc(big, B, Tp, c.heads, att, st);
-      if (rc != KWS_OK) break;
-    } else {
-      rc = att_core_ffma(big, B, Tp, c.heads, att, st);
-      if (rc != KWS_OK) break;
-    }
-    att_add_layernorm_kernel<<<static_cast<unsigned>(B), 1024, ln_smem, st>>>(att, x, L.ln1_g, L.ln1_b, Tp, N, ln_in_smem, y);
+    att_add_layernorm_kernel<<<static_cast<unsigned>(B), 1024, ln_smem, st>>>(att, x, W.ln1_g, W.ln1_b, Tp, L, N, ln_in_smem, y);
     KWS_LAUNCH_OK("att_add_layernorm_kernel");
-    rc = att_linear<true, false>(y, L.w_ff1, m->p_ff1[l], L.b_ff1, nullptr, Tp, rows, N, F, big, st);
-    if (rc == KWS_OK) rc = att_linear<false, false>(big, L.w_ff2, m->p_ff2[l], L.b_ff2, nullptr, Tp, rows, F, N, att, st);
+    rc = att_linear<true, false>(y, W.w_ff1, m->p_ff1[l], W.b_ff1, nullptr, Tp, L, rows, N, F, big, st);
+    if (rc == KWS_OK) rc = att_linear<false, false>(big, W.w_ff2, m->p_ff2[l], W.b_ff2, nullptr, Tp, L, rows, F, N, att, st);
     if (rc != KWS_OK) break;
-    att_add_layernorm_kernel<<<static_cast<unsigned>(B), 1024, ln_smem, st>>>(att, y, L.ln2_g, L.ln2_b, Tp, N, ln_in_smem, x);
+    att_add_layernorm_kernel<<<static_cast<unsigned>(B), 1024, ln_smem, st>>>(att, y, W.ln2_g, W.ln2_b, Tp, L, N, ln_in_smem, x);
     KWS_LAUNCH_OK("att_add_layernorm_kernel");
   }
   if (rc != KWS_OK) return rc;
   att_output_kernel<<<static_cast<unsigned>(ceil_div(rows, 128)), 128, sizeof(float) * (N * C + C), st>>>(
-      x, m->w_out, m->b_out, rows, N, C, c.use_relu, probs_out, logits_out);
+      x, m->w_out, m->b_out, rows, Tp, L, N, C, c.use_relu, probs_out, logits_out);
   KWS_LAUNCH_OK("att_output_kernel");
   return KWS_OK;
 }
@@ -493,10 +529,11 @@ extern "C" int kws_debug_att_linear(const float* A, const float* W_host, const f
   float* dW = nullptr;
   int rc = path == 0 ? att_pack_linear(W_host, K, N, &pk.w, &pk.nchunks) : att_upload(&dW, W_host, static_cast<size_t>(K) * N);
   if (rc == KWS_OK) {
-    if (relu) rc = add_pe ? att_linear<true, true>(A, dW, pk, bias, pe, Tp, rows, K, N, Y, st)
-                          : att_linear<true, false>(A, dW, pk, bias, pe, Tp, rows, K, N, Y, st);
-    else rc = add_pe ? att_linear<false, true>(A, dW, pk, bias, pe, Tp, rows, K, N, Y, st)
-                     : att_linear<false, false>(A, dW, pk, bias, pe, Tp, rows, K, N, Y, st);
+    const AttLens all{nullptr, Tp, 1};
+    if (relu) rc = add_pe ? att_linear<true, true>(A, dW, pk, bias, pe, Tp, all, rows, K, N, Y, st)
+                          : att_linear<true, false>(A, dW, pk, bias, pe, Tp, all, rows, K, N, Y, st);
+    else rc = add_pe ? att_linear<false, true>(A, dW, pk, bias, pe, Tp, all, rows, K, N, Y, st)
+                     : att_linear<false, false>(A, dW, pk, bias, pe, Tp, all, rows, K, N, Y, st);
   }
   const cudaError_t e = cudaStreamSynchronize(st);
   cudaFree(pk.w);
@@ -508,6 +545,11 @@ extern "C" int kws_debug_att_linear(const float* A, const float* W_host, const f
 
 extern "C" int kws_debug_att_core(const float* qkv, int64_t B, int32_t Tp, int32_t heads, int path, float* out,
                                   void* stream) {
+  return kws_debug_att_core_lens(qkv, B, Tp, nullptr, heads, path, out, stream);
+}
+
+extern "C" int kws_debug_att_core_lens(const float* qkv, int64_t B, int32_t Tp, const int32_t* lens, int32_t heads, int path,
+                                       float* out, void* stream) {
   clear_error();
   KWS_REQUIRE(qkv && out, "NULL pointer");
   KWS_REQUIRE(B >= 1 && B <= 65535 && Tp >= 1 && heads >= 1 && heads <= 64, "bad sizes");
@@ -515,7 +557,8 @@ extern "C" int kws_debug_att_core(const float* qkv, int64_t B, int32_t Tp, int32
   if (path == 0 && !att_core_tc_supported(Tp, heads, heads * kAttHeadDim))
     return fail(KWS_ERR_UNSUPPORTED, "the tensor-core attention core takes 1 <= T' <= 400 (T' = %d)", Tp);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int rc = path == 0 ? launch_att_core_tc(qkv, B, Tp, heads, out, st) : att_core_ffma(qkv, B, Tp, heads, out, st);
+  const AttLens L{lens, Tp, 1};
+  const int rc = path == 0 ? launch_att_core_tc(qkv, B, Tp, heads, L, out, st) : att_core_ffma(qkv, B, Tp, heads, L, 0, out, st);
   const cudaError_t e = cudaStreamSynchronize(st);
   if (rc != KWS_OK) return rc;
   if (e != cudaSuccess) return fail(KWS_ERR_CUDA, "attention core (path %d) failed: %s", path, cudaGetErrorString(e));
@@ -524,6 +567,12 @@ extern "C" int kws_debug_att_core(const float* qkv, int64_t B, int32_t Tp, int32
 
 extern "C" int kws_debug_att_add_layernorm(const float* a, const float* b, const float* gamma, const float* beta,
                                            int64_t B, int32_t Tp, int32_t N, int in_smem, float* y, void* stream) {
+  return kws_debug_att_add_layernorm_lens(a, b, gamma, beta, B, Tp, nullptr, N, in_smem, y, stream);
+}
+
+extern "C" int kws_debug_att_add_layernorm_lens(const float* a, const float* b, const float* gamma, const float* beta,
+                                                int64_t B, int32_t Tp, const int32_t* lens, int32_t N, int in_smem, float* y,
+                                                void* stream) {
   clear_error();
   KWS_REQUIRE(a && b && gamma && beta && y, "NULL pointer");
   KWS_REQUIRE(B >= 1 && B <= (1L << 31) - 1 && Tp >= 1 && N >= 1 && static_cast<int64_t>(Tp) * N < (1L << 31), "bad sizes");
@@ -533,8 +582,8 @@ extern "C" int kws_debug_att_add_layernorm(const float* a, const float* b, const
     return fail(KWS_ERR_UNSUPPORTED, "T' * N = %d floats do not fit the layer norm's shared memory", Tp * N);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   KWS_CUDA_OK(cudaFuncSetAttribute(att_add_layernorm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnSmemBytes));
-  att_add_layernorm_kernel<<<static_cast<unsigned>(B), 1024, in_smem ? bytes : 0, st>>>(a, b, gamma, beta, Tp, N,
-                                                                                       in_smem ? 1 : 0, y);
+  att_add_layernorm_kernel<<<static_cast<unsigned>(B), 1024, in_smem ? bytes : 0, st>>>(a, b, gamma, beta, Tp,
+                                                                                       AttLens{lens, Tp, 1}, N, in_smem ? 1 : 0, y);
   KWS_LAUNCH_OK("att_add_layernorm_kernel");
   const cudaError_t e = cudaStreamSynchronize(st);
   if (e != cudaSuccess) return fail(KWS_ERR_CUDA, "att_add_layernorm_kernel failed: %s", cudaGetErrorString(e));

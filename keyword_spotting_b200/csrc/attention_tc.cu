@@ -3,6 +3,8 @@
 //
 //   Y[r, n] = act( sum_k A[r, k] W[k, n] + bias[n] ) (+ pe[r % Tp, n])          A fp32 [rows, K], Y fp32 [rows, N]
 //
+// In a variable-length batch a tile whose 128 rows all lie at or past their utterances' T'_b loads and stores nothing.
+//
 // One CTA = a [128 rows, 128 columns] output tile, three CTAs per SM.  K is walked in chunks of 64: the CTA's 256 threads
 // read the A chunk from HBM (coalesced 16-byte loads), split every value into two fp16 terms (x = hi + lo, exact to
 // 2^-22) and store both in the tcgen05 K-major canonical layout in shared memory; the weight chunk arrives pre-split and
@@ -32,7 +34,9 @@ constexpr int kAlSmem = 2 * kAlPartA + 2 * kAlPartW;
 template <bool kRelu, bool kAddPe>
 __global__ void __launch_bounds__(kAlThreads, 3)
 att_linear_tc_kernel(const float* __restrict__ A, const unsigned char* __restrict__ wpack, const float* __restrict__ bias,
-                     const float* __restrict__ pe, int Tp, long rows, int K, int nchunks, int N, float* __restrict__ Y) {
+                     const float* __restrict__ pe, int Tp, AttLens lens, long rows, int K, int nchunks, int N,
+                     float* __restrict__ Y) {
+  if (!lens.tile_live(Tp, rows, blockIdx.x * static_cast<long>(kAlTile), kAlTile)) return;   // padding rows only
   extern __shared__ __align__(128) unsigned char smem[];
   unsigned char* sA = smem;                               // [hi | lo] x kAlPartA
   unsigned char* sW = smem + 2 * kAlPartA;                // [hi | lo] x kAlPartW
@@ -200,12 +204,12 @@ int att_pack_linear(const float* W, int K, int N, unsigned char** out, int* nchu
 }
 
 int launch_att_linear_tc(const float* A, const unsigned char* wpack, int nchunks, const float* bias, const float* pe, int Tp,
-                         long rows, int K, int N, bool relu, bool add_pe, float* Y, cudaStream_t st) {
+                         AttLens lens, long rows, int K, int N, bool relu, bool add_pe, float* Y, cudaStream_t st) {
   if (rows <= 0) return KWS_OK;
   dim3 grid(static_cast<unsigned>(ceil_div(rows, kAlTile)), static_cast<unsigned>(N / kAlTile));
   auto launch = [&](auto kernel) -> int {
     KWS_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kAlSmem));
-    kernel<<<grid, kAlThreads, kAlSmem, st>>>(A, wpack, bias, pe, Tp, rows, K, nchunks, N, Y);
+    kernel<<<grid, kAlThreads, kAlSmem, st>>>(A, wpack, bias, pe, Tp, lens, rows, K, nchunks, N, Y);
     return KWS_OK;
   };
   int rc;
@@ -218,7 +222,9 @@ int launch_att_linear_tc(const float* A, const unsigned char* wpack, int nchunks
 
 // ---------------------------------------------------------------------------------------------------------------------
 // Multi-head attention core on the tensor cores (models/attention_ctc.py:28-58): per (utterance, head)
-//     O = softmax(Q K^T / sqrt(16)) V        over ALL T' keys (no mask), T' <= 400, head size 16.
+//     O = softmax(Q K^T / sqrt(16)) V        over ALL T'_b keys of the utterance (no mask), T'_b <= 400, head size 16.
+// Rows are laid out with stride T' (the batch's longest); utterance b has its own T'_b <= T' rows and keys, and CTAs of
+// utterances with T'_b > 400 return at once (the FFMA core takes those).
 // One CTA per (utterance, head); K and V^T are split into fp16 hi/lo once and stay in shared memory as B operands, the
 // CTA then walks the utterance's query tiles of 128 rows:
 //   S = Q K^T   6 tcgen05.mma (3 hi/lo products x N = 256 + the rest, K = 16) into T' columns of TMEM;
@@ -230,7 +236,7 @@ int launch_att_linear_tc(const float* A, const unsigned char* wpack, int nchunks
 // fp32-grade throughout (the dropped lo x lo terms are 2^-22 relative): the model's 1e-4 parity tests are unchanged.
 constexpr int kAcThreads = 256;
 constexpr int kAcD = 16;
-constexpr int kAcMaxKeys = 400;                  // T' padded to a multiple of 16; TMEM: 400 score columns + 16 for O
+constexpr int kAcMaxKeys = kAttCoreTcMaxKeys;    // T' padded to a multiple of 16; TMEM: 400 score columns + 16 for O
 constexpr int kAcSboK = 2 * 128;                 // K operand [keys, 16]: two K-adjacent core matrices per 8-key group
 constexpr int kAcPartK = (kAcMaxKeys / 8) * kAcSboK;      // 12800
 constexpr int kAcSboV = (kAcMaxKeys / 8) * 128;  // V^T operand [16, keys]: 6400 between the two 8-row groups
@@ -245,7 +251,10 @@ __device__ __forceinline__ float ex2_fast(float x) {
 }
 
 __global__ void __launch_bounds__(kAcThreads, 1)
-att_core_tc_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __restrict__ out) {
+att_core_tc_kernel(const float* __restrict__ qkv, int Tp, int heads, AttLens lens, float* __restrict__ out) {
+  const long b = blockIdx.x / heads;
+  const int Tb = lens.rows_of(b);                               // this utterance's keys and queries; Tp is the row stride
+  if (Tb > kAcMaxKeys) return;
   extern __shared__ __align__(128) unsigned char smem[];
   unsigned char* sK = smem;                                      // [hi | lo] x kAcPartK
   unsigned char* sV = sK + 2 * kAcPartK;
@@ -256,9 +265,8 @@ att_core_tc_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __re
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int N = heads * kAcD;
   const int h = blockIdx.x % heads;
-  const long b = blockIdx.x / heads;
   const float* base = qkv + b * Tp * 3L * N + h * kAcD;
-  const int Kp = (Tp + 15) & ~15;                               // keys padded to whole MMA K steps
+  const int Kp = (Tb + 15) & ~15;                               // keys padded to whole MMA K steps
   const int groups = Kp / 16;
   const float scale = rsqrtf(static_cast<float>(kAcD)) * 1.4426950408889634f;     // 1/sqrt(d), in log2 units
 
@@ -273,7 +281,7 @@ att_core_tc_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __re
 #pragma unroll
     for (int c = 0; c < 4; ++c) {
       float4 k4 = make_float4(0.f, 0.f, 0.f, 0.f), v4 = k4;
-      if (j < Tp) {
+      if (j < Tb) {
         k4 = __ldg(reinterpret_cast<const float4*>(base + static_cast<long>(j) * 3 * N + N) + c);
         v4 = __ldg(reinterpret_cast<const float4*>(base + static_cast<long>(j) * 3 * N + 2 * N) + c);
       }
@@ -315,7 +323,7 @@ att_core_tc_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __re
   const int g_begin = ch == 0 ? 0 : g_split, g_end = ch == 0 ? g_split : groups;
   uint32_t phase = 0;
 
-  for (int i0 = 0; i0 < Tp; i0 += 128) {
+  for (int i0 = 0; i0 < Tb; i0 += 128) {
     // ---- Q tile: row = query i0 + r, scaled to log2 units, hi / lo
     if (tid < 128) {
       const int i = i0 + tid;
@@ -325,7 +333,7 @@ att_core_tc_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __re
 #pragma unroll
         for (int e = 0; e < 2; ++e) {
           float4 q4v = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (i < Tp) q4v = __ldg(reinterpret_cast<const float4*>(base + static_cast<long>(i) * 3 * N) + 2 * c + e);
+          if (i < Tb) q4v = __ldg(reinterpret_cast<const float4*>(base + static_cast<long>(i) * 3 * N) + 2 * c + e);
           v8[4 * e] = q4v.x * scale; v8[4 * e + 1] = q4v.y * scale; v8[4 * e + 2] = q4v.z * scale; v8[4 * e + 3] = q4v.w * scale;
         }
         uint4 hi, lo;
@@ -360,8 +368,8 @@ att_core_tc_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __re
     tc::fence_after_sync();
     // (a warp whose 32 query rows all lie past T' -- three of the four lane quarters of the last tile -- skips both passes:
     // its rows of P stay garbage, which only reaches its own, never stored, rows of O)
-    const bool warp_live = i0 + 32 * q4 < Tp;
-    const int g_tail = (Tp & 15) ? groups - 1 : groups;          // the one key group with padded keys, if any
+    const bool warp_live = i0 + 32 * q4 < Tb;
+    const int g_tail = (Tb & 15) ? groups - 1 : groups;          // the one key group with padded keys, if any
     // ---- pass 1: row maximum over this warp's key groups
     float mx = -INFINITY;
     if (warp_live) {
@@ -375,7 +383,7 @@ att_core_tc_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __re
         } else {
 #pragma unroll
           for (int e = 0; e < 16; ++e)
-            if (16 * g + e < Tp) mx = fmaxf(mx, __uint_as_float(v[e]));
+            if (16 * g + e < Tb) mx = fmaxf(mx, __uint_as_float(v[e]));
         }
       }
     }
@@ -394,8 +402,8 @@ att_core_tc_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __re
         for (int e = 0; e < 16; e += 2) {
           float p0 = ex2_fast(__uint_as_float(v[e]) - mx), p1 = ex2_fast(__uint_as_float(v[e + 1]) - mx);
           if (g >= g_tail) {                                     // padded keys carry no weight
-            if (16 * g + e >= Tp) p0 = 0.0f;
-            if (16 * g + e + 1 >= Tp) p1 = 0.0f;
+            if (16 * g + e >= Tb) p0 = 0.0f;
+            if (16 * g + e + 1 >= Tb) p1 = 0.0f;
           }
           sum += p0 + p1;
           const __half2 hh = __floats2half2_rn(p0, p1);
@@ -433,7 +441,7 @@ att_core_tc_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __re
       tc::ld16(tmem + lane_sel + kAcColO, v);
       tc::wait_ld();
       const int i = i0 + row;
-      if (i < Tp) {
+      if (i < Tb) {
         const float inv = 1.0f / (sSum[0][row] + sSum[1][row]);
         float4* dst = reinterpret_cast<float4*>(out + (b * Tp + i) * N + h * kAcD);
 #pragma unroll
@@ -451,11 +459,11 @@ att_core_tc_kernel(const float* __restrict__ qkv, int Tp, int heads, float* __re
 
 bool att_core_tc_supported(int Tp, int heads, int hidden) { return Tp >= 1 && Tp <= kAcMaxKeys && hidden == heads * kAcD; }
 
-int launch_att_core_tc(const float* qkv, long B, int Tp, int heads, float* out, cudaStream_t st) {
+int launch_att_core_tc(const float* qkv, long B, int Tp, int heads, AttLens lens, float* out, cudaStream_t st) {
   if (B <= 0) return KWS_OK;
   constexpr int smem = 2 * kAcPartK + 2 * kAcPartV + 2 * kAcPartQ;
   KWS_CUDA_OK(cudaFuncSetAttribute(att_core_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  att_core_tc_kernel<<<static_cast<unsigned>(B * heads), kAcThreads, smem, st>>>(qkv, Tp, heads, out);
+  att_core_tc_kernel<<<static_cast<unsigned>(B * heads), kAcThreads, smem, st>>>(qkv, Tp, heads, lens, out);
   KWS_LAUNCH_OK("att_core_tc_kernel");
   return KWS_OK;
 }

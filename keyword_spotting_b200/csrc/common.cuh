@@ -48,6 +48,32 @@ int fail(int code, const char* fmt, ...);
 
 inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// -------------------------------------------------------------------- attention_ctc: per-utterance lengths
+// T' of T mel frames (models/attention_ctc.py:88-90): kws_attention_frames and every attention kernel use this one rule.
+__host__ __device__ __forceinline__ int att_frames(int T, int combine) { return combine > 1 ? T / combine + 1 : T; }
+
+constexpr int kAttCoreTcMaxKeys = 400;   // the tensor-core attention core takes T' <= 400 (attention_tc.cu)
+
+// The lengths of a variable-length attention batch as every kernel sees them: utterance b has lens[b] valid frames,
+// clamped to [1, T], and T'_b = att_frames(lens[b], combine) rows.  lens == nullptr: every utterance has T frames.
+// The forward pass passes mel frames (T, combine of the model); the single-kernel debug entry points pass rows
+// (T = T', combine = 1).  Row strides stay T' = att_frames(T, combine) whatever the lengths.
+struct AttLens {
+  const int32_t* lens;
+  int T;
+  int combine;
+  __device__ __forceinline__ int frames_in(long b) const { return lens ? min(max(__ldg(lens + b), 1), T) : T; }
+  __device__ __forceinline__ int rows_of(long b) const { return att_frames(frames_in(b), combine); }
+  // does [r0, r0 + tile) of a [B * Tp, .] activation hold a row of some utterance's first T'_b rows?  (O(1): a tile that
+  // reaches the next utterance holds that utterance's row 0, which every utterance has)
+  __device__ __forceinline__ bool tile_live(int Tp, long rows, long r0, int tile) const {
+    if (!lens) return true;
+    const long b0 = r0 / Tp;
+    const long rlast = (r0 + tile < rows ? r0 + tile : rows) - 1;
+    return r0 - b0 * Tp < rows_of(b0) || (b0 + 1) * Tp <= rlast;
+  }
+};
+
 int sm_count();   // SMs of the current device (cached)
 
 // -------------------------------------------------------------------- model

@@ -56,23 +56,33 @@ def evaluate_softmax(softmax, correctness, lens=None, label_seqs: str = "1233", 
 
 
 def validate(model, batches: Iterable[Tuple], label_seqs: Optional[str] = None) -> ValidationResult:
-    """Run the validation set through ``model`` (a DeployModel).
+    """Run the validation set through ``model`` (a DeployModel or an AttentionDeployModel).
 
     ``batches`` yields ``(inputs, lens, correctness)``: inputs are mel frames ``[B, T, n_mel]`` (the valid
     queue's form, reader.py:282-305) or PCM ``[B, L]``; ``lens`` valid frames per utterance (or None).
+    PCM rows are taken as equal-length utterances.  For the attention model ``lens`` are mel frames: mel batches run
+    with them, and the decoder takes the model's ``output_lengths(lens)``.
     """
+    from .attention_ctc import AttentionDeployModel
     label_seqs = label_seqs or model.config.label_seqs
     res = ValidationResult(miss=0, target=0, false_accept=0, total=0)
     for inputs, lens, correctness in batches:
         x = inputs if isinstance(inputs, torch.Tensor) else np.asarray(inputs)
         B = x.shape[0]
-        state = torch.zeros((model.config.num_layers, B, model.config.hidden_size), dtype=torch.float32, device=model.device)
+        attention = isinstance(model, AttentionDeployModel)
         if x.ndim == 3:
-            probs, _ = model.run_mel(_tensors.to_device(x, torch.float32, model.device), state, seq_len=lens)
+            mel = _tensors.to_device(x, torch.float32, model.device)
         else:
             is_i16 = x.dtype in (np.int16, torch.int16)
-            probs, _ = model(_tensors.to_device(x, torch.int16 if is_i16 else torch.float32, model.device), state)
-        miss, target, fa, _ = evaluate_softmax(probs, correctness, lens=lens, label_seqs=label_seqs)
+            pcm = _tensors.to_device(x, torch.int16 if is_i16 else torch.float32, model.device)
+        if attention:
+            probs = model.run_mel(mel, lens=lens) if x.ndim == 3 else model(pcm)
+            dec_lens = None if lens is None else model.output_lengths(lens)
+        else:
+            state = torch.zeros((model.config.num_layers, B, model.config.hidden_size), dtype=torch.float32, device=model.device)
+            probs, _ = model.run_mel(mel, state, seq_len=lens) if x.ndim == 3 else model(pcm, state)
+            dec_lens = lens
+        miss, target, fa, _ = evaluate_softmax(probs, correctness, lens=dec_lens, label_seqs=label_seqs)
         res["miss"] += miss
         res["target"] += target
         res["false_accept"] += fa
