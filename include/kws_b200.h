@@ -146,6 +146,14 @@ int kws_model_reserve(kws_model* m, int64_t max_streams, int32_t max_frames);
 int kws_frontend_mel(kws_model* m, const void* pcm, int pcm_dtype, int64_t S, int64_t L,
                      int64_t ld_pcm, float* mel_out, void* stream);
 
+/* kws_frontend_mel over rows of their own lengths (kws_frontend_mel is this call with lengths = NULL).
+ * lengths: DEVICE int32 [S], valid samples per row, clamped to [0, L]; NULL = L for every row.  Row b has
+ * n_b = max(0, kws_num_frames(m, lengths[b])) frames; the row stride stays n = kws_num_frames(m, L).  No sample at or
+ * past lengths[b] is used (they are taken as zeros, as past the end of a row alone), so mel rows 0 .. n_b-1 are bit
+ * for bit those of kws_frontend_mel on pcm[b, :lengths[b]] alone; rows n_b .. n-1 are zero.                    */
+int kws_frontend_mel_lens(kws_model* m, const void* pcm, int pcm_dtype, int64_t S, int64_t L, int64_t ld_pcm,
+                          const int32_t* lengths, float* mel_out, void* stream);
+
 /* K2+K3 -- 2-layer TF-GRUCell recurrence with carried state, FC and softmax.
  * Replaces inference1 / inference2 / tf.nn.softmax (models/rnn_ctc.py:156-165,
  * 202-284).  The (mel frames, rnn_state) -> (softmax, rnn_state) form of the
@@ -164,6 +172,17 @@ int kws_gru_forward(kws_model* m, const float* mel, int64_t S, int32_t n,
 int kws_deploy_forward(kws_model* m, const void* pcm, int pcm_dtype, int64_t S, int64_t L,
                        int64_t ld_pcm, const float* state_in, float* probs_out,
                        float* state_out, float* logits_out, void* stream);
+
+/* kws_deploy_forward over rows of their own lengths (kws_deploy_forward is this call with lengths = NULL).
+ * lengths: DEVICE int32 [S], valid samples per row, clamped to [0, L]; NULL = L for every row.  L >= fft_size.
+ * Row b has n_b = max(0, kws_num_frames(m, lengths[b])) frames (computed on the device, never read on the host);
+ * probs / logits keep the row stride n = kws_num_frames(m, L).  For lengths[b] >= fft_size, rows < n_b of probs and
+ * logits and the row's state_out are bit for bit those of kws_deploy_forward on pcm[b, :lengths[b]] alone, for every
+ * precision, front end and the octbit graph (whose FC range covers the n_b valid frames).  Rows >= n_b are zero; a
+ * row with n_b = 0 has state_out = state_in.  No sample at or past lengths[b] is used (NaN there reaches nothing). */
+int kws_deploy_forward_lens(kws_model* m, const void* pcm, int pcm_dtype, int64_t S, int64_t L, int64_t ld_pcm,
+                            const int32_t* lengths, const float* state_in, float* probs_out, float* state_out,
+                            float* logits_out, void* stream);
 
 /* ----------------------------------------------------------------- decode
  * K4 -- batched CTC peak decoders + keyword test (utils/prediction.py:18-118).

@@ -94,10 +94,13 @@ _SIGNATURES = {
     "kws_num_frames": (c_int, [c_void_p, c_int64]),
     "kws_model_reserve": (c_int, [c_void_p, c_int64, c_int32]),
     "kws_frontend_mel": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_int64, c_void_p, c_void_p]),
+    "kws_frontend_mel_lens": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),
     "kws_gru_forward": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p,
                                 c_void_p, c_void_p, c_void_p]),
     "kws_deploy_forward": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_int64, c_void_p,
                                    c_void_p, c_void_p, c_void_p, c_void_p]),
+    "kws_deploy_forward_lens": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_int64, c_void_p, c_void_p,
+                                        c_void_p, c_void_p, c_void_p, c_void_p]),
     "kws_ctc_decode": (c_int, [c_void_p, c_int64, c_int32, c_int32, c_void_p, POINTER(DecodeParams),
                                c_char_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p]),
     "kws_edit_distance": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_int32, c_void_p, c_void_p]),

@@ -170,6 +170,11 @@ class AttentionDeployModel:
     def frames(self, T: int) -> int:
         return int(self._lib.kws_attention_frames(self._handle, int(T)))
 
+    def frame_counts(self, lengths):
+        """Mel frames of rows of ``lengths`` PCM samples (``DeployModel.frame_counts``), in the container type of
+        ``lengths``; ``output_lengths(frame_counts(lengths))`` are the decoder's ``lens`` for ``forward(lengths=)``."""
+        return self._frontend.frame_counts(lengths)
+
     def output_lengths(self, lens):
         """T'_b of utterances of ``lens`` valid mel frames, in the container type of ``lens`` (int, list, tuple, numpy
         or torch): the ``lens`` to give ``prediction.decode_batch`` / ``kws_ctc_decode`` for the posteriors of
@@ -230,25 +235,27 @@ class AttentionDeployModel:
     def forward(self, inputX, want_logits: bool = False, lengths=None):
         """PCM ``[L]`` or ``[B, L]`` (float scaled by 2^-15, or int16) -> softmax ``[B, T', C]``.
 
-        ``lengths [B]``: valid samples per row (fft_size <= lengths <= L); row b is then computed as a call on
-        ``inputX[b, :lengths[b]]`` alone, on its ``1 + (lengths[b] - fft_size) // hop_size`` frames (``run_mel``'s
-        ``lens``).  Those frames read no sample past lengths[b], so one front-end call on the padded batch serves.  The
-        front end's mel frames of a padded row may differ from those of the row alone in the last bits, so the result
-        matches a call on the row alone to within 1e-5, not bit for bit (``run_mel`` with ``lens`` is bit for bit)."""
+        ``lengths [B]`` (host or CUDA integers): valid samples per row.  Row b is then computed bit for bit as a call on
+        ``inputX[b, :lengths[b]]`` alone, on its ``frame_counts(lengths)[b]`` mel frames (``run_mel``'s ``lens``): the
+        front end (``kws_frontend_mel_lens``) reads no sample past lengths[b] and stages zeros there, as past the end of
+        the row alone.  Host lengths must lie in [fft_size, L]; CUDA lengths are not read on the host (no synchronisation):
+        the front end clamps them to [0, L] and the attention kernels the frame counts to [1, T]."""
         host = _tensors.is_host(inputX)
         lens = None
         if lengths is not None:
             shape = tuple(inputX.shape) if isinstance(inputX, torch.Tensor) else np.shape(inputX)
             B, L = (1, shape[0]) if len(shape) == 1 else shape[:2]
-            a = np.asarray(lengths.cpu().numpy() if isinstance(lengths, torch.Tensor) else lengths)
             c = self.config
-            if a.shape != (B,) or a.dtype.kind not in "iu":
-                raise _lib.InvalidArgumentError("lengths must be integers [%d], got %s %r" % (B, a.dtype, a.shape))
-            if B and (a.min() < c.fft_size or a.max() > L):
-                raise _lib.InvalidArgumentError("lengths must lie in [fft_size = %d, L = %d], got [%d, %d]"
-                                                % (c.fft_size, L, a.min(), a.max()))
-            lens = (1 + (a.astype(np.int64) - c.fft_size) // c.hop_size).astype(np.int32)
-        mel = self._frontend.frontend(inputX if not host else np.asarray(inputX))
+            if _tensors.is_host(lengths):
+                a = np.asarray(lengths.numpy() if isinstance(lengths, torch.Tensor) else lengths)
+                if a.shape != (B,) or a.dtype.kind not in "iu":
+                    raise _lib.InvalidArgumentError("lengths must be integers [%d], got %s %r" % (B, a.dtype, a.shape))
+                if B and (a.min() < c.fft_size or a.max() > L):
+                    raise _lib.InvalidArgumentError("lengths must lie in [fft_size = %d, L = %d], got [%d, %d]"
+                                                    % (c.fft_size, L, a.min(), a.max()))
+            lengths = self._frontend._check_lengths(lengths, B, L)            # int32 CUDA [B]
+            lens = self.frame_counts(lengths)
+        mel = self._frontend.frontend(inputX if not host else np.asarray(inputX), lengths=lengths)
         mel_dev = _tensors.to_device(mel, torch.float32, self.device)
         outs = self.run_mel(mel_dev, want_logits, lens=lens)
         if host:

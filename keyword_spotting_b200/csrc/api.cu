@@ -77,6 +77,7 @@ static void free_model(kws_model* m) {
   if (m->aux_stream) cudaStreamDestroy(m->aux_stream);
   cudaFree(m->scratch_mel);
   cudaFree(m->scratch_seq);
+  cudaFree(m->scratch_nfr);
   cudaFree(m->tc_xt);
   free_octbit(m);
   delete m;
@@ -228,7 +229,9 @@ extern "C" int kws_model_reserve(kws_model* m, int64_t max_streams, int32_t max_
   KWS_CUDA_OK(cudaDeviceSynchronize());      // nobody may still be using the old scratch
   cudaFree(m->scratch_mel);
   cudaFree(m->scratch_seq);
+  cudaFree(m->scratch_nfr);
   m->scratch_mel = m->scratch_seq = nullptr;
+  m->scratch_nfr = nullptr;
   m->cap_streams = 0;
   m->cap_frames = 0;
   const size_t mel_elems = mel_scratch_elems(S, n, m->cfg.n_mel);
@@ -236,9 +239,11 @@ extern "C" int kws_model_reserve(kws_model* m, int64_t max_streams, int32_t max_
   cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&m->scratch_mel), sizeof(float) * (mel_elems ? mel_elems : 1));
   if (e == cudaSuccess && m->cfg.num_layers > 1)
     e = cudaMalloc(reinterpret_cast<void**>(&m->scratch_seq), sizeof(float) * (seq_elems ? seq_elems : 1));
+  if (e == cudaSuccess) e = cudaMalloc(reinterpret_cast<void**>(&m->scratch_nfr), sizeof(int32_t) * (S > 0 ? S : 1));
   if (e != cudaSuccess) {
     cudaFree(m->scratch_mel);
-    m->scratch_mel = nullptr;
+    cudaFree(m->scratch_seq);
+    m->scratch_mel = m->scratch_seq = nullptr;
     return fail(KWS_ERR_ALLOC, "scratch allocation for %lld streams x %d frames failed: %s",
                 static_cast<long long>(S), n, cudaGetErrorString(e));
   }
@@ -258,6 +263,11 @@ static int check_pcm(const void* pcm, int dtype, int64_t S, int64_t L, int64_t l
 
 extern "C" int kws_frontend_mel(kws_model* m, const void* pcm, int pcm_dtype, int64_t S, int64_t L,
                                 int64_t ld_pcm, float* mel_out, void* stream) {
+  return kws_frontend_mel_lens(m, pcm, pcm_dtype, S, L, ld_pcm, nullptr, mel_out, stream);
+}
+
+extern "C" int kws_frontend_mel_lens(kws_model* m, const void* pcm, int pcm_dtype, int64_t S, int64_t L, int64_t ld_pcm,
+                                     const int32_t* lengths, float* mel_out, void* stream) {
   clear_error();
   KWS_REQUIRE(m != nullptr, "model is NULL");
   int rc = check_pcm(pcm, pcm_dtype, S, L, ld_pcm);
@@ -271,6 +281,7 @@ extern "C" int kws_frontend_mel(kws_model* m, const void* pcm, int pcm_dtype, in
   src.ld_body = ld_pcm;
   src.body_len = static_cast<int32_t>(L);
   src.body_dtype = pcm_dtype;
+  src.lengths = lengths;
   return launch_frontend(m, src, S, n, nullptr, mel_out, static_cast<cudaStream_t>(stream));
 }
 
@@ -299,9 +310,31 @@ extern "C" int kws_gru_forward(kws_model* m, const float* mel, int64_t S, int32_
   return launch_gru(m, a, static_cast<cudaStream_t>(stream));
 }
 
+namespace kws {
+// Rows t >= seq_len[s] of probs / logits [S, n, C] -> 0 (the recurrent kernels give them the dynamic_rnn value,
+// softmax of the bias).  One thread per (stream, frame).
+__global__ void zero_past_len_kernel(float* probs, float* logits, long S, int n, int C, const int32_t* seq_len) {
+  const long i = blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x;
+  if (i >= S * n) return;
+  const long s = i / n;
+  if (static_cast<int>(i - s * n) < __ldg(seq_len + s)) return;
+  for (int c = 0; c < C; ++c) {
+    probs[i * C + c] = 0.0f;
+    if (logits) logits[i * C + c] = 0.0f;
+  }
+}
+}  // namespace kws
+
 extern "C" int kws_deploy_forward(kws_model* m, const void* pcm, int pcm_dtype, int64_t S, int64_t L,
                                   int64_t ld_pcm, const float* state_in, float* probs_out, float* state_out,
                                   float* logits_out, void* stream) {
+  return kws_deploy_forward_lens(m, pcm, pcm_dtype, S, L, ld_pcm, nullptr, state_in, probs_out, state_out, logits_out,
+                                 stream);
+}
+
+extern "C" int kws_deploy_forward_lens(kws_model* m, const void* pcm, int pcm_dtype, int64_t S, int64_t L, int64_t ld_pcm,
+                                       const int32_t* lengths, const float* state_in, float* probs_out, float* state_out,
+                                       float* logits_out, void* stream) {
   clear_error();
   KWS_REQUIRE(m != nullptr, "model is NULL");
   int rc = check_pcm(pcm, pcm_dtype, S, L, ld_pcm);
@@ -318,10 +351,13 @@ extern "C" int kws_deploy_forward(kws_model* m, const void* pcm, int pcm_dtype, 
   src.ld_body = ld_pcm;
   src.body_len = static_cast<int32_t>(L);
   src.body_dtype = pcm_dtype;
+  src.lengths = lengths;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   KWS_CUDA_OK(cudaSetDevice(m->device));
   const bool tiled = mel_can_tile(m);
-  rc = launch_frontend(m, src, S, n, nullptr, m->scratch_mel, st, nullptr, tiled);
+  // with lengths, the front end writes every stream's frame count n_b: the recurrence's seq_len (never read on the host)
+  int32_t* nfr = lengths ? m->scratch_nfr : nullptr;
+  rc = launch_frontend(m, src, S, n, nullptr, m->scratch_mel, st, nullptr, tiled, nfr);
   if (rc != KWS_OK) return rc;
   KWS_REQUIRE(state_in && state_out && probs_out, "state / probs pointer is NULL");
   KWS_REQUIRE(reinterpret_cast<uintptr_t>(state_in) % 16 == 0 && reinterpret_cast<uintptr_t>(state_out) % 16 == 0,
@@ -331,9 +367,16 @@ extern "C" int kws_deploy_forward(kws_model* m, const void* pcm, int pcm_dtype, 
   a.x_tiled = tiled;
   a.S = S;
   a.n = n;
+  a.seq_len = nfr;
   a.state_in = state_in;
   a.state_out = state_out;
   a.probs = probs_out;
   a.logits = logits_out;
-  return launch_gru(m, a, st);
+  rc = launch_gru(m, a, st);
+  if (rc != KWS_OK || !lengths) return rc;
+  const long rows = static_cast<long>(S) * n;
+  zero_past_len_kernel<<<static_cast<unsigned>(ceil_div(rows, 256)), 256, 0, st>>>(probs_out, logits_out, S, n,
+                                                                                  m->cfg.num_classes, nfr);
+  KWS_LAUNCH_OK("zero_past_len_kernel");
+  return KWS_OK;
 }

@@ -138,6 +138,7 @@ struct kws_model {
   int32_t cap_frames = 0;
   float* scratch_mel = nullptr;   // [S, n, M]
   float* scratch_seq = nullptr;   // layer hand-off [tiles, n, H, 64]
+  int32_t* scratch_nfr = nullptr; // [S] frames per stream of a forward over streams of their own lengths
   // the octbit-rewritten graph (kws_model_set_octbit): per layer gates / candidate, and the FC
   bool octbit = false;
   kws::OctbitMatrix oct_gates[kws::kMaxLayers], oct_cand[kws::kMaxLayers], oct_fc;
@@ -162,6 +163,12 @@ struct PcmSource {
   const int16_t* head = nullptr;      // carried tail (server only), int16
   int64_t ld_head = 0;
   const int32_t* head_len = nullptr;  // [S] or null (= 0)
+  // [S] or null (= body_len): valid body samples per stream, clamped to [0, body_len].  Samples at or past it are never
+  // read and stage as zeros, so a stream of a padded batch is transformed exactly as the stream alone.
+  const int32_t* lengths = nullptr;
+  __device__ __forceinline__ int body_valid(long s) const {
+    return lengths ? min(max(__ldg(lengths + s), 0), body_len) : body_len;
+  }
 };
 
 // The streaming server's per-chunk pre-step, fused into the front end when the chunk fits one work item
@@ -181,7 +188,7 @@ bool frontend_uses_tc(const kws_model* m, int pcm_dtype);
 int default_frontend();           // KWS_FRONTEND=tc|fft in the environment, else fft
 int frontend_tc_item_frames();
 int launch_frontend_tc(const kws_model* m, const PcmSource& src, int64_t S, int32_t max_frames, const int32_t* nframes,
-                       float* mel_out, cudaStream_t st, const FrontendPre* pre, bool tiled_out);
+                       float* mel_out, cudaStream_t st, const FrontendPre* pre, bool tiled_out, int32_t* nframes_out);
 void build_mel_quads(const float* basis /*[201, M] host*/, int M, std::vector<MelQuad>* quads, int* quads_per_warp);
 // Stream-tiled mel scratch (front end -> tensor-core GRU, tc05.cuh "row-tiled A operand"): the fp16 MMA operand of
 // layer 0, [S/128 tiles][n frames][x_hi chunks | x_lo chunks][128 streams][8 mels]; chunk c holds mels 8c..8c+7 (zero
@@ -203,9 +210,11 @@ inline int mel_tile_chunks(const kws_model* m) { return m->layer[0].tc_kx / 8; }
 inline bool mel_tile_split(const kws_model* m) { return m->layer[0].tc_kxw != m->layer[0].tc_kx; }
 bool gru_tc_can_split(int in_dim, bool last, int device);                // gru_tc.cu
 bool gru_tc_layer_fits(int in_dim, bool split, bool last, int device);
+// With src.lengths, frames of a stream past its own length are zero rows of mel_out, and nframes_out (if not null)
+// receives every stream's frame count: the seq_len of the recurrent kernels.
 int launch_frontend(const kws_model* m, const PcmSource& src, int64_t S, int32_t max_frames,
                     const int32_t* nframes /*[S] or null*/, float* mel_out, cudaStream_t st,
-                    const FrontendPre* pre = nullptr, bool tiled_out = false);
+                    const FrontendPre* pre = nullptr, bool tiled_out = false, int32_t* nframes_out = nullptr);
 
 struct GruArgs {
   const float* x = nullptr;       // layer-0 input [S, n, M] row-major, or stream-tiled when x_tiled

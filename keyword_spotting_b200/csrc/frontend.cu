@@ -82,7 +82,7 @@ struct FrontendParams {
   int16_t* tail_next;       // [S, 400]
   int* len_next;            // [S]
   unsigned char* silence;   // [S]
-  int* nframes_out;         // [S]
+  int* nframes_out;         // [S] frames per stream (fused pre-step, or a forward over streams of their own lengths)
 };
 
 // Transposed magnitudes: bin k of frame slot sl sits at (k/2)*66 + 2*sl + (k&1), so the mel projection (lane = slot)
@@ -104,7 +104,10 @@ __device__ __forceinline__ float4 quad_to_float(uint2 q) {
                      static_cast<float>(static_cast<short>(q.y & 0xffffu)), static_cast<float>(static_cast<short>(q.y >> 16)));
 }
 
-template <bool kQuadsInSmem>
+// kLens: the streams have lengths of their own (p.src.lengths): zero-fill past each length, skip items past each stream's
+// last frame, write the frame counts.  Without them none of that is compiled in (the streaming server's path, and every
+// equal-length forward).
+template <bool kQuadsInSmem, bool kLens>
 __global__ void __launch_bounds__(kFeThreads, 2)
 frontend_kernel(const FrontendParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -136,6 +139,8 @@ frontend_kernel(const FrontendParams p) {
     if (items32) return static_cast<long>(static_cast<unsigned>(item) / static_cast<unsigned>(p.groups));
     return item / p.groups;
   };
+  // frames of a signal of tl samples (utils/stft.py:60-61), 0 below one frame
+  auto frames_of = [](int tl) -> int { return tl >= kFft ? 1 + (tl - kFft) / kHop : 0; };
   const bool i16 = p.src.body_dtype == KWS_PCM_I16;
   const int M = p.n_mel;
   const int Mp = M | 1;                               // odd row stride of the [32][M] output tile: conflict-free band writes
@@ -150,13 +155,22 @@ frontend_kernel(const FrontendParams p) {
   const bool last_quad_ok = tid < kFeLastQuads;
   auto load_quads = [&](long item, int head_len, uint2 (&pre)[kFeQuadRounds]) {
     const long s = stream_of(item);
-    const int q0 = static_cast<int>(item - s * p.groups) * kFeItemHop;
-    const int total_len = head_len + p.src.body_len;
+    const int g = static_cast<int>(item - s * p.groups);
+    const int q0 = g * kFeItemHop;
+    const int full_len = head_len + p.src.body_len;
+    const int total_len = kLens ? head_len + p.src.body_valid(s) : full_len;   // samples past the length stage as zeros
     // both pointers are indexed by the stream sample number
     const int16_t* body = static_cast<const int16_t*>(p.src.body) + s * p.src.ld_body - head_len;
     const int16_t* head = p.src.head + s * p.src.ld_head;             // only dereferenced below head_len
-    if (p.vec_ok && ((head_len | total_len) & 3) == 0) {
+    if (kLens && g * kFeItemFrames >= frames_of(total_len)) {
+      // an item past the stream's last frame loads nothing (the loop below writes its zero rows)
+#pragma unroll
+      for (int r = 0; r < kFeQuadRounds; ++r) pre[r] = make_uint2(0u, 0u);
+      return;
+    }
+    if (p.vec_ok && ((head_len | full_len) & 3) == 0) {
       // every quad lies entirely in the carried tail, in the chunk, or beyond the signal: one predicated 8-byte load
+      // (with lengths, the one quad that straddles a stream's length is masked when it is stored: store_quads)
 #pragma unroll
       for (int r = 0; r < kFeQuadRounds; ++r) {
         const int q = q0 + 4 * tid + 4 * kFeThreads * r;
@@ -193,11 +207,17 @@ frontend_kernel(const FrontendParams p) {
   float* my_stage = win + 4 * tid + kFeSkew * (tid / (kFeBlock / 4));
   // returns the thread's sum of |x| over the NEW samples (detector.py:168), exact in fp32 (<= 20 * 32768); samples
   // beyond the signal were loaded as zeros
-  auto store_quads = [&](int q0, int head_len, const uint2 (&pre)[kFeQuadRounds]) {
+  auto store_quads = [&](int q0, int head_len, int total_len, const uint2 (&pre)[kFeQuadRounds]) {
     float4 f[kFeQuadRounds];
 #pragma unroll
     for (int r = 0; r < kFeQuadRounds; ++r) {
       f[r] = quad_to_float(pre[r]);
+      if (kLens) {                                    // the quad that straddles the stream's length: zeros past it
+        const int q = q0 + 4 * tid + 4 * kFeThreads * r;
+        if (q + 1 >= total_len) f[r].y = 0.0f;
+        if (q + 2 >= total_len) f[r].z = 0.0f;
+        if (q + 3 >= total_len) f[r].w = 0.0f;
+      }
       if (r < kFeQuadRounds - 1 || last_quad_ok) *reinterpret_cast<float4*>(my_stage + (4 * kFeThreads + 4 * kFeSkew) * r) = f[r];
     }
     if (!p.fuse_pre) return 0;
@@ -212,6 +232,20 @@ frontend_kernel(const FrontendParams p) {
     return static_cast<int>(acc);
   };
 
+  // frames [fa, fb) of stream s in mel_out (either layout) -> zero: the rows past a stream's length
+  auto zero_rows = [&](long s, int fa, int fb) {
+    if (fb > p.max_frames) fb = p.max_frames;
+    if (fa >= fb) return;
+    if (p.tiled_out) {
+      const int per_frame = p.tile_split ? 2 * p.tile_chunks : p.tile_chunks;
+      uint4* dst = reinterpret_cast<uint4*>(p.mel_out) + ((s >> 7) * p.max_frames + fa) * static_cast<long>(per_frame) * 128 + (s & 127);
+      for (int i = tid; i < (fb - fa) * per_frame; i += kFeThreads) dst[static_cast<long>(i) * 128] = make_uint4(0u, 0u, 0u, 0u);
+    } else {
+      float* dst = p.mel_out + (s * p.max_frames + fa) * static_cast<long>(M);
+      for (int i = tid; i < (fb - fa) * M; i += kFeThreads) dst[i] = 0.0f;
+    }
+  };
+
   long item = blockIdx.x;
   uint2 pre[kFeQuadRounds];
   int head_len = 0;
@@ -224,8 +258,8 @@ frontend_kernel(const FrontendParams p) {
     const long s = stream_of(item);
     const int g = static_cast<int>(item - s * p.groups);
     if (!i16) head_len = p.src.head_len ? p.src.head_len[s] : 0;
-    const int total_len = head_len + p.src.body_len;
-    const int nfr_sig = total_len >= kFft ? 1 + (total_len - kFft) / kHop : 0;
+    const int total_len = head_len + (kLens ? p.src.body_valid(s) : p.src.body_len);
+    const int nfr_sig = frames_of(total_len);
     int nfr = p.fuse_pre ? nfr_sig : (p.nframes ? p.nframes[s] : nfr_sig);
     if (nfr > p.max_frames) nfr = p.max_frames;
     const int q0 = g * kFeItemHop;                    // stream sample held at window position 0
@@ -234,13 +268,23 @@ frontend_kernel(const FrontendParams p) {
     const long next = item + gridDim.x;
     int head_len_next = 0;
     if (i16 && next < items && p.src.head_len) head_len_next = p.src.head_len[stream_of(next)];
+    if (kLens && p.nframes_out && g == 0 && tid == 0) p.nframes_out[s] = nfr;
+    if (kLens && f0 >= nfr) {
+      // the item starts past the stream's last frame: zero rows and no PCM (load_quads loaded none), no barrier needed --
+      // the next item's staging writes only the window region, whose last reads precede this item
+      if (i16 && next < items) load_quads(next, head_len_next, pre);
+      zero_rows(s, f0, f0 + kFeItemFrames);
+      head_len = head_len_next;
+      continue;
+    }
 
     // ---- stage the window: stream samples [q0, q0 + 5360) -> win[i + 20*(i/320)], zero beyond the signal.
     int vad_acc = 0;
     if (i16) {
-      vad_acc = store_quads(q0, head_len, pre);
+      vad_acc = store_quads(q0, head_len, total_len, pre);
     } else {
-      // fp32 PCM: thread t takes samples t + 320*r, so the skewed position is simply t + 340*r
+      // fp32 PCM: thread t takes samples t + 320*r, so the skewed position is simply t + 340*r; samples past the
+      // stream's length are zeros (never read)
       const bool last_ok = tid < kFeWinSamples - kFeBlock * (kFeWinRounds - 1);   // the 17th round is partial
       const float* body = static_cast<const float*>(p.src.body) + s * p.src.ld_body + q0 + tid;
 #pragma unroll
@@ -391,6 +435,7 @@ frontend_kernel(const FrontendParams p) {
           dst[i] = out_tile[f * Mp + (i - f * M)];
         }
       }
+      if (kLens) zero_rows(s, f0 + nfi, f0 + kFeItemFrames);   // the item's frames past the stream's length
     }
     head_len = head_len_next;
   }
@@ -459,10 +504,12 @@ bool frontend_can_fuse_pre(const kws_model* m, int chunk_len, int tail_cap) {
 }
 
 int launch_frontend(const kws_model* m, const PcmSource& src, int64_t S, int32_t max_frames,
-                    const int32_t* nframes, float* mel_out, cudaStream_t st, const FrontendPre* pre, bool tiled_out) {
+                    const int32_t* nframes, float* mel_out, cudaStream_t st, const FrontendPre* pre, bool tiled_out,
+                    int32_t* nframes_out) {
   if (S <= 0) return KWS_OK;
   if (max_frames <= 0 && !pre) return KWS_OK;
-  if (frontend_uses_tc(m, src.body_dtype)) return launch_frontend_tc(m, src, S, max_frames, nframes, mel_out, st, pre, tiled_out);
+  if (frontend_uses_tc(m, src.body_dtype))
+    return launch_frontend_tc(m, src, S, max_frames, nframes, mel_out, st, pre, tiled_out, nframes_out);
   FrontendParams p;
   p.src = src;
   p.S = S;
@@ -487,7 +534,7 @@ int launch_frontend(const kws_model* m, const PcmSource& src, int64_t S, int32_t
   p.tail_next = nullptr;
   p.len_next = nullptr;
   p.silence = nullptr;
-  p.nframes_out = nullptr;
+  p.nframes_out = nframes_out;
   if (pre) {
     if (p.groups != 1 || src.body_dtype != KWS_PCM_I16)
       return fail(KWS_ERR_INVALID_ARGUMENT, "fused pre-step needs an int16 chunk that fits one work item");
@@ -498,8 +545,10 @@ int launch_frontend(const kws_model* m, const PcmSource& src, int64_t S, int32_t
     p.silence = pre->silence;
     p.nframes_out = pre->nframes_out;
   }
-  const bool in_smem = quads_in_smem(m);
-  auto kernel = in_smem ? frontend_kernel<true> : frontend_kernel<false>;
+  const bool in_smem = quads_in_smem(m), lens = src.lengths != nullptr;
+  if (lens && pre) return fail(KWS_ERR_INVALID_ARGUMENT, "the fused pre-step takes no stream lengths");
+  auto kernel = in_smem ? (lens ? frontend_kernel<true, true> : frontend_kernel<true, false>)
+                        : (lens ? frontend_kernel<false, true> : frontend_kernel<false, false>);
   const size_t smem = frontend_smem_bytes(m);
   // the attribute is per device: set it on every launch (a few hundred ns), never cached per thread
   KWS_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));

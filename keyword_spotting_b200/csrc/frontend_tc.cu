@@ -145,6 +145,12 @@ __device__ __forceinline__ float ft_sqrt(float x) {
   return y;
 }
 
+// frames of a signal of tl samples (utils/stft.py:60-61), 0 below one frame
+__device__ __forceinline__ int ft_frames_of(int tl) { return tl >= kFft ? 1 + (tl - kFft) / kHop : 0; }
+
+// kLens: the streams have lengths of their own (p.src.lengths), as in frontend_kernel (frontend.cu); without them none of
+// their handling is compiled in.
+template <bool kLens>
 __global__ void __launch_bounds__(kFtThreads, 1)
 frontend_tc_kernel(const FrontendTcParams p) {
   extern __shared__ __align__(128) unsigned char smem[];
@@ -269,7 +275,10 @@ frontend_tc_kernel(const FrontendTcParams p) {
       const int g = static_cast<int>(item - s * p.groups);
       const int buf = static_cast<int>(i & 1);
       const int head_len = p.src.head_len ? p.src.head_len[s] : 0;
-      const int total_len = head_len + p.src.body_len;
+      const int total_len = head_len + (kLens ? p.src.body_valid(s) : p.src.body_len);
+      // samples staged from PCM: none for an item past the stream's last frame (its rows are zeros), otherwise those
+      // below the stream's length -- the piece that straddles it goes element by element, the rest stage as zeros
+      const int ld_len = kLens && g * kFtFrames >= ft_frames_of(total_len) ? 0 : total_len;
       const int q0 = g * kFtItemHop;
       const int16_t* body = static_cast<const int16_t*>(p.src.body) + s * p.src.ld_body - head_len;   // indexed by stream sample
       const int16_t* head = p.src.head ? p.src.head + s * p.src.ld_head : nullptr;
@@ -289,7 +298,7 @@ frontend_tc_kernel(const FrontendTcParams p) {
         const int pc = ltid + kFtLoadThreads * rd;
         const int q = q0 + 8 * pc;
         pre[rd] = make_uint4(0u, 0u, 0u, 0u);
-        if (pc < n_pieces && fast && q + 8 <= total_len)
+        if (pc < n_pieces && fast && q + 8 <= ld_len)
           pre[rd] = __ldg(reinterpret_cast<const uint4*>((q < head_len ? head : body) + q));
       }
       if (i >= 2) ft_wait_hint(&bars[kFbBempty0 + buf], static_cast<uint32_t>(((i >> 1) + 1) & 1), 200);
@@ -302,13 +311,13 @@ frontend_tc_kernel(const FrontendTcParams p) {
         if (pc >= n_pieces) break;
         const int q = q0 + 8 * pc;
         uint4 v = pre[rd];
-        if (q < total_len && !(fast && q + 8 <= total_len)) {             // unaligned rows / the ragged end: element by element
+        if (q < ld_len && !(fast && q + 8 <= ld_len)) {                   // unaligned rows / the ragged end: element by element
           unsigned e[8];
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
             int x = 0;
             if (q + j < head_len) x = head[q + j];
-            else if (q + j < total_len) x = body[q + j];
+            else if (q + j < ld_len) x = body[q + j];
             e[j] = static_cast<unsigned>(x) & 0xffffu;
           }
           v = make_uint4(e[0] | (e[1] << 16), e[2] | (e[3] << 16), e[4] | (e[5] << 16), e[6] | (e[7] << 16));
@@ -390,13 +399,14 @@ frontend_tc_kernel(const FrontendTcParams p) {
       const int g = static_cast<int>(item - s * p.groups);
       const int buf = static_cast<int>(i & 1);
       const int head_len = p.src.head_len ? p.src.head_len[s] : 0;
-      const int total_len = head_len + p.src.body_len;
-      const int nfr_sig = total_len >= kFft ? 1 + (total_len - kFft) / kHop : 0;
+      const int total_len = head_len + (kLens ? p.src.body_valid(s) : p.src.body_len);
+      const int nfr_sig = ft_frames_of(total_len);
       int nfr = p.fuse_pre ? nfr_sig : (p.nframes ? p.nframes[s] : nfr_sig);
       if (nfr > p.max_frames) nfr = p.max_frames;
       const int f0 = g * kFtFrames;
       int nfi = nfr - f0;
       nfi = nfi < 0 ? 0 : (nfi > kFtFrames ? kFtFrames : nfi);
+      if (kLens && p.nframes_out && g == 0 && otid == 0) p.nframes_out[s] = nfr;
       ft_wait_hint(&bars[kFbMagFull0 + buf], static_cast<uint32_t>((i >> 1) & 1), 200);
       // bands q, q+8, ...: eight bins per trip (spans are zero-padded to multiples of 8): the eight magnitude loads
       // (32 consecutive floats each) and the two broadcast weight loads are independent, four accumulators
@@ -459,6 +469,17 @@ frontend_tc_kernel(const FrontendTcParams p) {
         for (int idx = otid; idx < total; idx += kFtOutThreads) {
           const int f = idx / M;
           dst[idx] = sOut[f * kFtOutStride + (idx - f * M)];
+        }
+      }
+      if (kLens) {                                   // the item's frames past the stream's length are zero rows
+        const int fa = f0 + nfi, fb = f0 + kFtFrames < p.max_frames ? f0 + kFtFrames : p.max_frames;
+        if (p.tiled_out) {
+          const int per_frame = p.tile_split ? 2 * p.tile_chunks : p.tile_chunks;
+          uint4* dst = reinterpret_cast<uint4*>(p.mel_out) + ((s >> 7) * p.max_frames + fa) * static_cast<long>(per_frame) * 128 + (s & 127);
+          for (int idx = otid; idx < (fb - fa) * per_frame; idx += kFtOutThreads) dst[static_cast<long>(idx) * 128] = make_uint4(0u, 0u, 0u, 0u);
+        } else {
+          float* dst = p.mel_out + (s * p.max_frames + fa) * static_cast<long>(M);
+          for (int idx = otid; idx < (fb - fa) * M; idx += kFtOutThreads) dst[idx] = 0.0f;
         }
       }
       asm volatile("bar.sync 3, 256;" ::: "memory");
@@ -638,7 +659,7 @@ int default_frontend() {
 int frontend_tc_item_frames() { return kFtFrames; }
 
 int launch_frontend_tc(const kws_model* m, const PcmSource& src, int64_t S, int32_t max_frames, const int32_t* nframes,
-                       float* mel_out, cudaStream_t st, const FrontendPre* pre, bool tiled_out) {
+                       float* mel_out, cudaStream_t st, const FrontendPre* pre, bool tiled_out, int32_t* nframes_out) {
   FrontendTcParams p;
   p.src = src;
   p.S = S;
@@ -663,7 +684,7 @@ int launch_frontend_tc(const kws_model* m, const PcmSource& src, int64_t S, int3
   p.tail_next = nullptr;
   p.len_next = nullptr;
   p.silence = nullptr;
-  p.nframes_out = nullptr;
+  p.nframes_out = nframes_out;
   if (pre) {
     if (p.groups != 1) return fail(KWS_ERR_INVALID_ARGUMENT, "fused pre-step needs a chunk that fits one work item");
     p.fuse_pre = 1;
@@ -687,11 +708,13 @@ int launch_frontend_tc(const kws_model* m, const PcmSource& src, int64_t S, int3
     for (int i = 0; i < 256; ++i) dbg_host[i] = 0;
     p.dbg = dbg_dev;
   }
+  if (src.lengths && pre) return fail(KWS_ERR_INVALID_ARGUMENT, "the fused pre-step takes no stream lengths");
+  auto kernel = src.lengths ? frontend_tc_kernel<true> : frontend_tc_kernel<false>;
   const size_t smem = frontend_tc_smem_bytes(p.mel_nw);
-  KWS_CUDA_OK(cudaFuncSetAttribute(frontend_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  KWS_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   const long items = S * p.groups;
   const long blocks = items < sm_count() ? items : sm_count();
-  frontend_tc_kernel<<<static_cast<unsigned>(blocks), kFtThreads, smem, st>>>(p);
+  kernel<<<static_cast<unsigned>(blocks), kFtThreads, smem, st>>>(p);
   if (dbg_on) {
     const cudaError_t e = cudaStreamSynchronize(st);
     fprintf(stderr, "[frontend_tc] S=%ld groups=%d sync=%s markers:", static_cast<long>(S), p.groups, cudaGetErrorString(e));

@@ -55,13 +55,16 @@ def evaluate_softmax(softmax, correctness, lens=None, label_seqs: str = "1233", 
     return miss, int(tgt.sum()), false_accept, trig_t.cpu().numpy()
 
 
-def validate(model, batches: Iterable[Tuple], label_seqs: Optional[str] = None) -> ValidationResult:
+def validate(model, batches: Iterable[Tuple], label_seqs: Optional[str] = None,
+             sample_lengths: bool = False) -> ValidationResult:
     """Run the validation set through ``model`` (a DeployModel or an AttentionDeployModel).
 
     ``batches`` yields ``(inputs, lens, correctness)``: inputs are mel frames ``[B, T, n_mel]`` (the valid
     queue's form, reader.py:282-305) or PCM ``[B, L]``; ``lens`` valid frames per utterance (or None).
-    PCM rows are taken as equal-length utterances.  For the attention model ``lens`` are mel frames: mel batches run
-    with them, and the decoder takes the model's ``output_lengths(lens)``.
+    By default PCM rows are taken as equal-length utterances.  With ``sample_lengths``, the ``lens`` of PCM batches are
+    valid samples per utterance: each model runs ``forward(..., lengths=lens)``, and the decoder takes its frame counts
+    (``frame_counts(lens)``; ``output_lengths`` of those for the attention model).  For the attention model the
+    ``lens`` of mel batches are mel frames: they run with them, and the decoder takes ``output_lengths(lens)``.
     """
     from .attention_ctc import AttentionDeployModel
     label_seqs = label_seqs or model.config.label_seqs
@@ -75,13 +78,21 @@ def validate(model, batches: Iterable[Tuple], label_seqs: Optional[str] = None) 
         else:
             is_i16 = x.dtype in (np.int16, torch.int16)
             pcm = _tensors.to_device(x, torch.int16 if is_i16 else torch.float32, model.device)
-        if attention:
+        by_samples = sample_lengths and x.ndim != 3 and lens is not None
+        if attention and by_samples:
+            probs = model(pcm, lengths=lens)
+            dec_lens = model.output_lengths(model.frame_counts(lens))
+        elif attention:
             probs = model.run_mel(mel, lens=lens) if x.ndim == 3 else model(pcm)
             dec_lens = None if lens is None else model.output_lengths(lens)
         else:
             state = torch.zeros((model.config.num_layers, B, model.config.hidden_size), dtype=torch.float32, device=model.device)
-            probs, _ = model.run_mel(mel, state, seq_len=lens) if x.ndim == 3 else model(pcm, state)
-            dec_lens = lens
+            if by_samples:
+                probs, _ = model(pcm, state, lengths=lens)
+                dec_lens = model.frame_counts(lens)
+            else:
+                probs, _ = model.run_mel(mel, state, seq_len=lens) if x.ndim == 3 else model(pcm, state)
+                dec_lens = lens
         miss, target, fa, _ = evaluate_softmax(probs, correctness, lens=dec_lens, label_seqs=label_seqs)
         res["miss"] += miss
         res["target"] += target

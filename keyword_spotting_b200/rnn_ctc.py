@@ -276,8 +276,42 @@ class DeployModel:
             raise _lib.InvalidArgumentError("rnn_initial_states must be [%d, %d, %d], got %r" % (L, S, H, tuple(st.shape)))
         return st
 
-    def forward(self, inputX, rnn_initial_states, want_logits: bool = False):
-        """(pcm, rnn_state) -> (softmax [S,n,C], rnn_state [L,S,H] [, logits])."""
+    def frame_counts(self, lengths):
+        """n_b = max(0, 1 + floor((lengths - fft_size) / hop_size)) frames of rows of ``lengths`` samples, in the
+        container type of ``lengths`` (int, list, tuple, numpy or torch): the ``lens`` to give
+        ``prediction.decode_batch`` / ``kws_ctc_decode`` for the posteriors of ``forward(pcm, state, lengths=lengths)``."""
+        fft, hop = self.config.fft_size, self.config.hop_size
+        if isinstance(lengths, torch.Tensor):
+            return torch.clamp((lengths - fft) // hop + 1, min=0)
+        if isinstance(lengths, np.ndarray):
+            return np.maximum((lengths - fft) // hop + 1, 0)
+        rule = lambda n: max(0, (int(n) - fft) // hop + 1)
+        if isinstance(lengths, (list, tuple)):
+            return type(lengths)(rule(n) for n in lengths)
+        return rule(lengths)
+
+    def _check_lengths(self, lengths, S: int, L: int):
+        """lengths -> int32 CUDA [S].  Host values are validated (0 <= lengths <= L); CUDA values are left to the
+        kernels, which clamp them to [0, L] (reading them here would synchronise the stream)."""
+        if not _tensors.is_host(lengths):
+            if tuple(lengths.shape) != (S,) or lengths.dtype.is_floating_point or lengths.dtype == torch.bool:
+                raise _lib.InvalidArgumentError("lengths must be integers [%d], got %s %r"
+                                                % (S, lengths.dtype, tuple(lengths.shape)))
+            return _tensors.to_device(lengths, torch.int32, self.device)
+        a = np.asarray(lengths.numpy() if isinstance(lengths, torch.Tensor) else lengths)
+        if a.shape != (S,) or a.dtype.kind not in "iu":
+            raise _lib.InvalidArgumentError("lengths must be integers [%d], got %s %r" % (S, a.dtype, a.shape))
+        if S and (a.min() < 0 or a.max() > L):
+            raise _lib.InvalidArgumentError("lengths must lie in [0, L = %d], got [%d, %d]" % (L, a.min(), a.max()))
+        return _tensors.to_device(a.astype(np.int32), torch.int32, self.device)
+
+    def forward(self, inputX, rnn_initial_states, want_logits: bool = False, lengths=None):
+        """(pcm, rnn_state) -> (softmax [S,n,C], rnn_state [L,S,H] [, logits]).
+
+        ``lengths [S]`` (host or CUDA integers): valid samples per row.  Row b is then computed as a call on
+        ``inputX[b, :lengths[b]]`` alone, bit for bit, on its ``frame_counts(lengths)[b]`` frames: no sample past
+        lengths[b] is read, its rows from there on are zero, and its state is the one after its own last frame (the
+        incoming state for a row shorter than one frame).  Host lengths must lie in [0, L]."""
         host = _tensors.is_host(inputX)
         pcm = inputX
         is_i16 = (isinstance(pcm, torch.Tensor) and pcm.dtype == torch.int16) or \
@@ -290,15 +324,16 @@ class DeployModel:
             raise _lib.InvalidArgumentError("inputX must be [L] or [S, L]")
         S, Lsig = x.shape
         st_in = self._prep_state(rnn_initial_states, S)
+        ln = None if lengths is None else self._check_lengths(lengths, S, Lsig)
         n = self.num_frames(Lsig)
         C = self.config.num_classes
         probs = torch.empty((S, max(n, 0), C), dtype=torch.float32, device=self.device)
         logits = torch.empty_like(probs) if want_logits else None
         st_out = torch.empty_like(st_in)
         with torch.cuda.device(self.device):
-            _lib.check(self._lib.kws_deploy_forward(
+            _lib.check(self._lib.kws_deploy_forward_lens(
                 self._handle, _tensors.ptr(x), _lib.PCM_I16 if is_i16 else _lib.PCM_F32, S, Lsig, x.stride(0) if S > 1 else Lsig,
-                _tensors.ptr(st_in), _tensors.ptr(probs), _tensors.ptr(st_out), _tensors.ptr(logits),
+                _tensors.ptr(ln), _tensors.ptr(st_in), _tensors.ptr(probs), _tensors.ptr(st_out), _tensors.ptr(logits),
                 _tensors.stream_ptr(self.device)))
         outs = [probs, st_out] + ([logits] if want_logits else [])
         if host:
@@ -308,21 +343,27 @@ class DeployModel:
 
     __call__ = forward
 
-    def frontend(self, inputX):
-        """PCM -> mel frames ``[S, n, M]`` (K1 alone)."""
+    def frontend(self, inputX, lengths=None):
+        """PCM -> mel frames ``[S, n, M]`` (K1 alone).
+
+        ``lengths [S]`` (host or CUDA integers, host values in [0, L]): valid samples per row; rows
+        ``< frame_counts(lengths)[b]`` are bit for bit those of ``frontend(inputX[b, :lengths[b]])``, the rest zero."""
         host = _tensors.is_host(inputX)
         is_i16 = (isinstance(inputX, torch.Tensor) and inputX.dtype == torch.int16) or \
                  (not isinstance(inputX, torch.Tensor) and np.asarray(inputX).dtype == np.int16)
         x = _tensors.to_device(inputX, torch.int16 if is_i16 else torch.float32, self.device)
         if x.dim() == 1:
             x = x.unsqueeze(0)
+        if x.dim() != 2:
+            raise _lib.InvalidArgumentError("inputX must be [L] or [S, L]")
         S, Lsig = x.shape
+        ln = None if lengths is None else self._check_lengths(lengths, S, Lsig)
         n = max(self.num_frames(Lsig), 0)
         mel = torch.empty((S, n, self.config.n_mel), dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
-            _lib.check(self._lib.kws_frontend_mel(self._handle, _tensors.ptr(x), _lib.PCM_I16 if is_i16 else _lib.PCM_F32,
-                                                  S, Lsig, x.stride(0) if S > 1 else Lsig, _tensors.ptr(mel),
-                                                  _tensors.stream_ptr(self.device)))
+            _lib.check(self._lib.kws_frontend_mel_lens(self._handle, _tensors.ptr(x), _lib.PCM_I16 if is_i16 else _lib.PCM_F32,
+                                                       S, Lsig, x.stride(0) if S > 1 else Lsig, _tensors.ptr(ln),
+                                                       _tensors.ptr(mel), _tensors.stream_ptr(self.device)))
         if host:
             torch.cuda.current_stream(self.device).synchronize()
             return _tensors.to_host(mel)
