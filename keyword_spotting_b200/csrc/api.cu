@@ -282,7 +282,7 @@ extern "C" int kws_frontend_mel_lens(kws_model* m, const void* pcm, int pcm_dtyp
   src.body_len = static_cast<int32_t>(L);
   src.body_dtype = pcm_dtype;
   src.lengths = lengths;
-  return launch_frontend(m, src, S, n, nullptr, mel_out, static_cast<cudaStream_t>(stream));
+  return launch_frontend(m, src, S, n, mel_out, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int kws_gru_forward(kws_model* m, const float* mel, int64_t S, int32_t n, const int32_t* seq_len,
@@ -357,7 +357,7 @@ extern "C" int kws_deploy_forward_lens(kws_model* m, const void* pcm, int pcm_dt
   const bool tiled = mel_can_tile(m);
   // with lengths, the front end writes every stream's frame count n_b: the recurrence's seq_len (never read on the host)
   int32_t* nfr = lengths ? m->scratch_nfr : nullptr;
-  rc = launch_frontend(m, src, S, n, nullptr, m->scratch_mel, st, nullptr, tiled, nfr);
+  rc = launch_frontend(m, src, S, n, m->scratch_mel, st, nullptr, tiled, nfr);
   if (rc != KWS_OK) return rc;
   KWS_REQUIRE(state_in && state_out && probs_out, "state / probs pointer is NULL");
   KWS_REQUIRE(reinterpret_cast<uintptr_t>(state_in) % 16 == 0 && reinterpret_cast<uintptr_t>(state_out) % 16 == 0,

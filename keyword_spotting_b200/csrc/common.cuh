@@ -171,15 +171,29 @@ struct PcmSource {
   }
 };
 
-// The streaming server's per-chunk pre-step, fused into the front end when the chunk fits one work item
-// (frontend_can_fuse_pre): VAD flag, frame count and next carried tail are produced by the same CTA that
-// stages the chunk, so the PCM is read once.
+// Chunk rules of the front end and the streaming server.  Frames of a signal of `total` samples (utils/stft.py:60-61),
+// 0 below one frame:
+__host__ __device__ __forceinline__ int frames_of(int total) { return total >= kFft ? 1 + (total - kFft) / kHop : 0; }
+// samples carried into the next chunk (detector.py:181-182): the last (total - 400) % 160 + 240, or all of them while
+// no frame fits
+__host__ __device__ __forceinline__ int tail_keep(int total) {
+  return total >= kFft ? (total - kFft) % kHop + (kFft - kHop) : total;
+}
+
+// The streaming server's per-chunk pre-step: VAD flag, frame count and next carried tail.  Fused into the front end
+// when the chunk fits one work item (frontend_can_fuse_pre), so that the CTA that stages the chunk produces them and
+// the PCM is read once; stream_pre_kernel (stream.cu) otherwise.
 struct FrontendPre {
   long long vad_limit = 0;            // speech iff sum|x_i16| > vad_limit
   int16_t* tail_next = nullptr;       // [S, 400]
   int32_t* len_next = nullptr;        // [S]
   unsigned char* silence = nullptr;   // [S]
-  int32_t* nframes_out = nullptr;     // [S]
+  // stream s's record, from the sum of |x_i16| over its new samples; its frame count goes to nframes[s]
+  __device__ __forceinline__ void record(long s, long long vad_sum, int frames, int keep, int32_t* nframes) const {
+    silence[s] = vad_sum > vad_limit ? 0 : 1;
+    nframes[s] = frames;
+    len_next[s] = keep;
+  }
 };
 bool frontend_can_fuse_pre(const kws_model* m, int chunk_len, int tail_cap);
 int build_frontend_tc_tables(kws_model* m, const float* basis /*[201, M] host*/);
@@ -187,8 +201,6 @@ void free_frontend_tc_tables(kws_model* m);
 bool frontend_uses_tc(const kws_model* m, int pcm_dtype);
 int default_frontend();           // KWS_FRONTEND=tc|fft in the environment, else fft
 int frontend_tc_item_frames();
-int launch_frontend_tc(const kws_model* m, const PcmSource& src, int64_t S, int32_t max_frames, const int32_t* nframes,
-                       float* mel_out, cudaStream_t st, const FrontendPre* pre, bool tiled_out, int32_t* nframes_out);
 void build_mel_quads(const float* basis /*[201, M] host*/, int M, std::vector<MelQuad>* quads, int* quads_per_warp);
 // Stream-tiled mel scratch (front end -> tensor-core GRU, tc05.cuh "row-tiled A operand"): the fp16 MMA operand of
 // layer 0, [S/128 tiles][n frames][x_hi chunks | x_lo chunks][128 streams][8 mels]; chunk c holds mels 8c..8c+7 (zero
@@ -210,11 +222,12 @@ inline int mel_tile_chunks(const kws_model* m) { return m->layer[0].tc_kx / 8; }
 inline bool mel_tile_split(const kws_model* m) { return m->layer[0].tc_kxw != m->layer[0].tc_kx; }
 bool gru_tc_can_split(int in_dim, bool last, int device);                // gru_tc.cu
 bool gru_tc_layer_fits(int in_dim, bool split, bool last, int device);
-// With src.lengths, frames of a stream past its own length are zero rows of mel_out, and nframes_out (if not null)
-// receives every stream's frame count: the seq_len of the recurrent kernels.
-int launch_frontend(const kws_model* m, const PcmSource& src, int64_t S, int32_t max_frames,
-                    const int32_t* nframes /*[S] or null*/, float* mel_out, cudaStream_t st,
-                    const FrontendPre* pre = nullptr, bool tiled_out = false, int32_t* nframes_out = nullptr);
+// Stream s gets min(frames_of(head_len + body length), max_frames) frames.  With src.lengths, frames of a stream past
+// its own length are zero rows of mel_out.  With src.lengths or pre, nframes_out receives every stream's frame count:
+// the seq_len of the recurrent kernels.
+int launch_frontend(const kws_model* m, const PcmSource& src, int64_t S, int32_t max_frames, float* mel_out,
+                    cudaStream_t st, const FrontendPre* pre = nullptr, bool tiled_out = false,
+                    int32_t* nframes_out = nullptr);
 
 struct GruArgs {
   const float* x = nullptr;       // layer-0 input [S, n, M] row-major, or stream-tiled when x_tiled

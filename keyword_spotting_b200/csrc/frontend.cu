@@ -27,9 +27,8 @@
 #include <cstring>
 #include <vector>
 
-#include "common.cuh"
-#include "tc05.cuh"
 #include "fft400.cuh"
+#include "frontend_io.cuh"
 
 namespace kws {
 
@@ -58,31 +57,12 @@ constexpr int kFeRegionFloats = kFeMagFloats > kFeWinFloats ? kFeMagFloats : kFe
 static_assert(kFeWinFloats <= kFeMagLive, "the window must not reach the rows that hold the zero bins");
 static_assert((kFeRegionFloats * 4) % 16 == 0, "mel quads follow the region and are read as float4");
 
-struct FrontendParams {
-  PcmSource src;
-  long S;
-  int max_frames;           // row stride of mel_out in frames
-  int groups;               // work items per stream = ceil(max_frames / 32)
-  const int* nframes;       // [S] or null -> frames from the signal length
-  int n_mel;
+struct FrontendParams : FrontendIo {
   const cpx* twiddle;       // [20*52] periodic k2-major table (fft::kTwSlots)
   const MelQuad* mel_q;     // [10 warps][quads_per_warp] (common.cuh)
   int mel_qpw;              // quads per warp (even)
   int vec_ok;               // int16 sources are 8-byte aligned with row strides % 4 == 0
-  float* mel_out;           // [S, max_frames, n_mel], or the recurrent kernel's fp16 operand (common.cuh) when tiled_out
-  int tiled_out;
-  int tile_chunks;          // tiled_out: chunks of 8 mels per half (kx / 8)
-  int tile_split;           // tiled_out: the lo half (what the fp16 rounding lost) follows the hi half
-  unsigned c_magic;         // ceil(2^32 / tile_chunks)
-  unsigned q_magic;         // ceil(2^32 / (n_mel / 4)): i / Q == umulhi(i, q_magic) for i < 2^16
   float mag_scale;          // 0.5 * (int16 input ? 2^-15 : 1), applied to the finished band sums
-  // fused server pre-step (only with groups == 1 and int16 input): VAD, frame count, next tail
-  int fuse_pre;
-  long long vad_limit;
-  int16_t* tail_next;       // [S, 400]
-  int* len_next;            // [S]
-  unsigned char* silence;   // [S]
-  int* nframes_out;         // [S] frames per stream (fused pre-step, or a forward over streams of their own lengths)
 };
 
 // Transposed magnitudes: bin k of frame slot sl sits at (k/2)*66 + 2*sl + (k&1), so the mel projection (lane = slot)
@@ -139,8 +119,6 @@ frontend_kernel(const FrontendParams p) {
     if (items32) return static_cast<long>(static_cast<unsigned>(item) / static_cast<unsigned>(p.groups));
     return item / p.groups;
   };
-  // frames of a signal of tl samples (utils/stft.py:60-61), 0 below one frame
-  auto frames_of = [](int tl) -> int { return tl >= kFft ? 1 + (tl - kFft) / kHop : 0; };
   const bool i16 = p.src.body_dtype == KWS_PCM_I16;
   const int M = p.n_mel;
   const int Mp = M | 1;                               // odd row stride of the [32][M] output tile: conflict-free band writes
@@ -158,7 +136,7 @@ frontend_kernel(const FrontendParams p) {
     const int g = static_cast<int>(item - s * p.groups);
     const int q0 = g * kFeItemHop;
     const int full_len = head_len + p.src.body_len;
-    const int total_len = kLens ? head_len + p.src.body_valid(s) : full_len;   // samples past the length stage as zeros
+    const int total_len = p.total_len<kLens>(s, head_len);       // samples past the length stage as zeros
     // both pointers are indexed by the stream sample number
     const int16_t* body = static_cast<const int16_t*>(p.src.body) + s * p.src.ld_body - head_len;
     const int16_t* head = p.src.head + s * p.src.ld_head;             // only dereferenced below head_len
@@ -232,20 +210,6 @@ frontend_kernel(const FrontendParams p) {
     return static_cast<int>(acc);
   };
 
-  // frames [fa, fb) of stream s in mel_out (either layout) -> zero: the rows past a stream's length
-  auto zero_rows = [&](long s, int fa, int fb) {
-    if (fb > p.max_frames) fb = p.max_frames;
-    if (fa >= fb) return;
-    if (p.tiled_out) {
-      const int per_frame = p.tile_split ? 2 * p.tile_chunks : p.tile_chunks;
-      uint4* dst = reinterpret_cast<uint4*>(p.mel_out) + ((s >> 7) * p.max_frames + fa) * static_cast<long>(per_frame) * 128 + (s & 127);
-      for (int i = tid; i < (fb - fa) * per_frame; i += kFeThreads) dst[static_cast<long>(i) * 128] = make_uint4(0u, 0u, 0u, 0u);
-    } else {
-      float* dst = p.mel_out + (s * p.max_frames + fa) * static_cast<long>(M);
-      for (int i = tid; i < (fb - fa) * M; i += kFeThreads) dst[i] = 0.0f;
-    }
-  };
-
   long item = blockIdx.x;
   uint2 pre[kFeQuadRounds];
   int head_len = 0;
@@ -258,10 +222,8 @@ frontend_kernel(const FrontendParams p) {
     const long s = stream_of(item);
     const int g = static_cast<int>(item - s * p.groups);
     if (!i16) head_len = p.src.head_len ? p.src.head_len[s] : 0;
-    const int total_len = head_len + (kLens ? p.src.body_valid(s) : p.src.body_len);
-    const int nfr_sig = frames_of(total_len);
-    int nfr = p.fuse_pre ? nfr_sig : (p.nframes ? p.nframes[s] : nfr_sig);
-    if (nfr > p.max_frames) nfr = p.max_frames;
+    const int total_len = p.total_len<kLens>(s, head_len);
+    const int nfr = p.frames(total_len);
     const int q0 = g * kFeItemHop;                    // stream sample held at window position 0
     const int f0 = g * kFeItemFrames;
     // the next item's carried-tail length is needed for its addresses: fetch it a whole item ahead
@@ -273,7 +235,7 @@ frontend_kernel(const FrontendParams p) {
       // the item starts past the stream's last frame: zero rows and no PCM (load_quads loaded none), no barrier needed --
       // the next item's staging writes only the window region, whose last reads precede this item
       if (i16 && next < items) load_quads(next, head_len_next, pre);
-      zero_rows(s, f0, f0 + kFeItemFrames);
+      p.zero_rows<kFeThreads>(s, f0, f0 + kFeItemFrames, tid);
       head_len = head_len_next;
       continue;
     }
@@ -301,11 +263,10 @@ frontend_kernel(const FrontendParams p) {
     __syncthreads();
 
     if (p.fuse_pre) {
-      // keep = (len-400)%160+240 last samples (detector.py:181-182); everything when no frame fits yet
-      const int keep = total_len >= kFft ? (total_len - kFft) % kHop + (kFft - kHop) : total_len;
+      const int keep = tail_keep(total_len);
       const int start = total_len - keep;
-      int16_t* tnext = p.tail_next + s * 400;
-      if (((start | keep) & 3) == 0 && (reinterpret_cast<uintptr_t>(p.tail_next) & 7) == 0) {
+      int16_t* tnext = p.pre.tail_next + s * 400;
+      if (((start | keep) & 3) == 0 && (reinterpret_cast<uintptr_t>(p.pre.tail_next) & 7) == 0) {
         // whole quads: the first keep/4 (<= 100) threads convert four staged samples back (exact) and store 8 bytes
         if (4 * tid < keep) {
           const int w = start + 4 * tid;
@@ -323,11 +284,7 @@ frontend_kernel(const FrontendParams p) {
       if (warp == 0) {                                 // <= 10 partial sums of at most 20 * 32768 each: int is enough
         const int part = lane < kFeWarps ? red[lane] : 0;
         const int sum = __reduce_add_sync(0xffffffffu, part);
-        if (lane == 0) {
-          p.silence[s] = static_cast<long long>(sum) > p.vad_limit ? 0 : 1;
-          p.nframes_out[s] = nfr;
-          p.len_next[s] = keep;
-        }
+        if (lane == 0) p.pre.record(s, sum, nfr, keep, p.nframes_out);
       }
     }
 
@@ -395,48 +352,9 @@ frontend_kernel(const FrontendParams p) {
     }
     __syncthreads();
     // ---- the item's frames are one contiguous block of mel_out
-    {
-      int nfi = nfr - f0;
-      if (nfi > kFeItemFrames) nfi = kFeItemFrames;
-      const int total = nfi > 0 ? nfi * M : 0;
-      if (p.tiled_out) {
-        // the recurrent kernel's layer-0 operand (common.cuh): per frame, chunks of 8 mels as fp16 and (split) chunks of
-        // what that rounding lost; the 16-byte piece (frame, chunk) of stream s sits between those of its 127 tile mates
-        const int nc = p.tile_chunks;
-        const int per_frame = p.tile_split ? 2 * nc : nc;
-        uint4* dst = reinterpret_cast<uint4*>(p.mel_out) + ((s >> 7) * p.max_frames + f0) * static_cast<long>(per_frame) * 128 + (s & 127);
-        const int pieces = nfi > 0 ? nfi * nc : 0;
-        for (int i = tid; i < pieces; i += kFeThreads) {
-          const int f = nc == 1 ? i : static_cast<int>(__umulhi(static_cast<unsigned>(i), p.c_magic));   // i / nc, i < 2^16
-          const int c = i - f * nc;
-          const float* src = out_tile + f * Mp + 8 * c;
-          float v[8];
-#pragma unroll
-          for (int j = 0; j < 8; ++j) v[j] = 8 * c + j < M ? src[j] : 0.0f;
-          uint4 hi, lo;
-          tc::split_half8(v, &hi, &lo);
-          dst[(f * per_frame + c) * 128] = hi;
-          if (p.tile_split) dst[(f * per_frame + nc + c) * 128] = lo;
-        }
-      } else if ((M & 3) == 0 && (reinterpret_cast<uintptr_t>(p.mel_out) & 15) == 0) {
-        // 16-byte pieces: chunk c (of Q) of frame f goes to row-major (s*n + f0 + f)*Q + c
-        const int Q = M >> 2;
-        float4* dst4 = reinterpret_cast<float4*>(p.mel_out) + (s * p.max_frames + f0) * static_cast<long>(Q);
-        for (int i = tid; i < (total >> 2); i += kFeThreads) {
-          const int f = Q == 1 ? i : static_cast<int>(__umulhi(static_cast<unsigned>(i), p.q_magic));   // i / Q, i < 2^16
-          const int c = i - f * Q;
-          const float* src = out_tile + f * Mp + 4 * c;
-          dst4[i] = make_float4(src[0], src[1], src[2], src[3]);
-        }
-      } else {
-        float* dst = p.mel_out + (s * p.max_frames + f0) * M;
-        for (int i = tid; i < total; i += kFeThreads) {
-          const int f = i / M;
-          dst[i] = out_tile[f * Mp + (i - f * M)];
-        }
-      }
-      if (kLens) zero_rows(s, f0 + nfi, f0 + kFeItemFrames);   // the item's frames past the stream's length
-    }
+    const int nfi = max(0, min(nfr - f0, kFeItemFrames));
+    p.store_tile<kFeThreads>(out_tile, Mp, s, f0, nfi, tid);
+    if (kLens) p.zero_rows<kFeThreads>(s, f0 + nfi, f0 + kFeItemFrames, tid);   // the item's frames past the stream's length
     head_len = head_len_next;
   }
 }
@@ -503,50 +421,41 @@ bool frontend_can_fuse_pre(const kws_model* m, int chunk_len, int tail_cap) {
   return chunk_len + tail_cap - 1 <= kFeWinSamples;
 }
 
-int launch_frontend(const kws_model* m, const PcmSource& src, int64_t S, int32_t max_frames,
-                    const int32_t* nframes, float* mel_out, cudaStream_t st, const FrontendPre* pre, bool tiled_out,
-                    int32_t* nframes_out) {
+int launch_frontend(const kws_model* m, const PcmSource& src, int64_t S, int32_t max_frames, float* mel_out,
+                    cudaStream_t st, const FrontendPre* pre, bool tiled_out, int32_t* nframes_out) {
   if (S <= 0) return KWS_OK;
   if (max_frames <= 0 && !pre) return KWS_OK;
-  if (frontend_uses_tc(m, src.body_dtype))
-    return launch_frontend_tc(m, src, S, max_frames, nframes, mel_out, st, pre, tiled_out, nframes_out);
-  FrontendParams p;
-  p.src = src;
-  p.S = S;
-  p.max_frames = max_frames;
-  p.groups = static_cast<int>(ceil_div(max_frames > 0 ? max_frames : 1, kFeItemFrames));
-  p.nframes = nframes;
-  p.n_mel = m->cfg.n_mel;
+  const bool tc = frontend_uses_tc(m, src.body_dtype);
+  FrontendIo io;
+  io.src = src;
+  io.S = S;
+  io.max_frames = max_frames;
+  io.groups = static_cast<int>(ceil_div(max_frames > 0 ? max_frames : 1, tc ? frontend_tc_item_frames() : kFeItemFrames));
+  io.n_mel = m->cfg.n_mel;
+  io.mel_out = mel_out;
+  io.tiled_out = tiled_out ? 1 : 0;
+  io.tile_chunks = tiled_out ? mel_tile_chunks(m) : 1;
+  io.tile_split = tiled_out && mel_tile_split(m) ? 1 : 0;
+  io.c_magic = static_cast<unsigned>(((1ull << 32) + io.tile_chunks - 1) / io.tile_chunks);
+  io.q_magic = m->cfg.n_mel >= 4 ? static_cast<unsigned>(((1ull << 32) + (m->cfg.n_mel / 4) - 1) / (m->cfg.n_mel / 4)) : 0u;
+  io.nframes_out = nframes_out;
+  io.fuse_pre = pre ? 1 : 0;
+  if (pre) {
+    if (io.groups != 1 || src.body_dtype != KWS_PCM_I16 || !nframes_out)
+      return fail(KWS_ERR_INVALID_ARGUMENT, "fused pre-step needs an int16 chunk that fits one work item, and nframes_out");
+    if (src.lengths) return fail(KWS_ERR_INVALID_ARGUMENT, "the fused pre-step takes no stream lengths");
+    io.pre = *pre;
+  }
+  if (tc) return launch_frontend_tc(m, io, st);
+
+  FrontendParams p{io};
   p.twiddle = reinterpret_cast<const cpx*>(m->twiddle400);
   p.mel_q = m->mel.quads;
   p.mel_qpw = m->mel.quads_per_warp;
   p.vec_ok = (reinterpret_cast<uintptr_t>(src.body) % 8 == 0 && src.ld_body % 4 == 0 &&
               reinterpret_cast<uintptr_t>(src.head) % 8 == 0 && src.ld_head % 4 == 0) ? 1 : 0;
-  p.mel_out = mel_out;
-  p.tiled_out = tiled_out ? 1 : 0;
-  p.q_magic = m->cfg.n_mel >= 4 ? static_cast<unsigned>(((1ull << 32) + (m->cfg.n_mel / 4) - 1) / (m->cfg.n_mel / 4)) : 0u;
-  p.tile_chunks = tiled_out ? mel_tile_chunks(m) : 1;
-  p.tile_split = tiled_out && mel_tile_split(m) ? 1 : 0;
-  p.c_magic = static_cast<unsigned>(((1ull << 32) + p.tile_chunks - 1) / p.tile_chunks);
   p.mag_scale = src.body_dtype == KWS_PCM_I16 ? 0.5f / 32768.0f : 0.5f;
-  p.fuse_pre = 0;
-  p.vad_limit = 0;
-  p.tail_next = nullptr;
-  p.len_next = nullptr;
-  p.silence = nullptr;
-  p.nframes_out = nframes_out;
-  if (pre) {
-    if (p.groups != 1 || src.body_dtype != KWS_PCM_I16)
-      return fail(KWS_ERR_INVALID_ARGUMENT, "fused pre-step needs an int16 chunk that fits one work item");
-    p.fuse_pre = 1;
-    p.vad_limit = pre->vad_limit;
-    p.tail_next = pre->tail_next;
-    p.len_next = pre->len_next;
-    p.silence = pre->silence;
-    p.nframes_out = pre->nframes_out;
-  }
   const bool in_smem = quads_in_smem(m), lens = src.lengths != nullptr;
-  if (lens && pre) return fail(KWS_ERR_INVALID_ARGUMENT, "the fused pre-step takes no stream lengths");
   auto kernel = in_smem ? (lens ? frontend_kernel<true, true> : frontend_kernel<true, false>)
                         : (lens ? frontend_kernel<false, true> : frontend_kernel<false, false>);
   const size_t smem = frontend_smem_bytes(m);

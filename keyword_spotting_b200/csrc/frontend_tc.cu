@@ -33,8 +33,7 @@
 
 #include <cuda_fp16.h>
 
-#include "common.cuh"
-#include "tc05.cuh"
+#include "frontend_io.cuh"
 
 namespace kws {
 
@@ -67,39 +66,14 @@ constexpr int kFtOutStride = 65;              // floats per frame row of the out
 enum { kFbBfull0 = 0, kFbBfull1, kFbBempty0, kFbBempty1, kFbDfull, kFbDempty, kFbMagFull0, kFbMagFull1, kFbMagEmpty0,
        kFbMagEmpty1, kFbNum };
 
-struct FrontendTcParams {
-  PcmSource src;
-  long S;
-  int max_frames;
-  int groups;               // work items per stream = ceil(max_frames / 30)
-  const int* nframes;
-  int n_mel;
+struct FrontendTcParams : FrontendIo {
   const uint32_t* tw;       // [2 tiles][2 parts][128 lanes][40] packed fp16 pairs
   const int4* mel_seg;      // [n_mel] {first bin, bins (multiple of 8), offset into mel_w (multiple of 4), 0}
   const float* mel_w;       // the spans' weights, concatenated and zero-padded
   int mel_nw;               // floats in mel_w (multiple of 4)
-  int vec_ok;
-  float* mel_out;
-  int tiled_out;
-  int tile_chunks;          // tiled_out: chunks of 8 mels per half (kx / 8), whether the lo half follows, ceil(2^32 / chunks)
-  int tile_split;
-  unsigned c_magic;
-  unsigned q_magic;
-  int fuse_pre;
-  long long vad_limit;
-  int16_t* tail_next;
-  int* len_next;
-  unsigned char* silence;
-  int* nframes_out;
-  volatile int* dbg;        // optional host-mapped timeline buffer (KWS_FT_DEBUG=1)
+  int vec_ok;               // int16 sources are 16-byte aligned with row strides % 8 == 0
 };
 
-// timeline (KWS_FT_DEBUG): low 32 bits of clock64 at key hand-overs of items 40..43 of CTA 0
-#define FT_TIME(role, ev)                                                                  \
-  do {                                                                                     \
-    if (p.dbg && lane == 0 && blockIdx.x == 0 && i >= 40 && i < 44)                        \
-      p.dbg[(static_cast<int>(i) - 40) * 64 + (role) * 8 + (ev)] = static_cast<int>(clock64()); \
-  } while (0)
 __device__ __forceinline__ void ft_arrive(uint64_t* bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tc::smem_u32(bar)) : "memory");
 }
@@ -144,9 +118,6 @@ __device__ __forceinline__ float ft_sqrt(float x) {
   asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
-
-// frames of a signal of tl samples (utils/stft.py:60-61), 0 below one frame
-__device__ __forceinline__ int ft_frames_of(int tl) { return tl >= kFft ? 1 + (tl - kFft) / kHop : 0; }
 
 // kLens: the streams have lengths of their own (p.src.lengths), as in frontend_kernel (frontend.cu); without them none of
 // their handling is compiled in.
@@ -252,18 +223,14 @@ frontend_tc_kernel(const FrontendTcParams p) {
     };
     for (long i = 0; i < n_mine; ++i) {
       const int buf = static_cast<int>(i & 1);
-      FT_TIME(0, 5);
       ft_spin(&bars[kFbBfull0 + buf], static_cast<uint32_t>((i >> 1) & 1));
-      FT_TIME(0, 0);
       if (i > 0) ft_spin(&bars[kFbDempty], static_cast<uint32_t>((i - 1) & 1));
       tc::fence_after_sync();
-      FT_TIME(0, 1);
       // (the buffer index is loop-carried, which the compiler cannot prove warp-uniform: branch on it so that every
       // descriptor inside is derived from kernel constants and stays in uniform registers -- no per-MMA broadcast loop)
       constexpr uint64_t kPart = static_cast<uint64_t>(kFtB1Part >> 4);
       if (buf == 0) gemm1(b1desc, b1desc + kPart, &bars[kFbDfull], &bars[kFbBempty0]);
       else gemm1(b1desc + 2 * kPart, b1desc + 3 * kPart, &bars[kFbDfull], &bars[kFbBempty1]);
-      FT_TIME(0, 2);
     }
   } else if (warp >= kFtLoadWarp0 && warp < kFtOutWarp0) {
     // ================================================================ PCM loaders: int16 -> (x_hi, x_lo) fp16 operands
@@ -275,20 +242,19 @@ frontend_tc_kernel(const FrontendTcParams p) {
       const int g = static_cast<int>(item - s * p.groups);
       const int buf = static_cast<int>(i & 1);
       const int head_len = p.src.head_len ? p.src.head_len[s] : 0;
-      const int total_len = head_len + (kLens ? p.src.body_valid(s) : p.src.body_len);
+      const int total_len = p.total_len<kLens>(s, head_len);
       // samples staged from PCM: none for an item past the stream's last frame (its rows are zeros), otherwise those
       // below the stream's length -- the piece that straddles it goes element by element, the rest stage as zeros
-      const int ld_len = kLens && g * kFtFrames >= ft_frames_of(total_len) ? 0 : total_len;
+      const int ld_len = kLens && g * kFtFrames >= frames_of(total_len) ? 0 : total_len;
       const int q0 = g * kFtItemHop;
       const int16_t* body = static_cast<const int16_t*>(p.src.body) + s * p.src.ld_body - head_len;   // indexed by stream sample
       const int16_t* head = p.src.head ? p.src.head + s * p.src.ld_head : nullptr;
       const bool fast = p.vec_ok && (head_len & 7) == 0;
-      // server pre-step (detector.py:168-183): keep = (len-400)%160+240 last samples; everything when no frame fits yet
-      const int keep = total_len >= kFft ? (total_len - kFft) % kHop + (kFft - kHop) : total_len;
+      // server pre-step (detector.py:168-183)
+      const int keep = tail_keep(total_len);
       const int start = total_len - keep;
-      int16_t* tnext = p.fuse_pre ? p.tail_next + s * 400 : nullptr;
-      const bool tail_fast = p.fuse_pre && ((start | keep) & 7) == 0 && (reinterpret_cast<uintptr_t>(p.tail_next) & 15) == 0;
-      if (warp == kFtLoadWarp0) FT_TIME(3, 0);
+      int16_t* tnext = p.fuse_pre ? p.pre.tail_next + s * 400 : nullptr;
+      const bool tail_fast = p.fuse_pre && ((start | keep) & 7) == 0 && (reinterpret_cast<uintptr_t>(p.pre.tail_next) & 15) == 0;
       const int n_pieces = p.fuse_pre ? kFtPieces + 10 : kFtPieces;       // the fused chunk may reach 5199 samples
       // every piece this thread owns is requested before anything is waited for: one HBM latency per item, not seven
       constexpr int kRounds = (kFtPieces + 10 + kFtLoadThreads - 1) / kFtLoadThreads;
@@ -377,16 +343,12 @@ frontend_tc_kernel(const FrontendTcParams p) {
         if (lane == 0) atomicAdd(&sVad[buf], vad);
         asm volatile("bar.sync 2, 224;" ::: "memory");
         if (ltid == 0) {
-          const int nfr_sig = total_len >= kFft ? 1 + (total_len - kFft) / kHop : 0;
-          p.silence[s] = static_cast<long long>(sVad[buf]) > p.vad_limit ? 0 : 1;
-          p.nframes_out[s] = nfr_sig < p.max_frames ? nfr_sig : p.max_frames;
-          p.len_next[s] = keep;
+          p.pre.record(s, sVad[buf], p.frames(total_len), keep, p.nframes_out);
           sVad[buf] = 0;
         }
       }
       tc::fence_proxy_async();
       ft_arrive(&bars[kFbBfull0 + buf]);
-      if (warp == kFtLoadWarp0) FT_TIME(3, 1);
     }
   } else if (warp >= kFtOutWarp0) {
     // ================================================================ mel projection + output: lane = frame
@@ -399,13 +361,9 @@ frontend_tc_kernel(const FrontendTcParams p) {
       const int g = static_cast<int>(item - s * p.groups);
       const int buf = static_cast<int>(i & 1);
       const int head_len = p.src.head_len ? p.src.head_len[s] : 0;
-      const int total_len = head_len + (kLens ? p.src.body_valid(s) : p.src.body_len);
-      const int nfr_sig = ft_frames_of(total_len);
-      int nfr = p.fuse_pre ? nfr_sig : (p.nframes ? p.nframes[s] : nfr_sig);
-      if (nfr > p.max_frames) nfr = p.max_frames;
+      const int nfr = p.frames(p.total_len<kLens>(s, head_len));
       const int f0 = g * kFtFrames;
-      int nfi = nfr - f0;
-      nfi = nfi < 0 ? 0 : (nfi > kFtFrames ? kFtFrames : nfi);
+      const int nfi = max(0, min(nfr - f0, kFtFrames));
       if (kLens && p.nframes_out && g == 0 && otid == 0) p.nframes_out[s] = nfr;
       ft_wait_hint(&bars[kFbMagFull0 + buf], static_cast<uint32_t>((i >> 1) & 1), 200);
       // bands q, q+8, ...: eight bins per trip (spans are zero-padded to multiples of 8): the eight magnitude loads
@@ -436,52 +394,8 @@ frontend_tc_kernel(const FrontendTcParams p) {
       }
       ft_arrive(&bars[kFbMagEmpty0 + buf]);          // this thread's magnitude reads are done
       asm volatile("bar.sync 3, 256;" ::: "memory");
-      const int total = nfi * M;
-      if (p.tiled_out) {
-        // the recurrent kernel's layer-0 operand (common.cuh): fp16 hi chunks and, split, lo chunks of 8 mels
-        const int nc = p.tile_chunks;
-        const int per_frame = p.tile_split ? 2 * nc : nc;
-        uint4* dst = reinterpret_cast<uint4*>(p.mel_out) + ((s >> 7) * p.max_frames + f0) * static_cast<long>(per_frame) * 128 + (s & 127);
-        const int pieces = nfi > 0 ? nfi * nc : 0;
-        for (int idx = otid; idx < pieces; idx += kFtOutThreads) {
-          const int f = nc == 1 ? idx : static_cast<int>(__umulhi(static_cast<unsigned>(idx), p.c_magic));
-          const int c = idx - f * nc;
-          const float* src = sOut + f * kFtOutStride + 8 * c;
-          float v[8];
-#pragma unroll
-          for (int j = 0; j < 8; ++j) v[j] = 8 * c + j < M ? src[j] : 0.0f;
-          uint4 hi, lo;
-          tc::split_half8(v, &hi, &lo);
-          dst[(f * per_frame + c) * 128] = hi;
-          if (p.tile_split) dst[(f * per_frame + nc + c) * 128] = lo;
-        }
-      } else if ((M & 3) == 0 && (reinterpret_cast<uintptr_t>(p.mel_out) & 15) == 0) {
-        const int Q = M >> 2;
-        float4* dst4 = reinterpret_cast<float4*>(p.mel_out) + (s * p.max_frames + f0) * static_cast<long>(Q);
-        for (int idx = otid; idx < (total >> 2); idx += kFtOutThreads) {
-          const int f = Q == 1 ? idx : static_cast<int>(__umulhi(static_cast<unsigned>(idx), p.q_magic));
-          const int c = idx - f * Q;
-          const float* src = sOut + f * kFtOutStride + 4 * c;
-          dst4[idx] = make_float4(src[0], src[1], src[2], src[3]);
-        }
-      } else {
-        float* dst = p.mel_out + (s * p.max_frames + f0) * M;
-        for (int idx = otid; idx < total; idx += kFtOutThreads) {
-          const int f = idx / M;
-          dst[idx] = sOut[f * kFtOutStride + (idx - f * M)];
-        }
-      }
-      if (kLens) {                                   // the item's frames past the stream's length are zero rows
-        const int fa = f0 + nfi, fb = f0 + kFtFrames < p.max_frames ? f0 + kFtFrames : p.max_frames;
-        if (p.tiled_out) {
-          const int per_frame = p.tile_split ? 2 * p.tile_chunks : p.tile_chunks;
-          uint4* dst = reinterpret_cast<uint4*>(p.mel_out) + ((s >> 7) * p.max_frames + fa) * static_cast<long>(per_frame) * 128 + (s & 127);
-          for (int idx = otid; idx < (fb - fa) * per_frame; idx += kFtOutThreads) dst[static_cast<long>(idx) * 128] = make_uint4(0u, 0u, 0u, 0u);
-        } else {
-          float* dst = p.mel_out + (s * p.max_frames + fa) * static_cast<long>(M);
-          for (int idx = otid; idx < (fb - fa) * M; idx += kFtOutThreads) dst[idx] = 0.0f;
-        }
-      }
+      p.store_tile<kFtOutThreads>(sOut, kFtOutStride, s, f0, nfi, otid);
+      if (kLens) p.zero_rows<kFtOutThreads>(s, f0 + nfi, f0 + kFtFrames, otid);   // the item's frames past the stream's length
       asm volatile("bar.sync 3, 256;" ::: "memory");
     }
   } else {
@@ -505,10 +419,8 @@ frontend_tc_kernel(const FrontendTcParams p) {
     const uint32_t dre = tmem + lane_sel + kFtColD + 32 * F, dim = dre + 128;
 
     for (long i = 0; i < n_mine; ++i) {
-      if (warp == 0 || warp == 4 || warp == 8 || warp == 15) FT_TIME(warp == 0 ? 4 : (warp == 15 ? 5 : warp >> 2), 0);
       ft_wait_hint(&bars[kFbDfull], static_cast<uint32_t>(i & 1), 100);
       tc::fence_after_sync();
-      if (warp == 0 || warp == 4 || warp == 8 || warp == 15) FT_TIME(warp == 0 ? 4 : (warp == 15 ? 5 : warp >> 2), 1);
       float2 mg[8];                                   // (|X_f(k)|, |X_f(200-k)|) of frames 8F .. 8F+7
       // TMEM reads run at ~64 B/clk per SM and are what this role is bound by: every column is read exactly once.
       // frames 8F+4sub .. +3 use blocks 16F+8sub .. +10 (two columns per block: x, (-1)^m x):
@@ -538,7 +450,6 @@ frontend_tc_kernel(const FrontendTcParams p) {
           for (int j = 0; j < 16; ++j) { re[8 + j] = a16[j]; im[8 + j] = b16[j]; }
           tc::fence_before_sync();                    // every TMEM read of this item is done: the half may be overwritten
           ft_arrive(&bars[kFbDempty]);
-          if (warp == 0 || warp == 4 || warp == 8 || warp == 15) FT_TIME(warp == 0 ? 4 : (warp == 15 ? 5 : warp >> 2), 2);
         }
 #pragma unroll
         for (int t = 0; t < 4; ++t) {
@@ -574,7 +485,6 @@ frontend_tc_kernel(const FrontendTcParams p) {
         }
       }
       ft_arrive(&bars[kFbMagFull0 + mbuf]);
-      if (warp == 0 || warp == 4 || warp == 8 || warp == 15) FT_TIME(warp == 0 ? 4 : (warp == 15 ? 5 : warp >> 2), 3);
     }
   }
   tc::fence_before_sync();
@@ -658,83 +568,20 @@ int default_frontend() {
 
 int frontend_tc_item_frames() { return kFtFrames; }
 
-int launch_frontend_tc(const kws_model* m, const PcmSource& src, int64_t S, int32_t max_frames, const int32_t* nframes,
-                       float* mel_out, cudaStream_t st, const FrontendPre* pre, bool tiled_out, int32_t* nframes_out) {
-  FrontendTcParams p;
-  p.src = src;
-  p.S = S;
-  p.max_frames = max_frames;
-  p.groups = static_cast<int>(ceil_div(max_frames > 0 ? max_frames : 1, kFtFrames));
-  p.nframes = nframes;
-  p.n_mel = m->cfg.n_mel;
+int launch_frontend_tc(const kws_model* m, const FrontendIo& io, cudaStream_t st) {
+  FrontendTcParams p{io};
   p.tw = m->fe_tc.tw;
   p.mel_seg = reinterpret_cast<const int4*>(m->fe_tc.mel_seg);
   p.mel_w = m->fe_tc.mel_w;
   p.mel_nw = m->fe_tc.mel_nw;
-  p.vec_ok = (reinterpret_cast<uintptr_t>(src.body) % 16 == 0 && src.ld_body % 8 == 0 &&
-              reinterpret_cast<uintptr_t>(src.head) % 16 == 0 && src.ld_head % 8 == 0) ? 1 : 0;
-  p.mel_out = mel_out;
-  p.tiled_out = tiled_out ? 1 : 0;
-  p.q_magic = m->cfg.n_mel >= 4 ? static_cast<unsigned>(((1ull << 32) + (m->cfg.n_mel / 4) - 1) / (m->cfg.n_mel / 4)) : 0u;
-  p.tile_chunks = tiled_out ? mel_tile_chunks(m) : 1;
-  p.tile_split = tiled_out && mel_tile_split(m) ? 1 : 0;
-  p.c_magic = static_cast<unsigned>(((1ull << 32) + p.tile_chunks - 1) / p.tile_chunks);
-  p.fuse_pre = 0;
-  p.vad_limit = 0;
-  p.tail_next = nullptr;
-  p.len_next = nullptr;
-  p.silence = nullptr;
-  p.nframes_out = nframes_out;
-  if (pre) {
-    if (p.groups != 1) return fail(KWS_ERR_INVALID_ARGUMENT, "fused pre-step needs a chunk that fits one work item");
-    p.fuse_pre = 1;
-    p.vad_limit = pre->vad_limit;
-    p.tail_next = pre->tail_next;
-    p.len_next = pre->len_next;
-    p.silence = pre->silence;
-    p.nframes_out = pre->nframes_out;
-  }
-  static volatile int* dbg_host = nullptr;
-  static int* dbg_dev = nullptr;
-  static const bool dbg_on = std::getenv("KWS_FT_DEBUG") != nullptr;
-  p.dbg = nullptr;
-  if (dbg_on) {
-    if (!dbg_host) {
-      int* h = nullptr;
-      KWS_CUDA_OK(cudaHostAlloc(reinterpret_cast<void**>(&h), 256 * sizeof(int), cudaHostAllocMapped));
-      KWS_CUDA_OK(cudaHostGetDevicePointer(reinterpret_cast<void**>(&dbg_dev), h, 0));
-      dbg_host = h;
-    }
-    for (int i = 0; i < 256; ++i) dbg_host[i] = 0;
-    p.dbg = dbg_dev;
-  }
-  if (src.lengths && pre) return fail(KWS_ERR_INVALID_ARGUMENT, "the fused pre-step takes no stream lengths");
-  auto kernel = src.lengths ? frontend_tc_kernel<true> : frontend_tc_kernel<false>;
+  p.vec_ok = (reinterpret_cast<uintptr_t>(io.src.body) % 16 == 0 && io.src.ld_body % 8 == 0 &&
+              reinterpret_cast<uintptr_t>(io.src.head) % 16 == 0 && io.src.ld_head % 8 == 0) ? 1 : 0;
+  auto kernel = io.src.lengths ? frontend_tc_kernel<true> : frontend_tc_kernel<false>;
   const size_t smem = frontend_tc_smem_bytes(p.mel_nw);
   KWS_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-  const long items = S * p.groups;
+  const long items = io.S * io.groups;
   const long blocks = items < sm_count() ? items : sm_count();
   kernel<<<static_cast<unsigned>(blocks), kFtThreads, smem, st>>>(p);
-  if (dbg_on) {
-    const cudaError_t e = cudaStreamSynchronize(st);
-    fprintf(stderr, "[frontend_tc] S=%ld groups=%d sync=%s markers:", static_cast<long>(S), p.groups, cudaGetErrorString(e));
-    fprintf(stderr, "\n");
-    if (dbg_host[1]) {
-      const unsigned t0 = static_cast<unsigned>(dbg_host[0]);
-      const char* roles[6] = {"mma : got_Bfull got_Dempty issued | (5) poll_Bfull", "epi warp 4: wait_Dfull got_Dfull arrive_Dempty mags_out",
-                              "epi warp 8: wait_Dfull got_Dfull arrive_Dempty mags_out", "load: start arrive_Bfull",
-                              "epi warp 0: wait_Dfull got_Dfull arrive_Dempty mags_out", "epi warp 15: wait_Dfull got_Dfull arrive_Dempty mags_out"};
-      for (int it = 0; it < 4; ++it)
-        for (int r = 0; r < 6; ++r) {
-          fprintf(stderr, "[frontend_tc] item %d %s:", 40 + it, roles[r]);
-          for (int e = 0; e < 6; ++e) {
-            const int v = dbg_host[it * 64 + r * 8 + e];
-            if (v) fprintf(stderr, " %u", static_cast<unsigned>(v) - t0);
-          }
-          fprintf(stderr, "\n");
-        }
-    }
-  }
   KWS_LAUNCH_OK("frontend_tc_kernel");
   return KWS_OK;
 }

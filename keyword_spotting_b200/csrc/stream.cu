@@ -25,12 +25,10 @@ namespace kws {
 
 constexpr int kTailCap = 400;
 
-// One warp per stream: VAD, frame count, next tail.
+// One warp per stream: the pre-step of a chunk that the front end cannot take in one work item.
 __global__ void __launch_bounds__(256)
-stream_pre_kernel(const int16_t* __restrict__ pcm, long ld, int chunk_len, long S, long long vad_limit,
-                  const int16_t* __restrict__ tail_cur, const int* __restrict__ len_cur,
-                  int16_t* __restrict__ tail_next, int* __restrict__ len_next,
-                  unsigned char* __restrict__ silence, int* __restrict__ nframes, int max_frames) {
+stream_pre_kernel(const int16_t* __restrict__ pcm, long ld, int chunk_len, long S, const int16_t* __restrict__ tail_cur,
+                  const int* __restrict__ len_cur, const FrontendPre pre, int* __restrict__ nframes, int max_frames) {
   const long s = (blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (s >= S) return;
@@ -56,15 +54,11 @@ stream_pre_kernel(const int16_t* __restrict__ pcm, long ld, int chunk_len, long 
   for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
   const int head = len_cur[s];
   const int total = head + chunk_len;
-  const int nfr = total >= kFft ? 1 + (total - kFft) / kHop : 0;
-  const int keep = total >= kFft ? (total - kFft) % kHop + (kFft - kHop) : total;   // detector.py:181-182
-  if (lane == 0) {
-    silence[s] = sum > vad_limit ? 0 : 1;
-    nframes[s] = nfr < max_frames ? nfr : max_frames;
-    len_next[s] = keep;
-  }
+  const int nfr = frames_of(total);
+  const int keep = tail_keep(total);
+  if (lane == 0) pre.record(s, sum, nfr < max_frames ? nfr : max_frames, keep, nframes);
   const int16_t* tcur = tail_cur + s * kTailCap;
-  int16_t* tnext = tail_next + s * kTailCap;
+  int16_t* tnext = pre.tail_next + s * kTailCap;
   for (int i = lane; i < keep; i += 32) {
     const int gidx = total - keep + i;
     tnext[i] = gidx < head ? tcur[gidx] : row[gidx - head];
@@ -205,10 +199,7 @@ static void free_stream(kws_stream* st) {
   delete st;
 }
 
-static int frames_for_chunk(int chunk_len) {      // with the longest possible carried tail (399)
-  const int total = chunk_len + kTailCap - 1;
-  return total >= kFft ? 1 + (total - kFft) / kHop : 0;
-}
+static int frames_for_chunk(int chunk_len) { return frames_of(chunk_len + kTailCap - 1); }   // with the longest tail (399)
 
 }  // namespace kws
 
@@ -336,7 +327,6 @@ extern "C" int kws_stream_step(kws_stream* st, const int16_t* pcm, int32_t chunk
   const int n_step = frames_for_chunk(chunk_len);
   const int C = m->cfg.num_classes;
 
-  const long long vad_limit = static_cast<long long>(st->cfg.vad_threshold) * 32768LL;
   PcmSource src;
   src.body = pcm;
   src.ld_body = ld_pcm;
@@ -352,26 +342,24 @@ extern "C" int kws_stream_step(kws_stream* st, const int16_t* pcm, int32_t chunk
     for (int i = 0; i < 4; ++i) KWS_CUDA_OK(cudaEventCreate(&tev[i]));
     KWS_CUDA_OK(cudaEventRecord(tev[0], cs));
   }
+  FrontendPre pre;
+  pre.vad_limit = static_cast<long long>(st->cfg.vad_threshold) * 32768LL;
+  pre.tail_next = st->tail[nxt];
+  pre.len_next = st->tail_len[nxt];
+  pre.silence = st->silence;
   if (fused) {
     // one pass over the chunk: VAD + tail carry + frame count + framing/FFT/mel
-    FrontendPre pre;
-    pre.vad_limit = vad_limit;
-    pre.tail_next = st->tail[nxt];
-    pre.len_next = st->tail_len[nxt];
-    pre.silence = st->silence;
-    pre.nframes_out = st->nframes;
-    int rc = launch_frontend(m, src, S, n_step, nullptr, st->mel, cs, &pre, tiled);
+    int rc = launch_frontend(m, src, S, n_step, st->mel, cs, &pre, tiled, st->nframes);
     if (rc != KWS_OK) return rc;
   } else {
     stream_pre_kernel<<<static_cast<unsigned>(ceil_div(S * 32, 256)), 256, 0, cs>>>(
-        pcm, ld_pcm, chunk_len, S, vad_limit, st->tail[cur], st->tail_len[cur], st->tail[nxt], st->tail_len[nxt],
-        st->silence, st->nframes, n_step);
+        pcm, ld_pcm, chunk_len, S, st->tail[cur], st->tail_len[cur], pre, st->nframes, n_step);
     KWS_LAUNCH_OK("stream_pre_kernel");
   }
 
   if (n_step > 0) {
     if (!fused) {
-      int rc = launch_frontend(m, src, S, n_step, st->nframes, st->mel, cs, nullptr, tiled);
+      int rc = launch_frontend(m, src, S, n_step, st->mel, cs, nullptr, tiled);
       if (rc != KWS_OK) return rc;
     }
     if (tev[1]) KWS_CUDA_OK(cudaEventRecord(tev[1], cs));

@@ -258,6 +258,51 @@ def test_streaming_server_irregular_chunks_and_window_overflow():
 
 
 @pytest.mark.parametrize("precision", ["fp32", "tc"])
+@pytest.mark.parametrize("frontend", ["fft", "tc"])
+def test_streaming_server_chunks_past_one_frontend_item(frontend, precision):
+    """Chunks whose [tail | chunk] no longer fits one front-end work item (more than 4961 new samples on the FFT
+    kernel, 4800 on the tensor-core one) run the separate pre-step kernel, then the front end over several items with
+    the carried tail in front.  The sizes cross both kernels' limits in both directions.  fp32 precision has the front
+    end write row-major mel, tc precision the recurrent kernel's fp16 row tiles.  Frames whose decode decision lies
+    within the contract tolerance of a threshold are decided on the GPU's softmax (_MarginJudge); everything else must
+    match the detector-loop oracle bit for bit."""
+    from keyword_spotting_b200 import DeployModel, StreamingDetector
+    from oracle import model as om, streaming as ost
+    from tests.test_gpu_parity_scale import _MarginJudge, _check_chunk
+    ow = _boost_fc(om.init_weights(seed=99, n_mel=40), gain=3.0)     # as test_streaming_server_on_the_tc_frontend
+    dm = DeployModel(make_config(40), to_product_weights(ow), precision=precision, frontend=frontend)
+    assert dm.frontend_kind == frontend
+    tol = TOL_FP32 if precision == "fp32" else TOL_CONTRACT
+    # tc precision: the oracle rounds the recurrent kernel's operands as the kernel does (fp16, layer-0 input split into
+    # hi + lo), so what is left is accumulation order.  Against the fp32 graph this FC reaches 1.3e-3 over chunks of 60
+    # to 100 frames from the operand rounding alone; test_streaming_server_tensor_core_mode holds that contract.
+    od = None if precision == "fp32" else np.float16
+    S = 40
+    rng = np.random.default_rng(12)
+    det = StreamingDetector(dm, S, max_chunk=16000, keyword="4321")
+    orc = ost.StreamOracle(ow, S, label="4321",
+                           forward=lambda x, st: om.deploy_forward(x, st, ow, np.float32, operand_dtype=od))
+    judge = _MarginJudge(0.4)
+    n_lab = 0
+    for i, n in enumerate([4961, 4962, 4800, 4801, 9600, 16000, 400, 12345, 5199]):
+        blk = synth_pcm16(rng, S, n, silent_frac=0.15)
+        trig, probs, nfr = det.step(blk, want_probs=True)
+        st = det.state().cpu().numpy()
+        labels, counts = det.window_labels()
+        judge.gpu = probs
+        want = orc.step(blk, decide_on=judge)
+        nf = want["softmax"].shape[1]
+        assert (nfr == nf).all(), (i, nfr[:4], nf)
+        assert np.abs(probs[:, :nf] - want["softmax"]).max() < tol, i
+        assert np.abs(st - want["state"]).max() < tol, i
+        _check_chunk(want, trig, probs, labels, counts, st, i)
+        n_lab += sum(len(l) // 2 for l in want["labels"])
+    assert n_lab > 100, n_lab
+    det.close()
+    dm.close()
+
+
+@pytest.mark.parametrize("precision", ["fp32", "tc"])
 def test_config2_full_size_properties(precision):
     """config 2: 4096 utterances x 3 s.  Oracle on a 16-utterance sample; for the rest the size-independent
     properties: batch independence (same utterance anywhere in the batch gives the same bits) and
