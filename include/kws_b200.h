@@ -256,6 +256,37 @@ int kws_stream_copy_state(kws_stream* st, float* state_out, void* stream);
 int kws_stream_labels(kws_stream* st, int32_t* labels_out, int32_t max_labels,
                       int32_t* counts_out, void* stream);
 
+/* Per-stream records: everything one stream carries from one chunk to the next, as a fixed-size, self-describing
+ * byte block, so that chosen streams can be saved, restored, compared or moved to another object or GPU between
+ * chunks.  Little-endian; every section is a multiple of 16 bytes (offsets in bytes, L = num_layers, H = hidden,
+ * W = window_chunks, Wp = W rounded up to 16):
+ *     0  uint32 magic 0x5253574B ("KWSR"), uint32 version 1, int32 L, int32 H
+ *    16  int32 W, int32 fpad (token slots per window entry, a multiple of 16), int32 record bytes, 0
+ *    32  int32 tail_len (carried PCM samples, 0..399), int32 win_n (window entries in use, 0..W), 0, 0
+ *    48  GRU state [L][H] fp32, raw bits
+ *    48 + 512 L           carried PCM tail [400] int16: the first tail_len samples
+ *    48 + 512 L + 800     slot_frames [Wp] uint8: frames of window entry q, oldest entry first
+ *    48 + 512 L + 800 + Wp  tokens [W][fpad] int8: per frame of entry q, the above-threshold winner class - 1, or -1
+ * record bytes = 848 + 512 L + Wp + W fpad (2368 at L = 2, W = 15, max_chunk = 4800).  Records are canonical: every
+ * byte that holds no state is zero (samples past tail_len, tokens past slot_frames[q], entries past win_n, padding),
+ * so the record of a stream does not depend on where its window ring starts, and export -> import -> export gives
+ * the same bytes.  Per-chunk scratch (VAD flags, frame counts, triggers, mel, probabilities) is not state: each step
+ * writes it before reading it.
+ *
+ * ids: DEVICE int64 [n]; records: DEVICE [n, kws_stream_record_bytes()], 16-byte aligned.  Both calls are
+ * stream-ordered, do not allocate and cost O(n), whatever the number of streams.  Ids must be distinct: with a
+ * duplicate id, which of its records lands is unspecified.
+ * Export of an id outside [0, n_streams) writes an all-zero record, which import rejects.
+ * Import treats every record as input from outside the program (it may come from disk).  status_out: DEVICE int32
+ * [n] or NULL; 0 = imported, 1 = id outside [0, n_streams), 2 = header does not match this object (magic, version,
+ * L, H, W, fpad or record bytes), 3 = malformed field (tail_len outside [0, 399], win_n outside [0, W], a used
+ * slot_frames above kws_stream_max_frames(), a used token outside [-1, num_classes - 3]).  A rejected record
+ * leaves its stream untouched.  An imported stream continues bit for bit as the exported one would have.        */
+int64_t kws_stream_record_bytes(const kws_stream* st);
+int kws_stream_export(kws_stream* st, const int64_t* ids, int64_t n, void* records, void* stream);
+int kws_stream_import(kws_stream* st, const int64_t* ids, int64_t n, const void* records,
+                      int32_t* status_out, void* stream);
+
 /* ----------------------------------------------------------------- wave server
  * The serving loop itself (HotwordDetector.start, detector.py:148-212: read a chunk -> model -> decode -> react,
  * forever) for all the streams of one GPU.  The streams are split into `waves` equal groups; a wave is one
@@ -299,6 +330,14 @@ int kws_server_stats(kws_server* s, int reset, double* p50_ms, double* p99_ms, d
 int kws_server_set_copy_only(kws_server* s, int copy_only);
 /* The wave's stream object (for kws_stream_labels / kws_stream_copy_state); owned by the server. */
 kws_stream* kws_server_wave_stream(kws_server* s, int32_t wave);
+/* kws_stream_export / kws_stream_import over the server's global stream ids [0, n_streams) (wave = id /
+ * streams_per_wave), records of kws_stream_record_bytes(kws_server_wave_stream(s, 0)) bytes.  Nothing may be in
+ * flight.  All ids go in one launch; the call synchronises `stream` before returning, so the next
+ * kws_server_submit sees the imported state.  The captured graphs stay valid: import writes the buffers they
+ * read.                                                                                                        */
+int kws_server_export(kws_server* s, const int64_t* ids, int64_t n, void* records, void* stream);
+int kws_server_import(kws_server* s, const int64_t* ids, int64_t n, const void* records, int32_t* status_out,
+                      void* stream);
 
 /* ----------------------------------------------------------------- octbit
  * K5 -- OctbitMatMul (octbit/octbit_mat_mul_op.cc:49-183; Python wrapper

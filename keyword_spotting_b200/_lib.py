@@ -113,6 +113,9 @@ _SIGNATURES = {
     "kws_stream_state": (c_void_p, [c_void_p]),
     "kws_stream_copy_state": (c_int, [c_void_p, c_void_p, c_void_p]),
     "kws_stream_labels": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_void_p]),
+    "kws_stream_record_bytes": (c_int64, [c_void_p]),
+    "kws_stream_export": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
+    "kws_stream_import": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
     "kws_server_create": (c_int, [c_void_p, POINTER(ServerConfig), POINTER(c_void_p)]),
     "kws_server_destroy": (c_int, [c_void_p]),
     "kws_server_info": (c_int, [c_void_p, POINTER(c_int64), POINTER(c_int32), POINTER(c_int32)]),
@@ -125,6 +128,8 @@ _SIGNATURES = {
                                  POINTER(c_int64), POINTER(c_int64)]),
     "kws_server_set_copy_only": (c_int, [c_void_p, c_int]),
     "kws_server_wave_stream": (c_void_p, [c_void_p, c_int32]),
+    "kws_server_export": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
+    "kws_server_import": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
     "kws_octbit_workspace_bytes": (c_size_t, [c_int64, c_int64]),
     "kws_octbit_matmul": (c_int, [c_void_p, c_void_p, c_void_p, c_float, c_int, c_int, c_int64, c_int64,
                                   c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),

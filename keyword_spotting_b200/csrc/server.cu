@@ -49,6 +49,8 @@ struct kws_server {
   std::vector<kws::Wave> waves;
   std::vector<float> latency_ms;    // one entry per completed (wave, chunk)
   long long triggers = 0;
+  kws::RecordSlots* record_table = nullptr;        // DEVICE [waves]: the record kernels' per-wave pointers
+  std::vector<kws::RecordSlots> record_table_host;
 };
 
 namespace kws {
@@ -70,6 +72,7 @@ static void free_server(kws_server* s) {
     if (w.st) kws_stream_destroy(w.st);
     if (w.cs) cudaStreamDestroy(w.cs);
   }
+  cudaFree(s->record_table);
   delete s;
 }
 
@@ -147,6 +150,9 @@ extern "C" int kws_server_create(kws_model* m, const kws_server_config* cfg, kws
       std::memset(w.host_trig[i], 0, sizeof(int32_t) * s->Sw);
     }
   }
+  s->record_table_host.resize(s->waves.size());
+  if (cudaMalloc(reinterpret_cast<void**>(&s->record_table), sizeof(RecordSlots) * s->waves.size()) != cudaSuccess)
+    return bail(fail(KWS_ERR_ALLOC, "record table of %zu waves", s->waves.size()));
   if (cfg->use_graphs) {
     // Two warm-up chunks per wave outside capture (first-use initialisation of every kernel must not happen under
     // capture), then forget them; then capture every (ingest slot, tail ping-pong) combination: kws_stream_step
@@ -307,6 +313,39 @@ extern "C" int kws_server_reset(kws_server* s) {
     KWS_CUDA_OK(cudaStreamSynchronize(w.cs));
   }
   return KWS_OK;
+}
+
+// The per-wave pointers of the record kernels, as of now: each wave's tail ping-pong half is the one its next chunk
+// reads (the captured graphs point at both halves, so writing there keeps them valid).
+static int upload_record_table(kws_server* s, cudaStream_t cs) {
+  KWS_REQUIRE(s != nullptr, "server is NULL");
+  for (const Wave& w : s->waves) KWS_REQUIRE(w.submitted == w.completed, "chunks are in flight");
+  KWS_CUDA_OK(cudaSetDevice(s->device));
+  for (size_t i = 0; i < s->waves.size(); ++i) s->record_table_host[i] = record_slots(s->waves[i].st);
+  KWS_CUDA_OK(cudaMemcpyAsync(s->record_table, s->record_table_host.data(), sizeof(RecordSlots) * s->waves.size(),
+                              cudaMemcpyHostToDevice, cs));
+  return KWS_OK;
+}
+
+extern "C" int kws_server_export(kws_server* s, const int64_t* ids, int64_t n, void* records, void* stream) {
+  clear_error();
+  cudaStream_t cs = static_cast<cudaStream_t>(stream);
+  int rc = upload_record_table(s, cs);
+  if (rc == KWS_OK)
+    rc = launch_record_export(s->waves[0].st, s->record_table, s->cfg.n_streams, ids, n, records, cs);
+  if (rc == KWS_OK) KWS_CUDA_OK(cudaStreamSynchronize(cs));
+  return rc;
+}
+
+extern "C" int kws_server_import(kws_server* s, const int64_t* ids, int64_t n, const void* records,
+                                 int32_t* status_out, void* stream) {
+  clear_error();
+  cudaStream_t cs = static_cast<cudaStream_t>(stream);
+  int rc = upload_record_table(s, cs);
+  if (rc == KWS_OK)
+    rc = launch_record_import(s->waves[0].st, s->record_table, s->cfg.n_streams, ids, n, records, status_out, cs);
+  if (rc == KWS_OK) KWS_CUDA_OK(cudaStreamSynchronize(cs));
+  return rc;
 }
 
 extern "C" kws_stream* kws_server_wave_stream(kws_server* s, int32_t wave) {

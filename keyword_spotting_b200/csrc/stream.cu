@@ -165,6 +165,183 @@ __global__ void zero_silent_state_kernel(float* state, long S, int layers, const
   if (silence[s]) state[idx] = 0.0f;
 }
 
+// ---- per-stream records (layout in include/kws_b200.h).  Every section starts and ends on a 16-byte boundary, so
+// both kernels move whole 16-byte pieces: one warp per record, lane-strided over its pieces.
+constexpr uint32_t kRecMagic = 0x5253574bu;   // "KWSR" as little-endian bytes
+constexpr uint32_t kRecVersion = 1;
+constexpr int kRecHeadPieces = 3;             // 48-byte header
+constexpr int kRecTailPieces = kTailCap * 2 / 16;
+
+struct RecordGeom {
+  long long total;                            // ids in [0, total)
+  long long per;                              // streams per object
+  int layers, W, fpad, max_frames, max_token;
+  int p_tail, p_slots, p_tok, pieces;         // section offsets in pieces (the state starts at kRecHeadPieces)
+  __device__ __forceinline__ uint4 head0() const { return make_uint4(kRecMagic, kRecVersion, layers, kHidden); }
+  __device__ __forceinline__ uint4 head1() const { return make_uint4(W, fpad, pieces * 16, 0); }
+};
+
+static RecordGeom record_geom(const kws_stream* st, long long total) {
+  RecordGeom g;
+  g.total = total;
+  g.per = st->S;
+  g.layers = st->model->cfg.num_layers;
+  g.W = st->cfg.window_chunks;
+  g.fpad = st->fpad;
+  g.max_frames = st->max_frames;
+  g.max_token = st->model->cfg.num_classes - 3;
+  g.p_tail = kRecHeadPieces + g.layers * kHidden / 4;
+  g.p_slots = g.p_tail + kRecTailPieces;
+  g.p_tok = g.p_slots + (g.W + 15) / 16;
+  g.pieces = g.p_tok + g.W * g.fpad / 16;
+  return g;
+}
+
+// v with bytes [keep, 16) zeroed
+__device__ __forceinline__ uint4 keep_bytes(uint4 v, int keep) {
+  uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int k = keep - 4 * i;
+    w[i] = k >= 4 ? w[i] : k <= 0 ? 0u : w[i] & ((1u << (8 * k)) - 1u);
+  }
+  return make_uint4(w[0], w[1], w[2], w[3]);
+}
+
+__device__ __forceinline__ bool record_target(const RecordGeom& g, const RecordSlots& one, const RecordSlots* table,
+                                              long long id, RecordSlots& o, long& s) {
+  if (id < 0 || id >= g.total) return false;
+  if (table) {
+    o = table[id / g.per];
+    s = static_cast<long>(id % g.per);
+  } else {
+    o = one;
+    s = static_cast<long>(id);
+  }
+  return true;
+}
+
+__global__ void __launch_bounds__(256)
+stream_export_kernel(const int64_t* __restrict__ ids, long n, const RecordGeom g, const RecordSlots one,
+                     const RecordSlots* __restrict__ table, uint4* __restrict__ records) {
+  const long r = (blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (r >= n) return;
+  uint4* rec = records + r * static_cast<long>(g.pieces);
+  const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
+  RecordSlots o;
+  long s = 0;
+  if (!record_target(g, one, table, ids[r], o, s)) {     // all zero: import rejects it (magic 0)
+    for (int p = lane; p < g.pieces; p += 32) rec[p] = zero;
+    return;
+  }
+  const int W = g.W, fpad = g.fpad;
+  const int tlen = o.tail_len[s], wn = o.win_n[s], wh = o.win_head[s];
+  const uint4* state = reinterpret_cast<const uint4*>(o.state + s * kHidden);
+  const uint4* tail = reinterpret_cast<const uint4*>(o.tail + s * kTailCap);
+  const unsigned char* sf = o.slot_frames + s * W;
+  const signed char* tok = o.tok + s * W * static_cast<long>(fpad);
+  for (int p = lane; p < g.pieces; p += 32) {
+    uint4 v = zero;
+    if (p < kRecHeadPieces) {
+      v = p == 0 ? g.head0() : p == 1 ? g.head1() : make_uint4(tlen, wn, 0u, 0u);
+    } else if (p < g.p_tail) {
+      const int q = p - kRecHeadPieces, l = q / (kHidden / 4), i = q % (kHidden / 4);
+      v = state[l * g.per * (kHidden / 4) + i];
+    } else if (p < g.p_slots) {
+      const int j = p - g.p_tail;                          // samples 8j .. 8j+7
+      if (8 * j < tlen) v = keep_bytes(tail[j], 2 * (tlen - 8 * j));
+    } else if (p < g.p_tok) {
+      uint32_t w[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+      for (int k = 0; k < 16; ++k) {
+        const int q = 16 * (p - g.p_slots) + k;            // window entry q, oldest first
+        if (q < wn) w[k >> 2] |= static_cast<uint32_t>(sf[(wh + q) % W]) << (8 * (k & 3));
+      }
+      v = make_uint4(w[0], w[1], w[2], w[3]);
+    } else {
+      const int b = 16 * (p - g.p_tok), q = b / fpad, t0 = b % fpad;
+      if (q < wn) {
+        const int sl = (wh + q) % W, f = sf[sl];
+        if (t0 < f) v = keep_bytes(*reinterpret_cast<const uint4*>(tok + sl * fpad + t0), f - t0);
+      }
+    }
+    rec[p] = v;
+  }
+}
+
+// Status per record: 0 imported, 1 id out of range, 2 header of another layout, 3 malformed field.  Every field is
+// checked before anything is written, so a rejected record leaves its stream untouched.
+__global__ void __launch_bounds__(256)
+stream_import_kernel(const int64_t* __restrict__ ids, long n, const RecordGeom g, const RecordSlots one,
+                     const RecordSlots* __restrict__ table, const uint4* __restrict__ records,
+                     int32_t* __restrict__ status) {
+  const long r = (blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (r >= n) return;
+  const uint4* rec = records + r * static_cast<long>(g.pieces);
+  const unsigned char* rsf = reinterpret_cast<const unsigned char*>(rec + g.p_slots);
+  const int W = g.W, fpad = g.fpad;
+  RecordSlots o;
+  long s = 0;
+  int st = 0, tlen = 0, wn = 0;
+  if (!record_target(g, one, table, ids[r], o, s)) {
+    st = 1;
+  } else {
+    const uint4 h0 = rec[0], h1 = rec[1], h2 = rec[2], e0 = g.head0(), e1 = g.head1();
+    tlen = static_cast<int>(h2.x);
+    wn = static_cast<int>(h2.y);
+    if (h0.x != e0.x || h0.y != e0.y || h0.z != e0.z || h0.w != e0.w || h1.x != e1.x || h1.y != e1.y || h1.z != e1.z) {
+      st = 2;
+    } else if (tlen < 0 || tlen >= kTailCap || wn < 0 || wn > W) {
+      st = 3;
+    } else {
+      bool bad = false;
+      for (int q = lane; q < wn; q += 32) bad |= rsf[q] > g.max_frames;
+      for (int p = g.p_tok + lane; p < g.pieces && !bad; p += 32) {
+        const int b = 16 * (p - g.p_tok), q = b / fpad, t0 = b % fpad;
+        if (q >= wn) break;                                // pieces only grow in q
+        const int f = rsf[q];
+        if (t0 >= f || f > g.max_frames) continue;
+        const uint4 v = rec[p];
+        const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int k = 0; k < 16; ++k) {
+          const int tk = static_cast<signed char>(w[k >> 2] >> (8 * (k & 3)));
+          bad |= t0 + k < f && (tk < -1 || tk > g.max_token);
+        }
+      }
+      if (__any_sync(0xffffffffu, bad)) st = 3;
+    }
+  }
+  if (lane == 0 && status) status[r] = st;
+  if (st != 0) return;
+  for (int p = lane; p < g.pieces; p += 32) {
+    if (p < kRecHeadPieces) continue;
+    if (p < g.p_tail) {
+      const int q = p - kRecHeadPieces, l = q / (kHidden / 4), i = q % (kHidden / 4);
+      reinterpret_cast<uint4*>(o.state + (static_cast<long>(l) * g.per + s) * kHidden)[i] = rec[p];
+    } else if (p < g.p_slots) {
+      const int j = p - g.p_tail;
+      reinterpret_cast<uint4*>(o.tail + s * kTailCap)[j] = keep_bytes(rec[p], 2 * (tlen - 8 * j));
+    } else if (p < g.p_tok) {
+      for (int k = 0; k < 16; ++k) {
+        const int q = 16 * (p - g.p_slots) + k;
+        if (q < W) o.slot_frames[s * W + q] = q < wn ? rsf[q] : 0;
+      }
+    } else {
+      const int b = 16 * (p - g.p_tok), q = b / fpad, t0 = b % fpad;
+      const int keep = q < wn ? rsf[q] - t0 : 0;
+      *reinterpret_cast<uint4*>(o.tok + (s * W + q) * static_cast<long>(fpad) + t0) = keep_bytes(rec[p], keep);
+    }
+  }
+  if (lane == 0) {
+    o.tail_len[s] = tlen;
+    o.win_head[s] = 0;
+    o.win_n[s] = wn;
+  }
+}
+
 template <typename T>
 static int dev_alloc(T** p, size_t n, bool zero) {
   *p = nullptr;
@@ -200,6 +377,48 @@ static void free_stream(kws_stream* st) {
 }
 
 static int frames_for_chunk(int chunk_len) { return frames_of(chunk_len + kTailCap - 1); }   // with the longest tail (399)
+
+RecordSlots record_slots(const kws_stream* st) {
+  RecordSlots o;
+  o.state = st->state;
+  o.tail = st->tail[st->cur];
+  o.tail_len = st->tail_len[st->cur];
+  o.tok = st->tok;
+  o.slot_frames = st->slot_frames;
+  o.win_head = st->win_head;
+  o.win_n = st->win_n;
+  return o;
+}
+
+int64_t record_bytes(const kws_stream* st) { return 16LL * record_geom(st, 0).pieces; }
+
+static int check_record_args(const kws_stream* st, const int64_t* ids, int64_t n, const void* records) {
+  KWS_REQUIRE(st != nullptr, "stream handle is NULL");
+  KWS_REQUIRE(n >= 0, "n must be >= 0");
+  KWS_REQUIRE(n == 0 || (ids != nullptr && records != nullptr), "ids / records are NULL");
+  KWS_REQUIRE(reinterpret_cast<uintptr_t>(records) % 16 == 0, "records must be 16-byte aligned");
+  return KWS_OK;
+}
+
+int launch_record_export(const kws_stream* st, const RecordSlots* table, int64_t total, const int64_t* ids, int64_t n,
+                         void* records, cudaStream_t cs) {
+  const int rc = check_record_args(st, ids, n, records);
+  if (rc != KWS_OK || n == 0) return rc;
+  stream_export_kernel<<<static_cast<unsigned>(ceil_div(n * 32, 256)), 256, 0, cs>>>(
+      ids, n, record_geom(st, total), record_slots(st), table, static_cast<uint4*>(records));
+  KWS_LAUNCH_OK("stream_export_kernel");
+  return KWS_OK;
+}
+
+int launch_record_import(const kws_stream* st, const RecordSlots* table, int64_t total, const int64_t* ids, int64_t n,
+                         const void* records, int32_t* status_out, cudaStream_t cs) {
+  const int rc = check_record_args(st, ids, n, records);
+  if (rc != KWS_OK || n == 0) return rc;
+  stream_import_kernel<<<static_cast<unsigned>(ceil_div(n * 32, 256)), 256, 0, cs>>>(
+      ids, n, record_geom(st, total), record_slots(st), table, static_cast<const uint4*>(records), status_out);
+  KWS_LAUNCH_OK("stream_import_kernel");
+  return KWS_OK;
+}
 
 }  // namespace kws
 
@@ -288,6 +507,23 @@ extern "C" int kws_stream_copy_state(kws_stream* st, float* state_out, void* str
                               sizeof(float) * st->S * st->model->cfg.num_layers * kHidden,
                               cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(stream)));
   return KWS_OK;
+}
+
+extern "C" int64_t kws_stream_record_bytes(const kws_stream* st) { return st ? record_bytes(st) : 0; }
+
+extern "C" int kws_stream_export(kws_stream* st, const int64_t* ids, int64_t n, void* records, void* stream) {
+  clear_error();
+  KWS_REQUIRE(st != nullptr, "stream handle is NULL");
+  KWS_CUDA_OK(cudaSetDevice(st->device));
+  return launch_record_export(st, nullptr, st->S, ids, n, records, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int kws_stream_import(kws_stream* st, const int64_t* ids, int64_t n, const void* records,
+                                 int32_t* status_out, void* stream) {
+  clear_error();
+  KWS_REQUIRE(st != nullptr, "stream handle is NULL");
+  KWS_CUDA_OK(cudaSetDevice(st->device));
+  return launch_record_import(st, nullptr, st->S, ids, n, records, status_out, static_cast<cudaStream_t>(stream));
 }
 
 // Debug: device time of the three parts of a step (front end incl. the fused pre-step | GRU layers | decode + trigger),

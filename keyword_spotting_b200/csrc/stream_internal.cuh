@@ -36,3 +36,27 @@ struct kws_stream {
   bool consumed_valid[2] = {false, false};
 };
 
+namespace kws {
+
+// Per-stream records (kws_stream_export / kws_stream_import, include/kws_b200.h): where the record kernels find the
+// carried state of one stream object.  tail / tail_len are the ping-pong half the next step reads (index cur).
+struct RecordSlots {
+  float* state = nullptr;
+  int16_t* tail = nullptr;
+  int32_t* tail_len = nullptr;
+  signed char* tok = nullptr;
+  unsigned char* slot_frames = nullptr;
+  int32_t* win_head = nullptr;
+  int32_t* win_n = nullptr;
+};
+RecordSlots record_slots(const kws_stream* st);
+int64_t record_bytes(const kws_stream* st);
+// Records of ids in [0, total).  table == nullptr: the ids are streams of `st` itself (total = st->S).  Otherwise id g
+// is stream g % st->S of the object table[g / st->S] (DEVICE), every object laid out as `st`.
+int launch_record_export(const kws_stream* st, const RecordSlots* table, int64_t total, const int64_t* ids, int64_t n,
+                         void* records, cudaStream_t cs);
+int launch_record_import(const kws_stream* st, const RecordSlots* table, int64_t total, const int64_t* ids, int64_t n,
+                         const void* records, int32_t* status_out, cudaStream_t cs);
+
+}  // namespace kws
+

@@ -15,6 +15,7 @@ import torch
 
 from . import _lib, _tensors
 from .rnn_ctc import DeployModel
+from .streaming import raise_rejected, record_ids, record_input
 
 
 class WaveServer:
@@ -142,3 +143,30 @@ class WaveServer:
                                                        counts[w * Sw:].data_ptr(), _tensors.stream_ptr(self.device)))
             torch.cuda.synchronize(self.device)
         return _tensors.to_host(labels), _tensors.to_host(counts)
+
+    # -- per-stream records over global stream ids (kws_server_export / kws_server_import)
+    @property
+    def record_bytes(self) -> int:
+        """Bytes of one stream's record (the layout of ``StreamingDetector.export_streams``)."""
+        return int(self._lib.kws_stream_record_bytes(self._lib.kws_server_wave_stream(self._handle, 0)))
+
+    def export_streams(self, ids) -> torch.Tensor:
+        """Records of global streams ``ids`` -> ``torch.uint8`` CUDA ``[n, record_bytes]``.  Nothing may be in
+        flight; returns when the records are written."""
+        idx = record_ids(ids, self.n_streams, self.device, distinct=False)
+        out = torch.empty((idx.numel(), self.record_bytes), dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.kws_server_export(self._handle, _tensors.ptr(idx), idx.numel(), _tensors.ptr(out),
+                                                   _tensors.stream_ptr(self.device)))
+        return out
+
+    def import_streams(self, ids, records):
+        """Make global streams ``ids`` continue from ``records`` (host or device); the next ``submit`` sees them.
+        Nothing may be in flight.  Raises ``InvalidArgumentError`` naming every rejected record."""
+        idx = record_ids(ids, self.n_streams, self.device, distinct=True)
+        recs = record_input(records, idx.numel(), self.record_bytes, self.device)
+        status = torch.empty(idx.numel(), dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.kws_server_import(self._handle, _tensors.ptr(idx), idx.numel(), _tensors.ptr(recs),
+                                                   _tensors.ptr(status), _tensors.stream_ptr(self.device)))
+        raise_rejected(idx, status)

@@ -114,3 +114,77 @@ class StreamingDetector:
                                                    _tensors.stream_ptr(self.device)))
         torch.cuda.current_stream(self.device).synchronize()
         return _tensors.to_host(labels), _tensors.to_host(counts)
+
+    # -- per-stream records (kws_stream_export / kws_stream_import)
+    @property
+    def record_bytes(self) -> int:
+        """Bytes of one stream's record (layout in include/kws_b200.h)."""
+        return int(self._lib.kws_stream_record_bytes(self._handle))
+
+    def export_streams(self, ids) -> torch.Tensor:
+        """Records of streams ``ids`` -> ``torch.uint8`` CUDA ``[n, record_bytes]``: everything each stream carries
+        into its next chunk, as plain bytes (move them to another GPU with ``.to(device)``, or to disk)."""
+        idx = record_ids(ids, self.n_streams, self.device, distinct=False)
+        out = torch.empty((idx.numel(), self.record_bytes), dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.kws_stream_export(self._handle, _tensors.ptr(idx), idx.numel(), _tensors.ptr(out),
+                                                   _tensors.stream_ptr(self.device)))
+        return out
+
+    def import_streams(self, ids, records):
+        """Make streams ``ids`` continue from ``records`` (from ``export_streams`` of an object of the same layout,
+        host or device).  Raises ``InvalidArgumentError`` naming every rejected record; those streams are left as
+        they were.  Reads the status back, so it synchronises the current stream."""
+        idx = record_ids(ids, self.n_streams, self.device, distinct=True)
+        recs = record_input(records, idx.numel(), self.record_bytes, self.device)
+        status = torch.empty(idx.numel(), dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.kws_stream_import(self._handle, _tensors.ptr(idx), idx.numel(), _tensors.ptr(recs),
+                                                   _tensors.ptr(status), _tensors.stream_ptr(self.device)))
+        raise_rejected(idx, status)
+
+
+_REJECTED = {1: "id out of range", 2: "header does not match this object", 3: "malformed field"}
+
+
+def record_ids(ids, n_streams: int, device, distinct: bool) -> torch.Tensor:
+    """ids -> int64 CUDA [n].  Host ids are validated (integers in [0, n_streams), distinct when ``distinct``); CUDA
+    ids are left to the kernels (reading them here would synchronise the stream)."""
+    if not _tensors.is_host(ids):
+        if ids.dim() != 1 or ids.dtype.is_floating_point or ids.dtype.is_complex or ids.dtype == torch.bool:
+            raise _lib.InvalidArgumentError("ids must be integers [n], got %s %r" % (ids.dtype, tuple(ids.shape)))
+        return _tensors.to_device(ids, torch.int64, device)
+    a = np.asarray(ids.numpy() if isinstance(ids, torch.Tensor) else ids)
+    if a.ndim == 1 and a.size == 0:
+        a = a.astype(np.int64)
+    if a.ndim != 1 or a.dtype.kind not in "iu":
+        raise _lib.InvalidArgumentError("ids must be integers [n], got %s %r" % (a.dtype, a.shape))
+    if a.size and (a.min() < 0 or a.max() >= n_streams):
+        raise _lib.InvalidArgumentError("ids must lie in [0, %d), got [%d, %d]" % (n_streams, a.min(), a.max()))
+    if distinct and np.unique(a).size != a.size:
+        raise _lib.InvalidArgumentError("ids must be distinct")
+    return _tensors.to_device(a.astype(np.int64), torch.int64, device)
+
+
+def record_input(records, n: int, record_bytes: int, device) -> torch.Tensor:
+    """uint8 records (CUDA or host tensor, numpy array) of n * record_bytes bytes -> CUDA [n, record_bytes]."""
+    if isinstance(records, torch.Tensor):
+        ok = records.dtype == torch.uint8 and records.numel() == n * record_bytes
+    else:
+        records = np.asarray(records)
+        if not records.flags.writeable:           # e.g. np.frombuffer of bytes read from a file
+            records = records.copy()
+        ok = records.dtype == np.uint8 and records.size == n * record_bytes
+    if not ok:
+        raise _lib.InvalidArgumentError("records must be uint8 [%d, %d], got %s %r" % (n, record_bytes, records.dtype,
+                                                                                     tuple(records.shape)))
+    return _tensors.to_device(records, torch.uint8, device).reshape(n, record_bytes)
+
+
+def raise_rejected(ids: torch.Tensor, status: torch.Tensor):
+    st = _tensors.to_host(status)
+    bad = np.nonzero(st)[0]
+    if bad.size:
+        idv = _tensors.to_host(ids)
+        raise _lib.InvalidArgumentError("%d record(s) rejected: %s" % (bad.size, "; ".join(
+            "entry %d (id %d): %s" % (i, idv[i], _REJECTED.get(int(st[i]), "status %d" % st[i])) for i in bad[:16])))
