@@ -59,8 +59,8 @@ typedef struct kws_model_config {
   int32_t hidden;      /* 128 -- the only size the kernels are built for        */
   int32_t num_layers;  /* 2                                                     */
   int32_t num_classes; /* 6                                                     */
-  int32_t fft_size;    /* 400                                                   */
-  int32_t hop_size;    /* 160                                                   */
+  int32_t fft_size;    /* 400; any of 16..512 (frame, rfft length)              */
+  int32_t hop_size;    /* 160; any of 1..fft_size                               */
 } kws_model_config;
 
 /* HOST pointers to fp32 weights in the TF variable layout (row = input index):
@@ -88,15 +88,18 @@ typedef enum kws_precision {
   KWS_PRECISION_TC_FP16 = 1
 } kws_precision;
 
-/* Formulation of the front end (K1).  Both produce the same mel frames (parity tests run on both).
+/* Formulation of the front end (K1) of a 400/160 model.  Both produce the same mel frames (parity tests run on both).
  *   KWS_FRONTEND_FFT (default): packed-real 20x20 FFT on the CUDA cores / shared memory (csrc/frontend.cu).
  *   KWS_FRONTEND_TC: hop-block partial DFTs on tcgen05 with the twiddles in tensor memory (csrc/frontend_tc.cu);
- *     int16 PCM and n_mel <= 64 only -- other inputs run on the FFT kernel.  Same speed on B200, see DESIGN.md. */
+ *     int16 PCM and n_mel <= 64 only -- other inputs run on the FFT kernel.  Same speed on B200, see DESIGN.md.
+ * Models of any other fft_size / hop_size run the general front end (csrc/frontend_dft.cu: the real DFT as one
+ * tcgen05 product per 128 frames), whatever kws_model_set_frontend says; its fp32 PCM must lie in (-2, 2). */
 typedef enum kws_frontend {
   KWS_FRONTEND_FFT = 0,
   KWS_FRONTEND_TC = 1
 } kws_frontend;
 
+/* Rejects (KWS_ERR_INVALID_ARGUMENT) fft_size outside [16, 512] and hop_size outside [1, fft_size]. */
 int kws_model_create(const kws_model_config* cfg, const kws_model_weights* host_weights,
                      int device, kws_model** out);
 int kws_model_set_frontend(kws_model* m, int frontend);
@@ -259,15 +262,16 @@ int kws_stream_labels(kws_stream* st, int32_t* labels_out, int32_t max_labels,
 /* Per-stream records: everything one stream carries from one chunk to the next, as a fixed-size, self-describing
  * byte block, so that chosen streams can be saved, restored, compared or moved to another object or GPU between
  * chunks.  Little-endian; every section is a multiple of 16 bytes (offsets in bytes, L = num_layers, H = hidden,
- * W = window_chunks, Wp = W rounded up to 16):
+ * W = window_chunks, Wp = W rounded up to 16, T = the tail capacity max(400, fft_size rounded up to 8)):
  *     0  uint32 magic 0x5253574B ("KWSR"), uint32 version 1, int32 L, int32 H
  *    16  int32 W, int32 fpad (token slots per window entry, a multiple of 16), int32 record bytes, 0
- *    32  int32 tail_len (carried PCM samples, 0..399), int32 win_n (window entries in use, 0..W), 0, 0
+ *    32  int32 tail_len (carried PCM samples, 0..fft_size - 1), int32 win_n (window entries in use, 0..W), 0, 0
  *    48  GRU state [L][H] fp32, raw bits
- *    48 + 512 L           carried PCM tail [400] int16: the first tail_len samples
- *    48 + 512 L + 800     slot_frames [Wp] uint8: frames of window entry q, oldest entry first
- *    48 + 512 L + 800 + Wp  tokens [W][fpad] int8: per frame of entry q, the above-threshold winner class - 1, or -1
- * record bytes = 848 + 512 L + Wp + W fpad (2368 at L = 2, W = 15, max_chunk = 4800).  Records are canonical: every
+ *    48 + 512 L           carried PCM tail [T] int16: the first tail_len samples
+ *    48 + 512 L + 2T      slot_frames [Wp] uint8: frames of window entry q, oldest entry first
+ *    48 + 512 L + 2T + Wp  tokens [W][fpad] int8: per frame of entry q, the above-threshold winner class - 1, or -1
+ * record bytes = 48 + 512 L + 2T + Wp + W fpad (2368 at L = 2, W = 15, max_chunk = 4800, fft_size <= 400: T = 400).
+ * A record of another tail capacity differs in the record-bytes field of its header.  Records are canonical: every
  * byte that holds no state is zero (samples past tail_len, tokens past slot_frames[q], entries past win_n, padding),
  * so the record of a stream does not depend on where its window ring starts, and export -> import -> export gives
  * the same bytes.  Per-chunk scratch (VAD flags, frame counts, triggers, mel, probabilities) is not state: each step
@@ -279,7 +283,7 @@ int kws_stream_labels(kws_stream* st, int32_t* labels_out, int32_t max_labels,
  * Export of an id outside [0, n_streams) writes an all-zero record, which import rejects.
  * Import treats every record as input from outside the program (it may come from disk).  status_out: DEVICE int32
  * [n] or NULL; 0 = imported, 1 = id outside [0, n_streams), 2 = header does not match this object (magic, version,
- * L, H, W, fpad or record bytes), 3 = malformed field (tail_len outside [0, 399], win_n outside [0, W], a used
+ * L, H, W, fpad or record bytes), 3 = malformed field (tail_len outside [0, fft_size - 1], win_n outside [0, W], a used
  * slot_frames above kws_stream_max_frames(), a used token outside [-1, num_classes - 3]).  A rejected record
  * leaves its stream untouched.  An imported stream continues bit for bit as the exported one would have.        */
 int64_t kws_stream_record_bytes(const kws_stream* st);

@@ -14,7 +14,7 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.path.join(HERE, "libkws_b200.so")
-SOURCES = ["api.cu", "posenc.cu", "octbit.cu", "octbit_tc.cu", "frontend.cu", "frontend_tc.cu", "gru.cu", "gru_octbit.cu", "gru_tc.cu", "decode.cu", "stream.cu", "server.cu", "tc_debug.cu", "attention.cu", "attention_tc.cu"]
+SOURCES = ["api.cu", "posenc.cu", "octbit.cu", "octbit_tc.cu", "frontend.cu", "frontend_tc.cu", "frontend_dft.cu", "gru.cu", "gru_octbit.cu", "gru_tc.cu", "decode.cu", "stream.cu", "server.cu", "tc_debug.cu", "attention.cu", "attention_tc.cu"]
 OBJ_DIR = os.path.join(HERE, "build")
 _ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]   # B200 only
 NVCC_COMPILE_FLAGS = _ARCH + ["-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]

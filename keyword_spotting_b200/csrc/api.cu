@@ -62,6 +62,7 @@ static void free_model(kws_model* m) {
   cudaFree(m->mel_basis);
   cudaFree(m->mel.quads);
   free_frontend_tc_tables(m);
+  free_frontend_dft_tables(m);
   cudaFree(m->twiddle400);
   for (int l = 0; l < kMaxLayers; ++l) {
     cudaFree(m->layer[l].gates_kernel);
@@ -107,8 +108,9 @@ extern "C" int kws_model_create(const kws_model_config* cfg, const kws_model_wei
   KWS_REQUIRE(cfg->num_layers >= 1 && cfg->num_layers <= kMaxLayers, "num_layers must be in [1, %d]", kMaxLayers);
   KWS_REQUIRE(cfg->num_classes >= 2 && cfg->num_classes <= kMaxClasses, "num_classes must be in [2, %d]", kMaxClasses);
   KWS_REQUIRE(cfg->n_mel >= 1 && cfg->n_mel <= kMaxMel, "n_mel must be in [1, %d]", kMaxMel);
-  KWS_REQUIRE(cfg->fft_size == kFft && cfg->hop_size == kHop,
-              "the front end is built for fft_size=%d hop_size=%d (config/rnn_config.py:57-58)", kFft, kHop);
+  KWS_REQUIRE(cfg->fft_size >= 16 && cfg->fft_size <= 512 && cfg->hop_size >= 1 && cfg->hop_size <= cfg->fft_size,
+              "fft_size must be in [16, 512] and hop_size in [1, fft_size] (got fft_size=%d hop_size=%d)",
+              cfg->fft_size, cfg->hop_size);
   KWS_REQUIRE(w->mel_basis && w->fc_w && w->fc_b, "NULL weight pointer");
   for (int l = 0; l < cfg->num_layers; ++l)
     KWS_REQUIRE(w->gates_kernel[l] && w->gates_bias[l] && w->cand_kernel[l] && w->cand_bias[l],
@@ -126,21 +128,23 @@ extern "C" int kws_model_create(const kws_model_config* cfg, const kws_model_wei
   m->device = device;
   m->frontend = default_frontend();
   const int M = cfg->n_mel, H = kHidden, C = cfg->num_classes;
-  int rc = upload(&m->mel_basis, w->mel_basis, static_cast<size_t>(kBins) * M);
-  {
+  int rc = upload(&m->mel_basis, w->mel_basis, static_cast<size_t>(cfg->fft_size / 2 + 1) * M);
+  if (frontend_is_default_frame(m)) {
     // non-zero part of the basis as balanced per-warp quad lists (exact for any basis: zeros contribute nothing)
     std::vector<kws::MelQuad> quads;
     kws::build_mel_quads(w->mel_basis, M, &quads, &m->mel.quads_per_warp);
     if (rc == KWS_OK) rc = upload(&m->mel.quads, quads.data(), quads.size());
+    if (rc == KWS_OK) rc = build_frontend_tc_tables(m, w->mel_basis);
+    std::vector<float2> tw(20 * 52);          // periodic k2-major table of W400^(n1*k2) (fft400.cuh: kTwStride = 52)
+    for (int k2 = 0; k2 < 20; ++k2)
+      for (int j = 0; j < 52; ++j) {
+        const double a = -2.0 * M_PI * static_cast<double>((j % 20) * k2) / kFft;
+        tw[k2 * 52 + j] = make_float2(static_cast<float>(std::cos(a)), static_cast<float>(std::sin(a)));
+      }
+    if (rc == KWS_OK) rc = upload(&m->twiddle400, tw.data(), tw.size());
+  } else if (rc == KWS_OK) {
+    rc = build_frontend_dft_tables(m, w->mel_basis);
   }
-  if (rc == KWS_OK) rc = build_frontend_tc_tables(m, w->mel_basis);
-  std::vector<float2> tw(20 * 52);          // periodic k2-major table of W400^(n1*k2) (fft400.cuh: kTwStride = 52)
-  for (int k2 = 0; k2 < 20; ++k2)
-    for (int j = 0; j < 52; ++j) {
-      const double a = -2.0 * M_PI * static_cast<double>((j % 20) * k2) / kFft;
-      tw[k2 * 52 + j] = make_float2(static_cast<float>(std::cos(a)), static_cast<float>(std::sin(a)));
-    }
-  if (rc == KWS_OK) rc = upload(&m->twiddle400, tw.data(), tw.size());
   for (int l = 0; l < cfg->num_layers && rc == KWS_OK; ++l) {
     const int in = l == 0 ? M : H;
     m->layer[l].in_dim = in;

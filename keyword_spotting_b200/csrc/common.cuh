@@ -110,6 +110,12 @@ struct MelSparse {               // non-zero part of the mel basis as per-warp l
   int quads_per_warp = 0;
 };
 
+struct FrontendDftTables {       // general front end (frontend_dft.cu): every frame other than 400/160
+  void* tw = nullptr;            // fp16 twiddles [chunks][hi | lo][ncols x 32], canonical K-major
+  void* mel_seg = nullptr;       // int4 [n_mel]: {first bin, bins, offset into mel_w, 0}
+  float* mel_w = nullptr;        // the bands' non-zero spans, concatenated
+};
+
 struct FrontendTcTables {        // tensor-core front end (frontend_tc.cu)
   bool ready = false;
   uint32_t* tw = nullptr;        // twiddles as TMEM rows [2 tiles][2 parts][128][40]
@@ -125,10 +131,12 @@ struct kws_model {
   int device = 0;
   int precision = KWS_PRECISION_TC_FP16;
   int frontend = KWS_FRONTEND_FFT;   // K1 formulation (kws_model_set_frontend)
-  float* mel_basis = nullptr;     // [201, M] dense, as given
+  float* mel_basis = nullptr;     // [fft/2+1, M] dense, as given
+  // 400/160 models: the FFT and tensor-core front ends' tables; every other frame: the DFT front end's (fe_dft.tw set)
   kws::MelSparse mel;
   kws::FrontendTcTables fe_tc;
   float2* twiddle400 = nullptr;   // [20*52] periodic k2-major twiddles (fft400.cuh kTwStride)
+  kws::FrontendDftTables fe_dft;
   kws::LayerWeights layer[kws::kMaxLayers];
   float* fc_w = nullptr;          // [H, C]
   float* fc_b = nullptr;          // [C]
@@ -173,19 +181,27 @@ struct PcmSource {
 
 // Chunk rules of the front end and the streaming server.  Frames of a signal of `total` samples (utils/stft.py:60-61),
 // 0 below one frame:
-__host__ __device__ __forceinline__ int frames_of(int total) { return total >= kFft ? 1 + (total - kFft) / kHop : 0; }
-// samples carried into the next chunk (detector.py:181-182): the last (total - 400) % 160 + 240, or all of them while
-// no frame fits
-__host__ __device__ __forceinline__ int tail_keep(int total) {
-  return total >= kFft ? (total - kFft) % kHop + (kFft - kHop) : total;
+__host__ __device__ __forceinline__ int frames_of(int total, int fft, int hop) {
+  return total >= fft ? 1 + (total - fft) / hop : 0;
 }
+// samples carried into the next chunk (detector.py:181-182): the last (total - fft) % hop + fft - hop, or all of them
+// while no frame fits
+__host__ __device__ __forceinline__ int tail_keep(int total, int fft, int hop) {
+  return total >= fft ? (total - fft) % hop + (fft - hop) : total;
+}
+// the same at 400/160, the frame of the FFT and tensor-core front ends
+__host__ __device__ __forceinline__ int frames_of(int total) { return frames_of(total, kFft, kHop); }
+__host__ __device__ __forceinline__ int tail_keep(int total) { return tail_keep(total, kFft, kHop); }
+// Longest carried tail of a frame of fft samples is fft - 1; its buffer holds max(400, ceil8(fft)) samples per stream
+// (400 keeps the record layout of every fft_size <= 400, 16-byte pieces keep the record kernels' moves whole).
+inline int tail_capacity(int fft) { return fft <= 400 ? 400 : (fft + 7) / 8 * 8; }
 
 // The streaming server's per-chunk pre-step: VAD flag, frame count and next carried tail.  Fused into the front end
 // when the chunk fits one work item (frontend_can_fuse_pre), so that the CTA that stages the chunk produces them and
 // the PCM is read once; stream_pre_kernel (stream.cu) otherwise.
 struct FrontendPre {
   long long vad_limit = 0;            // speech iff sum|x_i16| > vad_limit
-  int16_t* tail_next = nullptr;       // [S, 400]
+  int16_t* tail_next = nullptr;       // [S, tail capacity] (400 whenever the pre-step is fused)
   int32_t* len_next = nullptr;        // [S]
   unsigned char* silence = nullptr;   // [S]
   // stream s's record, from the sum of |x_i16| over its new samples; its frame count goes to nframes[s]
@@ -198,6 +214,10 @@ struct FrontendPre {
 bool frontend_can_fuse_pre(const kws_model* m, int chunk_len, int tail_cap);
 int build_frontend_tc_tables(kws_model* m, const float* basis /*[201, M] host*/);
 void free_frontend_tc_tables(kws_model* m);
+// 400/160 runs the FFT / tensor-core front ends; every other frame runs the DFT front end (frontend_dft.cu)
+inline bool frontend_is_default_frame(const kws_model* m) { return m->cfg.fft_size == kFft && m->cfg.hop_size == kHop; }
+int build_frontend_dft_tables(kws_model* m, const float* basis /*[fft/2+1, M] host*/);
+void free_frontend_dft_tables(kws_model* m);
 bool frontend_uses_tc(const kws_model* m, int pcm_dtype);
 int default_frontend();           // KWS_FRONTEND=tc|fft in the environment, else fft
 int frontend_tc_item_frames();

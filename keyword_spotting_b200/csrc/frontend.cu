@@ -415,6 +415,7 @@ static size_t frontend_smem_bytes(const kws_model* m) {
 }
 
 bool frontend_can_fuse_pre(const kws_model* m, int chunk_len, int tail_cap) {
+  if (!frontend_is_default_frame(m)) return false;    // the DFT front end leaves the pre-step to stream_pre_kernel
   // the whole [tail | chunk] must fit one work item: 32 frames / 5360 samples here, 30 frames (<= 5199 samples) on
   // the tensor-core kernel
   if (frontend_uses_tc(m, KWS_PCM_I16)) return chunk_len + tail_cap - 1 <= kFft + kHop * (frontend_tc_item_frames() - 1) + kHop - 1;
@@ -446,6 +447,7 @@ int launch_frontend(const kws_model* m, const PcmSource& src, int64_t S, int32_t
     if (src.lengths) return fail(KWS_ERR_INVALID_ARGUMENT, "the fused pre-step takes no stream lengths");
     io.pre = *pre;
   }
+  if (!frontend_is_default_frame(m)) return launch_frontend_dft(m, io, st);
   if (tc) return launch_frontend_tc(m, io, st);
 
   FrontendParams p{io};

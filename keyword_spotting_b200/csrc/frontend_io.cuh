@@ -1,4 +1,4 @@
-// What the two front-end kernels (frontend.cu: FFT, frontend_tc.cu: tensor cores) share around their transforms: the
+// What the front-end kernels (frontend.cu: FFT, frontend_tc.cu: tensor cores, frontend_dft.cu: other frames) share around their transforms: the
 // launch parameters, a stream's length and frame count, the copy of a finished [frames, n_mel] tile into mel_out in
 // its three layouts, the zero rows past a stream's length, and the fused pre-step's per-stream record.
 #pragma once
@@ -96,5 +96,6 @@ struct FrontendIo {
 };
 
 int launch_frontend_tc(const kws_model* m, const FrontendIo& io, cudaStream_t st);   // frontend_tc.cu
+int launch_frontend_dft(const kws_model* m, const FrontendIo& io, cudaStream_t st);  // frontend_dft.cu
 
 }  // namespace kws

@@ -5,7 +5,8 @@
 //   1. VAD on the NEW samples: sum|x| > 30 (utils/basic_vad.py:17-18, detector.py:168).
 //      Done in exact integer arithmetic on the int16 PCM: sum|x_i16| > 30*32768.
 //      Silence -> GRU state zeroed and decision window cleared (detector.py:171-177).
-//   2. carried tail ++ chunk; keep (len-400)%160+240 samples for next time (detector.py:179-183)
+//   2. carried tail ++ chunk; keep (len-fft)%hop+fft-hop samples for next time (detector.py:179-183), (len-400)%160+240
+//      at the default frame
 //   3. model call on the concatenation (detector.py:190-193)         -> K1, K2+K3
 //   4. window.add(softmax) with at most 15 chunks (utils/queue.py:16-38, detector.py:195)
 //   5. ctc_decode2 over the whole window (detector.py:197-200), ctc_predict(.., '1233')
@@ -23,12 +24,20 @@
 
 namespace kws {
 
-constexpr int kTailCap = 400;
+constexpr int kTailCap = 400;   // carried-tail capacity at the default frame (tail_capacity(400))
 
-// One warp per stream: the pre-step of a chunk that the front end cannot take in one work item.
+// The frame of a model other than 400/160, and its carried-tail capacity.
+struct ChunkRule {
+  int fft, hop, tail_cap;
+};
+
+// One warp per stream: the pre-step of a chunk that the front end cannot take in one work item.  kDefault: the
+// 400/160 frame as compile-time constants (rule unused); otherwise the model's frame from rule.
+template <bool kDefault>
 __global__ void __launch_bounds__(256)
 stream_pre_kernel(const int16_t* __restrict__ pcm, long ld, int chunk_len, long S, const int16_t* __restrict__ tail_cur,
-                  const int* __restrict__ len_cur, const FrontendPre pre, int* __restrict__ nframes, int max_frames) {
+                  const int* __restrict__ len_cur, const FrontendPre pre, int* __restrict__ nframes, int max_frames,
+                  const ChunkRule rule) {
   const long s = (blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (s >= S) return;
@@ -54,11 +63,12 @@ stream_pre_kernel(const int16_t* __restrict__ pcm, long ld, int chunk_len, long 
   for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
   const int head = len_cur[s];
   const int total = head + chunk_len;
-  const int nfr = frames_of(total);
-  const int keep = tail_keep(total);
+  const int nfr = kDefault ? frames_of(total) : frames_of(total, rule.fft, rule.hop);
+  const int keep = kDefault ? tail_keep(total) : tail_keep(total, rule.fft, rule.hop);
   if (lane == 0) pre.record(s, sum, nfr < max_frames ? nfr : max_frames, keep, nframes);
-  const int16_t* tcur = tail_cur + s * kTailCap;
-  int16_t* tnext = pre.tail_next + s * kTailCap;
+  const long cap = kDefault ? kTailCap : rule.tail_cap;
+  const int16_t* tcur = tail_cur + s * cap;
+  int16_t* tnext = pre.tail_next + s * cap;
   for (int i = lane; i < keep; i += 32) {
     const int gidx = total - keep + i;
     tnext[i] = gidx < head ? tcur[gidx] : row[gidx - head];
@@ -170,12 +180,12 @@ __global__ void zero_silent_state_kernel(float* state, long S, int layers, const
 constexpr uint32_t kRecMagic = 0x5253574bu;   // "KWSR" as little-endian bytes
 constexpr uint32_t kRecVersion = 1;
 constexpr int kRecHeadPieces = 3;             // 48-byte header
-constexpr int kRecTailPieces = kTailCap * 2 / 16;
 
 struct RecordGeom {
   long long total;                            // ids in [0, total)
   long long per;                              // streams per object
   int layers, W, fpad, max_frames, max_token;
+  int fft, tail_cap;                          // tail_len < fft; the tail section holds tail_cap samples
   int p_tail, p_slots, p_tok, pieces;         // section offsets in pieces (the state starts at kRecHeadPieces)
   __device__ __forceinline__ uint4 head0() const { return make_uint4(kRecMagic, kRecVersion, layers, kHidden); }
   __device__ __forceinline__ uint4 head1() const { return make_uint4(W, fpad, pieces * 16, 0); }
@@ -190,8 +200,10 @@ static RecordGeom record_geom(const kws_stream* st, long long total) {
   g.fpad = st->fpad;
   g.max_frames = st->max_frames;
   g.max_token = st->model->cfg.num_classes - 3;
+  g.fft = st->model->cfg.fft_size;
+  g.tail_cap = st->tail_cap;
   g.p_tail = kRecHeadPieces + g.layers * kHidden / 4;
-  g.p_slots = g.p_tail + kRecTailPieces;
+  g.p_slots = g.p_tail + g.tail_cap / 8;
   g.p_tok = g.p_slots + (g.W + 15) / 16;
   g.pieces = g.p_tok + g.W * g.fpad / 16;
   return g;
@@ -238,7 +250,7 @@ stream_export_kernel(const int64_t* __restrict__ ids, long n, const RecordGeom g
   const int W = g.W, fpad = g.fpad;
   const int tlen = o.tail_len[s], wn = o.win_n[s], wh = o.win_head[s];
   const uint4* state = reinterpret_cast<const uint4*>(o.state + s * kHidden);
-  const uint4* tail = reinterpret_cast<const uint4*>(o.tail + s * kTailCap);
+  const uint4* tail = reinterpret_cast<const uint4*>(o.tail + s * static_cast<long>(g.tail_cap));
   const unsigned char* sf = o.slot_frames + s * W;
   const signed char* tok = o.tok + s * W * static_cast<long>(fpad);
   for (int p = lane; p < g.pieces; p += 32) {
@@ -293,7 +305,7 @@ stream_import_kernel(const int64_t* __restrict__ ids, long n, const RecordGeom g
     wn = static_cast<int>(h2.y);
     if (h0.x != e0.x || h0.y != e0.y || h0.z != e0.z || h0.w != e0.w || h1.x != e1.x || h1.y != e1.y || h1.z != e1.z) {
       st = 2;
-    } else if (tlen < 0 || tlen >= kTailCap || wn < 0 || wn > W) {
+    } else if (tlen < 0 || tlen >= g.fft || wn < 0 || wn > W) {
       st = 3;
     } else {
       bool bad = false;
@@ -323,7 +335,7 @@ stream_import_kernel(const int64_t* __restrict__ ids, long n, const RecordGeom g
       reinterpret_cast<uint4*>(o.state + (static_cast<long>(l) * g.per + s) * kHidden)[i] = rec[p];
     } else if (p < g.p_slots) {
       const int j = p - g.p_tail;
-      reinterpret_cast<uint4*>(o.tail + s * kTailCap)[j] = keep_bytes(rec[p], 2 * (tlen - 8 * j));
+      reinterpret_cast<uint4*>(o.tail + s * static_cast<long>(g.tail_cap))[j] = keep_bytes(rec[p], 2 * (tlen - 8 * j));
     } else if (p < g.p_tok) {
       for (int k = 0; k < 16; ++k) {
         const int q = 16 * (p - g.p_slots) + k;
@@ -376,7 +388,11 @@ static void free_stream(kws_stream* st) {
   delete st;
 }
 
-static int frames_for_chunk(int chunk_len) { return frames_of(chunk_len + kTailCap - 1); }   // with the longest tail (399)
+// frames of a chunk with the longest carried tail (fft - 1 samples)
+static int frames_for_chunk(const kws_model* m, int chunk_len) {
+  const int fft = m->cfg.fft_size;
+  return frames_of(chunk_len + fft - 1, fft, m->cfg.hop_size);
+}
 
 RecordSlots record_slots(const kws_stream* st) {
   RecordSlots o;
@@ -435,7 +451,7 @@ extern "C" int kws_stream_create(kws_model* m, const kws_stream_config* cfg, kws
   KWS_REQUIRE(m->cfg.num_classes >= 3 && m->cfg.num_classes <= 11, "streaming decode needs 3..11 classes");
   KWS_REQUIRE(std::memchr(cfg->keyword, 0, sizeof(cfg->keyword)) != nullptr && std::strlen(cfg->keyword) <= 16,
               "keyword must be a NUL-terminated string of at most 16 characters");
-  const int mf = frames_for_chunk(cfg->max_chunk);
+  const int mf = frames_for_chunk(m, cfg->max_chunk);
   KWS_REQUIRE(mf <= 255, "max_chunk produces more than 255 frames per chunk");
   KWS_CUDA_OK(cudaSetDevice(m->device));
   kws_stream* st = new kws_stream();
@@ -444,6 +460,7 @@ extern "C" int kws_stream_create(kws_model* m, const kws_stream_config* cfg, kws
   st->cfg = *cfg;
   st->S = cfg->n_streams;
   st->max_frames = mf;
+  st->tail_cap = tail_capacity(m->cfg.fft_size);
   st->fpad = (mf + 15) / 16 * 16;
   if (st->fpad == 0) st->fpad = 16;
   st->kw = dec::parse_keyword(cfg->keyword);
@@ -451,7 +468,7 @@ extern "C" int kws_stream_create(kws_model* m, const kws_stream_config* cfg, kws
   const int L = m->cfg.num_layers, C = m->cfg.num_classes, M = m->cfg.n_mel, W = cfg->window_chunks;
   int rc = dev_alloc(&st->state, S * L * kHidden, true);
   for (int i = 0; i < 2 && rc == KWS_OK; ++i) {
-    rc = dev_alloc(&st->tail[i], S * kTailCap, true);
+    rc = dev_alloc(&st->tail[i], S * st->tail_cap, true);
     if (rc == KWS_OK) rc = dev_alloc(&st->tail_len[i], S, true);
   }
   if (rc == KWS_OK) rc = dev_alloc(&st->silence, S, true);
@@ -560,7 +577,7 @@ extern "C" int kws_stream_step(kws_stream* st, const int16_t* pcm, int32_t chunk
   KWS_CUDA_OK(cudaSetDevice(m->device));
   const long S = st->S;
   const int cur = st->cur, nxt = cur ^ 1;
-  const int n_step = frames_for_chunk(chunk_len);
+  const int n_step = frames_for_chunk(m, chunk_len);
   const int C = m->cfg.num_classes;
 
   PcmSource src;
@@ -569,9 +586,9 @@ extern "C" int kws_stream_step(kws_stream* st, const int16_t* pcm, int32_t chunk
   src.body_len = chunk_len;
   src.body_dtype = KWS_PCM_I16;
   src.head = st->tail[cur];
-  src.ld_head = kTailCap;
+  src.ld_head = st->tail_cap;
   src.head_len = st->tail_len[cur];
-  const bool fused = frontend_can_fuse_pre(m, chunk_len, kTailCap);
+  const bool fused = frontend_can_fuse_pre(m, chunk_len, st->tail_cap);
   const bool tiled = mel_can_tile(m);
   cudaEvent_t tev[4] = {nullptr, nullptr, nullptr, nullptr};
   if (g_step_timing_on) {
@@ -588,8 +605,10 @@ extern "C" int kws_stream_step(kws_stream* st, const int16_t* pcm, int32_t chunk
     int rc = launch_frontend(m, src, S, n_step, st->mel, cs, &pre, tiled, st->nframes);
     if (rc != KWS_OK) return rc;
   } else {
-    stream_pre_kernel<<<static_cast<unsigned>(ceil_div(S * 32, 256)), 256, 0, cs>>>(
-        pcm, ld_pcm, chunk_len, S, st->tail[cur], st->tail_len[cur], pre, st->nframes, n_step);
+    const ChunkRule rule{m->cfg.fft_size, m->cfg.hop_size, st->tail_cap};
+    auto pre_kernel = frontend_is_default_frame(m) ? stream_pre_kernel<true> : stream_pre_kernel<false>;
+    pre_kernel<<<static_cast<unsigned>(ceil_div(S * 32, 256)), 256, 0, cs>>>(
+        pcm, ld_pcm, chunk_len, S, st->tail[cur], st->tail_len[cur], pre, st->nframes, n_step, rule);
     KWS_LAUNCH_OK("stream_pre_kernel");
   }
 

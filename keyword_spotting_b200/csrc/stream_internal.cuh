@@ -13,7 +13,8 @@ struct kws_stream {
   int fpad = 0;             // token slots per window entry (multiple of 16)
   kws::dec::Keyword kw;
   float* state = nullptr;           // [L, S, H]
-  int16_t* tail[2] = {nullptr, nullptr};     // [S, 400] ping-pong
+  int tail_cap = 400;       // carried-tail capacity per stream: tail_capacity(fft_size)
+  int16_t* tail[2] = {nullptr, nullptr};     // [S, tail_cap] ping-pong
   int32_t* tail_len[2] = {nullptr, nullptr}; // [S]
   int cur = 0;
   unsigned char* silence = nullptr; // [S] 1 = VAD said silence for the current chunk

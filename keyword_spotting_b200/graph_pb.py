@@ -10,7 +10,7 @@ numbers from TensorFlow's public .proto files) and maps the variable names of mo
     model/drnn/multi_rnn_cell/cell_{l}/gru_cell/gates/{kernel|weights}, .../{bias|biases}      (:236-243, get_cell)
     model/drnn/multi_rnn_cell/cell_{l}/gru_cell/candidate/{kernel|weights}, .../{bias|biases}
     model/weightsClasses, model/biasesClasses                                                  (:265-273)
-    the [201, n_mel] float Const feeding model/mel                                             (:139-148)
+    the [fft_size/2 + 1, n_mel] float Const feeding model/mel                                             (:139-148)
 
 and, for the octbit-rewritten graph, every ``OctbitMatMul`` node to (qint8 weight ``[out, in]``, ``scale``, ``bias``)
 (octbit/octbit_graph.py:527-536).
@@ -217,12 +217,14 @@ def constants(nodes: List[Node]) -> Dict[str, np.ndarray]:
 _CELL = re.compile(r"(?:^|/)cell_(\d+)/gru_cell/(gates|candidate)/(kernel|weights|bias|biases)$")
 
 
-def rnn_ctc_weights(nodes: List[Node], n_mel: Optional[int] = None, scope: str = "model"):
+def rnn_ctc_weights(nodes: List[Node], n_mel: Optional[int] = None, scope: str = "model", fft_size: int = 400):
     """Frozen rnn_ctc deployment graph -> keyword_spotting_b200.ModelWeights (and the implied sizes)."""
     from .rnn_ctc import ModelWeights
     consts = constants(nodes)
     layers: Dict[int, Dict[str, np.ndarray]] = {}
     fc_w = fc_b = mel = None
+    bins = fft_size // 2 + 1
+    other = []
     for name, val in consts.items():
         if scope and not name.startswith(scope + "/"):
             continue
@@ -238,8 +240,11 @@ def rnn_ctc_weights(nodes: List[Node], n_mel: Optional[int] = None, scope: str =
             fc_w = val.astype(np.float32)
         elif name.endswith("/biasesClasses"):
             fc_b = val.astype(np.float32)
-        elif val.dtype == np.float32 and val.ndim == 2 and val.shape[0] == 201 and (n_mel is None or val.shape[1] == n_mel):
-            mel = val
+        elif val.dtype == np.float32 and val.ndim == 2 and (n_mel is None or val.shape[1] == n_mel):
+            if val.shape[0] == bins:
+                mel = val
+            else:
+                other.append(tuple(val.shape))
     if not layers or fc_w is None or fc_b is None:
         raise GraphFormatError("not an rnn_ctc deployment graph: GRU / FC constants missing under scope %r" % scope)
     L = max(layers) + 1
@@ -248,7 +253,11 @@ def rnn_ctc_weights(nodes: List[Node], n_mel: Optional[int] = None, scope: str =
         if missing:
             raise GraphFormatError("layer %d lacks %s" % (l, sorted(missing)))
     if mel is None:
-        raise GraphFormatError("the [201, n_mel] mel basis Const was not found")
+        hint = ""
+        if other:
+            hint = " (float [rows, n_mel] Consts of other shapes: %s; a [fft_size/2 + 1, n_mel] basis needs that fft_size)" % (
+                ", ".join("[%d, %d]" % s for s in other))
+        raise GraphFormatError("the [%d, n_mel] mel basis Const of fft_size = %d was not found%s" % (bins, fft_size, hint))
     return ModelWeights.from_arrays(mel, [layers[l]["gates_kernel"] for l in range(L)],
                                     [layers[l]["gates_bias"] for l in range(L)],
                                     [layers[l]["candidate_kernel"] for l in range(L)],
@@ -298,7 +307,7 @@ def octbit_nodes(nodes: List[Node]) -> List[OctbitNode]:
     return out
 
 
-def rnn_ctc_octbit_weights(nodes: List[Node], n_mel: Optional[int] = None, scope: str = "model"):
+def rnn_ctc_octbit_weights(nodes: List[Node], n_mel: Optional[int] = None, scope: str = "model", fft_size: int = 400):
     """Octbit-rewritten rnn_ctc deployment graph (``graph_octbit.pb``, main.py:357-371) ->
     ``(ModelWeights, OctbitModelWeights)``.
 
@@ -331,4 +340,4 @@ def rnn_ctc_octbit_weights(nodes: List[Node], n_mel: Optional[int] = None, scope
             patched.append(n2)
         else:
             patched.append(n)
-    return rnn_ctc_weights(patched, n_mel=n_mel, scope=scope), ow
+    return rnn_ctc_weights(patched, n_mel=n_mel, scope=scope, fft_size=fft_size), ow

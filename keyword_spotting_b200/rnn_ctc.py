@@ -43,7 +43,7 @@ class ModelWeights:
     TF names (SURVEY.md 8f-3): ``model/drnn/multi_rnn_cell/cell_{l}/gru_cell/
     {gates,candidate}/{kernel,bias}``, ``model/weightsClasses``, ``model/biasesClasses``.
     """
-    mel_basis: np.ndarray                                   # [201, M]
+    mel_basis: np.ndarray                                   # [fft_size/2 + 1, M]
     gates_kernel: List[np.ndarray] = field(default_factory=list)   # [in+H, 2H]
     gates_bias: List[np.ndarray] = field(default_factory=list)     # [2H]
     cand_kernel: List[np.ndarray] = field(default_factory=list)    # [in+H, H]
@@ -58,11 +58,12 @@ class ModelWeights:
                    [f(a) for a in cand_kernel], [f(a) for a in cand_bias], f(fc_w), f(fc_b))
 
     @classmethod
-    def from_frozen_graph(cls, path_or_bytes, n_mel: Optional[int] = None):
+    def from_frozen_graph(cls, path_or_bytes, n_mel: Optional[int] = None, fft_size: int = 400):
         """Weights of a frozen deployment ``graph.pb`` (main.py:339-348), read without TensorFlow
-        (keyword_spotting_b200/graph_pb.py)."""
+        (keyword_spotting_b200/graph_pb.py).  ``fft_size``: the model's frame; its mel basis is
+        ``[fft_size/2 + 1, n_mel]``."""
         from . import graph_pb
-        return graph_pb.rnn_ctc_weights(graph_pb.load_graph(path_or_bytes), n_mel=n_mel)
+        return graph_pb.rnn_ctc_weights(graph_pb.load_graph(path_or_bytes), n_mel=n_mel, fft_size=fft_size)
 
     @classmethod
     def random_init(cls, config: Config, seed: int = 1234):
@@ -151,7 +152,9 @@ class DeployModel:
                  precision: str = "tc", frontend: Optional[str] = None):
         """``precision``: ``"tc"`` (default) = tcgen05 tensor cores, fp16 operands / fp32 accumulate and state;
         ``"fp32"`` = every product in fp32 on the CUDA cores (the accuracy baseline).
-        ``frontend``: ``"fft"`` (default) or ``"tc"`` (hop-block DFTs on tcgen05; int16 PCM) -- same results, same speed."""
+        ``frontend``: ``"fft"`` (default) or ``"tc"`` (hop-block DFTs on tcgen05; int16 PCM) -- same results, same speed.
+        Both are 400/160 kernels: a model of any other ``fft_size`` / ``hop_size`` runs the general DFT front end
+        (csrc/frontend_dft.cu) whatever ``frontend`` says."""
         self.config = config or Config()
         self.device = _tensors.require_cuda(device)
         self.weights = weights if weights is not None else ModelWeights.random_init(self.config)
@@ -196,7 +199,8 @@ class DeployModel:
         """The reference's deployable artefact ``graph_octbit.pb`` (main.py:357-371): float cell_0 + OctbitMatMul
         everywhere else, read without TensorFlow and run through the octbit kernels."""
         from . import graph_pb
-        weights, octw = graph_pb.rnn_ctc_octbit_weights(graph_pb.load_graph(path_or_bytes), n_mel=n_mel)
+        fft_size = config.fft_size if config is not None else Config.fft_size
+        weights, octw = graph_pb.rnn_ctc_octbit_weights(graph_pb.load_graph(path_or_bytes), n_mel=n_mel, fft_size=fft_size)
         cfg = config or Config(n_mel=weights.mel_basis.shape[1], num_layers=len(weights.gates_kernel))
         model = cls(cfg, weights, device=device, precision="fp32")
         model.set_octbit(octw)
