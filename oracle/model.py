@@ -203,6 +203,37 @@ def _split_product(x, W, od, dtype):
     return np.matmul(xh, Wh) + np.matmul(xl, Wh) + np.matmul(xh, Wl)
 
 
+# The tensor-core kernel's shared-memory plan for layer 0 (gru_tc.cu: gru_tc_smem_bytes, gru_tc_x_buffers,
+# gru_tc_can_split; api.cu: the split and fit decisions at model creation).  `cap` is the device's opt-in
+# shared-memory limit per block; TC_SMEM_OPTIN_B200 is the B200's (227 KB).
+TC_SMEM_OPTIN_B200 = 232448
+_TC_TILE_CHUNK = 2048          # one 8-column chunk of a 128-stream fp16 operand tile
+_TC_FC_OPERAND = 16 * HIDDEN * 2
+_TC_MAX_CLASSES = 8
+_TC_NUM_BARS = 11
+
+
+def tc_smem_bytes(kxw: int, last: bool, nbuf: int) -> int:
+    return (768 * (kxw + HIDDEN) + nbuf * (kxw // 8) * _TC_TILE_CHUNK + 4 * 384
+            + ((_TC_FC_OPERAND + 4 * (4 * 6 + _TC_MAX_CLASSES) * 128) if last else 0) + _TC_NUM_BARS * 8 + 16)
+
+
+def tc_x_buffers(kxw: int, last: bool, cap: int = TC_SMEM_OPTIN_B200) -> int:
+    """x buffers the kernel keeps for a layer with `kxw` operand columns: 2, 1, or 0 (does not fit)."""
+    for nbuf in (2, 1):
+        if tc_smem_bytes(kxw, last, nbuf) <= cap:
+            return nbuf
+    return 0
+
+
+def tc_layer0_plan(n_mel: int, num_layers: int, cap: int = TC_SMEM_OPTIN_B200) -> Tuple[bool, int]:
+    """(split, x buffers) of layer 0 on the tensor-core kernel; 0 buffers: the model runs the fp32 kernel."""
+    last = num_layers == 1
+    kx = (n_mel + 15) // 16 * 16
+    split = n_mel <= 64 and tc_x_buffers(2 * kx, last, cap) > 0
+    return split, tc_x_buffers(2 * kx if split else kx, last, cap)
+
+
 def gru_cell(x, h, gates_kernel, gates_bias, cand_kernel, cand_bias, dtype=np.float32, operand_dtype=None,
              split_x=False):
     """One TF GRUCell step.  NOTE reset gate is applied to h BEFORE the
@@ -250,13 +281,14 @@ def gru_forward(x: np.ndarray, state: np.ndarray, w: Weights,
     S, n, _ = x.shape
     h = [state[l].astype(dtype).copy() for l in range(w.num_layers)]
     out = np.zeros((S, n, w.hidden), dtype=dtype)
+    split0 = operand_dtype is not None and tc_layer0_plan(x.shape[2], w.num_layers)[0]
     for t in range(n):
         inp = x[:, t, :]
         live = None if seq_len is None else (t < np.asarray(seq_len))[:, None]
         for l in range(w.num_layers):
             new_h = gru_cell(inp, h[l], w.gates_kernel[l], w.gates_bias[l],
                              w.cand_kernel[l], w.cand_bias[l], dtype, operand_dtype,
-                             split_x=(operand_dtype is not None and l == 0 and inp.shape[1] <= 64))
+                             split_x=(split0 and l == 0))
             if live is not None:
                 new_h = np.where(live, new_h, h[l])
             h[l] = new_h
