@@ -463,10 +463,6 @@ int kws_debug_att_core_lens(const float* qkv, int64_t B, int32_t Tp, const int32
 int kws_debug_att_add_layernorm_lens(const float* a, const float* b, const float* gamma, const float* beta, int64_t B,
                                      int32_t Tp, const int32_t* lens, int32_t N, int in_smem, float* y, void* stream);
 
-/* Debug: enable/disable and read the phase timeline (SM clock ticks) of the first tile of CTA 0 of the last
- * tensor-core GRU launch; see csrc/gru_tc.cu.  host_out may be NULL (only set the switch).               */
-int kws_debug_tc_timeline(int enable, long long* host_out, int count);
-
 /* Debug / test (host only, needs no device): the front end's per-warp mel "quad" lists for a basis [201, n_mel]
  * (csrc/frontend.cu, build_mel_quads).  quads_out receives records of 8 ints {4 weights (float bits), magnitude row byte
  * offset, output band byte offset or -1, 0, 0}, 10 warps x the returned quads-per-warp; quads_out may be NULL.     */

@@ -41,11 +41,6 @@ def is_stale() -> bool:
 
 def build(force: bool = False, verbose: bool = False) -> str:
     """Compile every CUDA source into keyword_spotting_b200/libkws_b200.so."""
-    override = os.environ.get("KWS_B200_LIB")            # experiments: a library built elsewhere (same ABI)
-    if override and not force:
-        if not os.path.exists(override):
-            raise ImportError("KWS_B200_LIB=%s does not exist" % override)
-        return override
     if not force and not is_stale():
         return LIB_PATH
     nvcc = _nvcc()

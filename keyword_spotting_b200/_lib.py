@@ -151,7 +151,6 @@ _SIGNATURES = {
                                             c_void_p, c_void_p]),
     "kws_debug_att_add_layernorm_lens": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_int32,
                                                  c_int, c_void_p, c_void_p]),
-    "kws_debug_tc_timeline": (c_int, [c_int, c_void_p, c_int]),
     "kws_debug_step_timing": (c_int, [c_int, c_void_p, c_void_p]),
     "kws_debug_mel_quads": (c_int, [c_void_p, c_int, c_void_p, c_int]),
 }

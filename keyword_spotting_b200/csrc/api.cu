@@ -209,13 +209,6 @@ extern "C" int kws_model_set_frontend(kws_model* m, int frontend) {
 
 extern "C" int kws_model_get_frontend(const kws_model* m) { return m ? m->frontend : -1; }
 
-namespace kws {
-int launch_gru(kws_model* m, const GruArgs& a, cudaStream_t st) {
-  if (m->octbit) return launch_gru_octbit(m, a, st);
-  return model_uses_tc(m) ? launch_gru_tc(m, a, st) : launch_gru_fp32(m, a, st);
-}
-}  // namespace kws
-
 extern "C" int kws_num_frames(const kws_model* m, int64_t L) {
   const int fft = m ? m->cfg.fft_size : kFft, hop = m ? m->cfg.hop_size : kHop;
   // 1 + floor((L - fft) / hop) with floor toward -inf (utils/stft.py:60-61)
@@ -224,33 +217,40 @@ extern "C" int kws_num_frames(const kws_model* m, int64_t L) {
   return static_cast<int>(1 + q);
 }
 
+namespace kws {
+int grow_scratch(void** buf, size_t* cap, size_t bytes, const char* what) {
+  if (bytes <= *cap) return KWS_OK;
+  KWS_CUDA_OK(cudaDeviceSynchronize());      // another stream may still read the old buffer
+  cudaFree(*buf);
+  *buf = nullptr;
+  *cap = 0;
+  const cudaError_t e = cudaMalloc(buf, bytes);
+  if (e != cudaSuccess) {
+    *buf = nullptr;
+    return fail(KWS_ERR_ALLOC, "%s of %zu bytes: allocation failed: %s", what, bytes, cudaGetErrorString(e));
+  }
+  *cap = bytes;
+  return KWS_OK;
+}
+}  // namespace kws
+
 extern "C" int kws_model_reserve(kws_model* m, int64_t max_streams, int32_t max_frames) {
   KWS_REQUIRE(m != nullptr, "model is NULL");
   if (max_streams <= m->cap_streams && max_frames <= m->cap_frames) return KWS_OK;
   const int64_t S = max_streams > m->cap_streams ? max_streams : m->cap_streams;
   const int32_t n = max_frames > m->cap_frames ? max_frames : m->cap_frames;
   KWS_CUDA_OK(cudaSetDevice(m->device));
-  KWS_CUDA_OK(cudaDeviceSynchronize());      // nobody may still be using the old scratch
-  cudaFree(m->scratch_mel);
-  cudaFree(m->scratch_seq);
-  cudaFree(m->scratch_nfr);
-  m->scratch_mel = m->scratch_seq = nullptr;
-  m->scratch_nfr = nullptr;
   m->cap_streams = 0;
   m->cap_frames = 0;
-  const size_t mel_elems = mel_scratch_elems(S, n, m->cfg.n_mel);
-  const size_t seq_elems = seq_scratch_elems(S, n, m->cfg.num_layers);
-  cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&m->scratch_mel), sizeof(float) * (mel_elems ? mel_elems : 1));
-  if (e == cudaSuccess && m->cfg.num_layers > 1)
-    e = cudaMalloc(reinterpret_cast<void**>(&m->scratch_seq), sizeof(float) * (seq_elems ? seq_elems : 1));
-  if (e == cudaSuccess) e = cudaMalloc(reinterpret_cast<void**>(&m->scratch_nfr), sizeof(int32_t) * (S > 0 ? S : 1));
-  if (e != cudaSuccess) {
-    cudaFree(m->scratch_mel);
-    cudaFree(m->scratch_seq);
-    m->scratch_mel = m->scratch_seq = nullptr;
-    return fail(KWS_ERR_ALLOC, "scratch allocation for %lld streams x %d frames failed: %s",
-                static_cast<long long>(S), n, cudaGetErrorString(e));
-  }
+  int rc = grow_scratch(reinterpret_cast<void**>(&m->scratch_mel), &m->scratch_mel_bytes,
+                        sizeof(float) * mel_scratch_elems(S, n, m->cfg.n_mel), "mel scratch");
+  if (rc == KWS_OK)
+    rc = grow_scratch(reinterpret_cast<void**>(&m->scratch_seq), &m->scratch_seq_bytes,
+                      sizeof(float) * seq_scratch_elems(S, n, m->cfg.num_layers), "layer hand-off scratch");
+  if (rc == KWS_OK)
+    rc = grow_scratch(reinterpret_cast<void**>(&m->scratch_nfr), &m->scratch_nfr_bytes, sizeof(int32_t) * S,
+                      "frame count scratch");
+  if (rc != KWS_OK) return rc;
   m->cap_streams = S;
   m->cap_frames = n;
   return KWS_OK;

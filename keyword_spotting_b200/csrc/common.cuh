@@ -141,17 +141,18 @@ struct kws_model {
   float* fc_w = nullptr;          // [H, C]
   float* fc_b = nullptr;          // [C]
   std::vector<float> fc_w_host, fc_b_host;   // host copies (the tensor-core kernel takes them as kernel parameters)
-  // scratch owned by the model (grown by kws_model_reserve)
+  // scratch owned by the model (grown by kws_model_reserve for up to cap_streams x cap_frames)
   int64_t cap_streams = 0;
   int32_t cap_frames = 0;
   float* scratch_mel = nullptr;   // [S, n, M]
   float* scratch_seq = nullptr;   // layer hand-off [tiles, n, H, 64]
   int32_t* scratch_nfr = nullptr; // [S] frames per stream of a forward over streams of their own lengths
+  size_t scratch_mel_bytes = 0, scratch_seq_bytes = 0, scratch_nfr_bytes = 0;
   // the octbit-rewritten graph (kws_model_set_octbit): per layer gates / candidate, and the FC
   bool octbit = false;
   kws::OctbitMatrix oct_gates[kws::kMaxLayers], oct_cand[kws::kMaxLayers], oct_fc;
   float* oct_y_rows = nullptr;    // [S, n, H] last-layer outputs for the FC (non-stream forwards)
-  size_t oct_y_cap = 0;
+  size_t oct_y_bytes = 0;
   bool tc_fits = true;            // every layer fits the tensor-core recurrent kernel's shared memory (set at creation)
   void* tc_xt = nullptr;          // row-tiled fp16 copy of a caller's row-major x (kws_gru_forward on the tensor-core path)
   size_t tc_xt_bytes = 0;
@@ -267,12 +268,20 @@ inline size_t seq_scratch_elems(int64_t S, int32_t n, int num_layers) {
   if (num_layers < 2) return 0;
   return static_cast<size_t>(ceil_div(S, 128) * 2) * (n > 0 ? n : 1) * kHidden * 64 * (num_layers > 2 ? 2 : 1);
 }
-int launch_gru(kws_model* m, const GruArgs& a, cudaStream_t st);        // dispatches on m->precision
-int launch_gru_fp32(kws_model* m, const GruArgs& a, cudaStream_t st);   // gru.cu   (exact fp32 FFMA)
-int launch_gru_tc(kws_model* m, const GruArgs& a, cudaStream_t st);     // gru_tc.cu (tcgen05, fp16 operands)
-int launch_gru_octbit(kws_model* m, const GruArgs& a, cudaStream_t st); // gru_octbit.cu (the octbit-rewritten graph)
-int launch_gru_fp32_layer(kws_model* m, const GruArgs& a, int l, const float* x_tiled, float* y_tiled, float* y_rows,
-                          cudaStream_t st);                             // gru.cu: one fp32 layer without the FC
+// gru.cu: every recurrent forward.  A call without frames passes the state through and zeroes the streams flagged by
+// zero_state; otherwise the layers run on the tensor cores (model_uses_tc) or on the CUDA cores (fp32 and octbit).
+int launch_gru(kws_model* m, const GruArgs& a, cudaStream_t st);
+// gru_tc.cu: all layers of a call with frames, through the inter-layer hand-off buffer `hand_off` (L > 1)
+int launch_gru_tc(kws_model* m, const GruArgs& a, float* hand_off, cudaStream_t st);
+// gru_octbit.cu: octbit layer l (x_tiled / y_tiled in gru.cu's [tile64][t][unit][64] hand-off, y_rows [S, n, H] or
+// null), and the octbit graph's FC + softmax on the last layer's y_rows
+int launch_octbit_layer(kws_model* m, const GruArgs& a, int l, const float* x_tiled, float* y_tiled, float* y_rows,
+                        cudaStream_t st);
+int launch_octbit_fc(kws_model* m, const GruArgs& a, const float* y_rows, cudaStream_t st);
 void free_octbit(kws_model* m);
+// Model-owned scratch grows through this one rule: nothing when *cap >= bytes; otherwise synchronise the device (another
+// stream may still read the old buffer), free, allocate.  On failure the buffer is null, *cap is 0 and the call returns
+// KWS_ERR_ALLOC.
+int grow_scratch(void** buf, size_t* cap, size_t bytes, const char* what);
 
 }  // namespace kws

@@ -17,6 +17,8 @@
 // an 8-stream x 4-unit register tile for r, u and c of the SAME hidden units, so the
 // gate algebra needs no exchange.  This is the exact-fp32 (FFMA) path: it is the
 // accuracy baseline for the tensor-core kernel and the always-available back end.
+//
+// launch_gru at the end is the host driver of all three back ends (this kernel, gru_tc.cu and gru_octbit.cu).
 #include "common.cuh"
 
 namespace kws {
@@ -360,22 +362,26 @@ static int launch_layer_fp32(kws_model* m, const GruArgs& a, int l, const float*
   return KWS_OK;
 }
 
-int launch_gru_fp32_layer(kws_model* m, const GruArgs& a, int l, const float* x_tiled, float* y_tiled, float* y_rows,
-                          cudaStream_t st) {
-  return launch_layer_fp32(m, a, l, x_tiled, y_tiled, y_rows, false, st);
+// zero the carried state of the streams flagged by zero_state (a call without frames)
+__global__ void zero_flagged_state_kernel(float* state, long S, int layers, const unsigned char* flags) {
+  const long idx = blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x;
+  const long total = static_cast<long>(layers) * S * kH;
+  if (idx >= total) return;
+  const long s = (idx / kH) % S;
+  if (flags[s]) state[idx] = 0.0f;
 }
 
-int launch_gru_fp32(kws_model* m, const GruArgs& a, cudaStream_t st) {
+int launch_gru(kws_model* m, const GruArgs& a, cudaStream_t st) {
   if (a.S <= 0) return KWS_OK;
   const int L = m->cfg.num_layers;
-  const long ntiles = ceil_div(a.S, kTs);
   if (a.n <= 0) {
-    // no frames: the state is carried through unchanged (or zeroed where asked)
-    if (a.state_out != a.state_in || a.zero_state) {
-      // handled by the caller for the zero_state case; plain copy here
-      if (a.state_out != a.state_in)
-        KWS_CUDA_OK(cudaMemcpyAsync(a.state_out, a.state_in, sizeof(float) * L * a.S * kH,
-                                    cudaMemcpyDeviceToDevice, st));
+    if (a.state_out != a.state_in)
+      KWS_CUDA_OK(cudaMemcpyAsync(a.state_out, a.state_in, sizeof(float) * L * a.S * kH, cudaMemcpyDeviceToDevice, st));
+    if (a.zero_state) {
+      const long total = static_cast<long>(L) * a.S * kH;
+      zero_flagged_state_kernel<<<static_cast<unsigned>(ceil_div(total, 256)), 256, 0, st>>>(a.state_out, a.S, L,
+                                                                                              a.zero_state);
+      KWS_LAUNCH_OK("zero_flagged_state_kernel");
     }
     return KWS_OK;
   }
@@ -384,14 +390,31 @@ int launch_gru_fp32(kws_model* m, const GruArgs& a, cudaStream_t st) {
     if (rc != KWS_OK) return rc;
   }
   float* seq = a.seq_scratch ? a.seq_scratch : m->scratch_seq;
-  const long per_buf = ntiles * a.n * static_cast<long>(kH) * kTs;
+  if (model_uses_tc(m)) return launch_gru_tc(m, a, seq, st);
+
+  // CUDA cores.  The float graph fuses the FC into its last layer; the octbit graph's last layer writes y_rows for
+  // fc_octbit_softmax_kernel.  Layers the rewriter left in fp32 (cell_0) run the fp32 kernel in either graph.
+  float* y_rows = nullptr;
+  if (m->octbit) {
+    y_rows = a.y_rows_scratch;
+    if (!y_rows) {
+      const int rc = grow_scratch(reinterpret_cast<void**>(&m->oct_y_rows), &m->oct_y_bytes,
+                                  sizeof(float) * a.S * a.n * kH, "octbit FC input scratch");
+      if (rc != KWS_OK) return rc;
+      y_rows = m->oct_y_rows;
+    }
+  }
+  const long per_buf = ceil_div(a.S, kTs) * a.n * static_cast<long>(kH) * kTs;
   for (int l = 0; l < L; ++l) {
     const bool last = l == L - 1;
-    const int rc = launch_layer_fp32(m, a, l, l > 0 ? seq + ((l - 1) & 1) * per_buf : nullptr, last ? nullptr : seq + (l & 1) * per_buf, nullptr,
-                                     last, st);
+    const float* x_tiled = l == 0 ? nullptr : seq + ((l - 1) & 1) * per_buf;
+    float* y_tiled = last ? nullptr : seq + (l & 1) * per_buf;
+    float* yr = last ? y_rows : nullptr;
+    const int rc = m->oct_gates[l].wq ? launch_octbit_layer(m, a, l, x_tiled, y_tiled, yr, st)
+                                      : launch_layer_fp32(m, a, l, x_tiled, y_tiled, yr, last && !m->octbit, st);
     if (rc != KWS_OK) return rc;
   }
-  return KWS_OK;
+  return m->octbit ? launch_octbit_fc(m, a, y_rows, st) : KWS_OK;
 }
 
 }  // namespace kws

@@ -55,27 +55,6 @@ struct GruOctParams {
   const unsigned char* zero_state;
 };
 
-__device__ __forceinline__ void mma_u8s8_16832(int (&c)[4], const unsigned (&a)[4], unsigned b0, unsigned b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k32.row.col.s32.u8.s8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};\n"
-      : "+r"(c[0]), "+r"(c[1]), "+r"(c[2]), "+r"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-
-// The op's quantiser for ONE stream's row(s): min / max -> (bscale, offset, signedness)   (:90-124)
-__device__ __forceinline__ QuantParams quant_from_range(float mn, float mx) {
-  QuantParams p;
-  p.is_signed = mn < 0.0f;
-  if (p.is_signed) {
-    p.bscale = __fdiv_rn(fmaxf(-mn, mx), 127.0f);
-    p.offset = 127.0f;
-  } else {
-    p.bscale = __fdiv_rn(mx, 254.0f);
-    p.offset = 0.0f;
-  }
-  return p;
-}
-
 // Warp-level: ranges of the 16 rows of `af`, then their u8 images in `q`.  Lane = (row = lane / 2, half = lane % 2).
 __device__ __forceinline__ void quantise_rows(const float* af, unsigned char* q, float* bscale_out, int* signed_out, int lane) {
   const int row = lane >> 1, half = lane & 1;
@@ -131,7 +110,7 @@ __device__ __forceinline__ void oct_mma_chunk(int (&acc)[8][4], const OctMatDev&
       const signed char* wr = m.wq + static_cast<long>(n0 + 8 * j + g) * kOctK + k0 + 4 * t;
       const unsigned b0 = __ldg(reinterpret_cast<const unsigned*>(wr));
       const unsigned b1 = __ldg(reinterpret_cast<const unsigned*>(wr + 16));
-      mma_u8s8_16832(acc[j], a, b0, b1);
+      mma_u8s8(acc[j], a, b0, b1);
     }
   }
 }
@@ -353,21 +332,6 @@ fc_octbit_softmax_kernel(const FcOctParams p) {
   }
 }
 
-__global__ void __launch_bounds__(256)
-oct_find_candidates_kernel(const signed char* __restrict__ w, int B, int K, int* __restrict__ cand_count,
-                           unsigned short* __restrict__ cand) {
-  // one thread per output row: a deterministic, ordered list (the order does not matter for the sum)
-  const int n = blockIdx.x * blockDim.x + threadIdx.x;
-  if (n >= B) return;
-  int cnt = 0;
-  for (int kp = 0; kp < K / 2; ++kp) {
-    const int w0 = w[static_cast<long>(n) * K + 2 * kp], w1 = w[static_cast<long>(n) * K + 2 * kp + 1];
-    const bool same_sign = (w0 > 0 && w1 > 0) || (w0 < 0 && w1 < 0);
-    if (same_sign && abs(w0) + abs(w1) >= 129) cand[static_cast<long>(n) * (K / 2) + cnt++] = static_cast<unsigned short>(kp);
-  }
-  cand_count[n] = cnt;
-}
-
 static void free_oct(OctbitMatrix& o) {
   cudaFree(o.wq);
   cudaFree(o.obias);
@@ -384,7 +348,7 @@ void free_octbit(kws_model* m) {
   free_oct(m->oct_fc);
   cudaFree(m->oct_y_rows);
   m->oct_y_rows = nullptr;
-  m->oct_y_cap = 0;
+  m->oct_y_bytes = 0;
   m->octbit = false;
 }
 
@@ -400,8 +364,11 @@ static int upload_oct(OctbitMatrix* dst, const int8_t* wq, const float* obias, f
   KWS_CUDA_OK(cudaMemcpy(dst->obias, obias, sizeof(float) * B, cudaMemcpyHostToDevice));
   KWS_CUDA_OK(cudaMalloc(reinterpret_cast<void**>(&dst->cand_count), sizeof(int) * B));
   KWS_CUDA_OK(cudaMalloc(reinterpret_cast<void**>(&dst->cand), sizeof(unsigned short) * static_cast<size_t>(B) * (K / 2)));
-  oct_find_candidates_kernel<<<static_cast<unsigned>(ceil_div(B, 256)), 256>>>(dst->wq, B, K, dst->cand_count, dst->cand);
-  KWS_LAUNCH_OK("oct_find_candidates_kernel");
+  // the list order is the atomics' and differs from run to run; the correction is an integer sum over the list
+  KWS_CUDA_OK(cudaMemset(dst->cand_count, 0, sizeof(int) * B));
+  octbit_find_candidates_kernel<<<static_cast<unsigned>(ceil_div(static_cast<int64_t>(B) * (K / 2), 256)), 256>>>(
+      dst->wq, B, K, dst->cand_count, dst->cand);
+  KWS_LAUNCH_OK("octbit_find_candidates_kernel");
   KWS_CUDA_OK(cudaDeviceSynchronize());
   return KWS_OK;
 }
@@ -416,66 +383,32 @@ static OctMatDev dev_view(const OctbitMatrix& o) {
   return d;
 }
 
-// fp32 layers through gru.cu (one layer at a time), octbit layers through gru_octbit_layer_kernel, then the FC.
-int launch_gru_octbit(kws_model* m, const GruArgs& a, cudaStream_t st) {
-  if (a.S <= 0) return KWS_OK;
-  const int L = m->cfg.num_layers;
-  if (a.n <= 0) {
-    if (a.state_out != a.state_in)
-      KWS_CUDA_OK(cudaMemcpyAsync(a.state_out, a.state_in, sizeof(float) * L * a.S * kHidden, cudaMemcpyDeviceToDevice, st));
-    return KWS_OK;
-  }
-  if (!a.seq_scratch) {
-    const int rc = kws_model_reserve(m, a.S, a.n);
-    if (rc != KWS_OK) return rc;
-  }
-  float* seq = a.seq_scratch ? a.seq_scratch : m->scratch_seq;
-  float* y_rows = a.y_rows_scratch;
-  if (!y_rows) {
-    const size_t need = static_cast<size_t>(a.S) * a.n * kHidden;
-    if (m->oct_y_cap < need) {
-      KWS_CUDA_OK(cudaDeviceSynchronize());
-      cudaFree(m->oct_y_rows);
-      m->oct_y_rows = nullptr;
-      m->oct_y_cap = 0;
-      KWS_CUDA_OK(cudaMalloc(reinterpret_cast<void**>(&m->oct_y_rows), sizeof(float) * need));
-      m->oct_y_cap = need;
-    }
-    y_rows = m->oct_y_rows;
-  }
-  const long ntiles = ceil_div(a.S, kOctTile);
-  const long per_buf = ntiles * a.n * static_cast<long>(kHidden) * kOctTile;
-  for (int l = 0; l < L; ++l) {
-    const bool last = l == L - 1;
-    const float* x_tiled = l == 0 ? nullptr : seq + ((l - 1) & 1) * per_buf;
-    float* y_tiled = last ? nullptr : seq + (l & 1) * per_buf;
-    if (!m->oct_gates[l].wq) {
-      // a layer the rewriter left in fp32 (cell_0): the exact fp32 kernel, hand-off in the tiled layout
-      const int rc = launch_gru_fp32_layer(m, a, l, x_tiled, y_tiled, last ? y_rows : nullptr, st);
-      if (rc != KWS_OK) return rc;
-      continue;
-    }
-    GruOctParams p;
-    p.S = a.S;
-    p.n = a.n;
-    p.x_tiled = x_tiled;
-    p.y_tiled = y_tiled;
-    p.y_rows = last ? y_rows : nullptr;
-    p.g = dev_view(m->oct_gates[l]);
-    p.c = dev_view(m->oct_cand[l]);
-    p.bg = m->layer[l].gates_bias;
-    p.bc = m->layer[l].cand_bias;
-    p.h_in = a.state_in + static_cast<long>(l) * a.S * kHidden;
-    p.h_out = a.state_out + static_cast<long>(l) * a.S * kHidden;
-    p.seq_len = a.seq_len;
-    p.zero_state = a.zero_state;
-    const size_t smem = gru_octbit_smem_bytes();
-    KWS_CUDA_OK(cudaFuncSetAttribute(gru_octbit_layer_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    const long parts = ntiles * kOctPartsPerTile;
-    const long blocks = parts < 3L * sm_count() ? parts : 3L * sm_count();
-    gru_octbit_layer_kernel<<<static_cast<unsigned>(blocks), kOctThreads, smem, st>>>(p);
-    KWS_LAUNCH_OK("gru_octbit_layer_kernel");
-  }
+int launch_octbit_layer(kws_model* m, const GruArgs& a, int l, const float* x_tiled, float* y_tiled, float* y_rows,
+                        cudaStream_t st) {
+  GruOctParams p;
+  p.S = a.S;
+  p.n = a.n;
+  p.x_tiled = x_tiled;
+  p.y_tiled = y_tiled;
+  p.y_rows = y_rows;
+  p.g = dev_view(m->oct_gates[l]);
+  p.c = dev_view(m->oct_cand[l]);
+  p.bg = m->layer[l].gates_bias;
+  p.bc = m->layer[l].cand_bias;
+  p.h_in = a.state_in + static_cast<long>(l) * a.S * kHidden;
+  p.h_out = a.state_out + static_cast<long>(l) * a.S * kHidden;
+  p.seq_len = a.seq_len;
+  p.zero_state = a.zero_state;
+  const size_t smem = gru_octbit_smem_bytes();
+  KWS_CUDA_OK(cudaFuncSetAttribute(gru_octbit_layer_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  const long parts = ceil_div(a.S, kOctTile) * kOctPartsPerTile;
+  const long blocks = parts < 3L * sm_count() ? parts : 3L * sm_count();
+  gru_octbit_layer_kernel<<<static_cast<unsigned>(blocks), kOctThreads, smem, st>>>(p);
+  KWS_LAUNCH_OK("gru_octbit_layer_kernel");
+  return KWS_OK;
+}
+
+int launch_octbit_fc(kws_model* m, const GruArgs& a, const float* y_rows, cudaStream_t st) {
   FcOctParams f;
   f.S = a.S;
   f.n = a.n;

@@ -42,11 +42,6 @@
 // dropped lo*lo term is 2^-22 relative), i.e. at fp32-grade accuracy for +6 small MMAs per step: the front end
 // writes both halves of the split.  With it the deviation from the fp32 graph stays below 1e-3 (contract) on
 // probabilities and state; see DESIGN.md.
-//
-// Build-time experiment switches (tools/build_variant.sh <name> gru_tc.cu -D...; select the result with KWS_B200_LIB):
-//   KWS_ABL_NOX1, KWS_ABL_NOLO  ablations -- drop layer 1's x loads/stores or the lo halves of h' to TIME what they cost
-//                               (the results are wrong by construction);  KWS_L2_PREFETCH=<steps>  bulk L2 prefetch of layer
-//                               1's x that many steps ahead (measured: -1 %, off by default).
 #include <type_traits>
 #include <vector>
 
@@ -82,7 +77,6 @@ struct GruTcParams {
   int C;
   float* probs;                // [S, n, C]
   float* logits;               // [S, n, C] or null
-  int timeline;                // record g_tc_timeline (debug)
   // FC weights [128][8] + bias [8] by value (copied to shared memory by the last layer's CTAs)
   float fcw[kHidden * kTcMaxClasses];
   float fcb[kTcMaxClasses];
@@ -174,10 +168,6 @@ __device__ __forceinline__ void mbar_acquire(uint64_t* bar, uint32_t parity) {
   tc::mbar_wait(bar, parity);
   tc::fence_after_sync();
 }
-
-// Optional phase timeline of the first tile of CTA 0 (clock64 at each hand-over), for kws_debug_tc_timeline.
-__device__ long long g_tc_timeline[64 * 8];
-static int g_tc_timeline_on = 0;
 
 enum { kBarXF0 = 0, kBarXF1, kBarAX, kBarXD, kBarAH, kBarARH, kBarR, kBarU, kBarC, kBarF, kBarFR, kNumBars };
 
@@ -364,10 +354,6 @@ gru_tc_kernel(const GruTcParams p) {
           ++nf;
         }
         if (kXSmem && two && has_next) prefetch(ntile, nt1, buf ^ 1);      // the other buffer's last readers were the previous step's MMAs
-#ifdef KWS_L2_PREFETCH
-        if (!kXSmem && t + KWS_L2_PREFETCH < t_end && tc::elect_one())                // the gate threads' x loads of a later step: HBM -> L2 now
-          tc::bulk_prefetch_l2(p.x_f16 + (tile * p.n + t + KWS_L2_PREFETCH) * static_cast<long>(16 * kTcTile * 8), 16 * tc::kTileChunkBytes);
-#endif
         issue_x(buf, colDu, 1);                                            // u gate
         issue_h(colDu, 1);
         if (tc::elect_one()) tc::commit(&bars[kBarU]);
@@ -441,11 +427,7 @@ gru_tc_kernel(const GruTcParams p) {
       uint32_t xr[kXSmem ? 1 : 16];
       const uint32_t my_ax = tmem + lane_sel + colAx + 16 * ublk;
       auto load_x = [&](int t) {
-#ifdef KWS_ABL_NOX1
-        if (false) {
-#else
         if (!kXSmem) {
-#endif
           // chunk q of stream `row` sits at ((tile*n + t)*16 + q)*128 + row: a warp reads 512 contiguous bytes
           const uint4* src = reinterpret_cast<const uint4*>(p.x_f16) + ((tile * p.n + t) * 16 + 4 * ublk) * kTcTile + row;
 #pragma unroll
@@ -457,11 +439,7 @@ gru_tc_kernel(const GruTcParams p) {
         }
       };
       auto store_x = [&]() {
-#ifdef KWS_ABL_NOX1
-        if (false) {
-#else
         if (!kXSmem) {
-#endif
 #pragma unroll
           for (int q = 0; q < 4; ++q) {
             const uint32_t v[4] = {xr[kXSmem ? 0 : 4 * q], xr[kXSmem ? 0 : 4 * q + 1], xr[kXSmem ? 0 : 4 * q + 2],
@@ -561,12 +539,9 @@ gru_tc_kernel(const GruTcParams p) {
         const uint32_t par = it & 1;
         const bool more = t + 1 < t_end;
         if (!kXSmem && more) load_x(t + 1);                        // coalesced global loads in flight under the r gate
-        const bool tl = p.timeline && blockIdx.x == 0 && tid == 0 && tile == blockIdx.x && t < 64;
         // ---- r gate: keep fp16(r*h) in registers until the u-gate MMAs have finished reading A_h
         uint32_t rh[kTcUnits / 2];
-        if (tl) g_tc_timeline[t * 8 + 0] = clock64();
         mbar_acquire(&bars[kBarR], par);
-        if (tl) g_tc_timeline[t * 8 + 1] = clock64();
 #pragma unroll
         for (int c = 0; c < 2; ++c) {
           uint32_t v[16];
@@ -584,7 +559,6 @@ gru_tc_kernel(const GruTcParams p) {
             rh[j / 2 + 1] = tc::pack_half2(rh23.x, rh23.y);
           }
         }
-        if (tl) g_tc_timeline[t * 8 + 2] = clock64();
         const bool have_logits = kLast && t > p.t0;                // the previous step's, issued behind this step's r gate
         if (have_logits) {
           if (ublk == 0) read_logits(nf & 1, emit_prev);
@@ -598,7 +572,6 @@ gru_tc_kernel(const GruTcParams p) {
           tc::st8(my_ah + 8 * c, v);
         }
         tmem_publish(&bars[kBarARH]);
-        if (tl) g_tc_timeline[t * 8 + 3] = clock64();
         if (have_logits && ublk == 0) emit_probs(t - 1);
         // ---- u gate (beside the candidate MMAs): read once, kept in registers until the update
         float u[kTcUnits];
@@ -626,9 +599,7 @@ gru_tc_kernel(const GruTcParams p) {
           }
         }
         // ---- candidate and state update: only what the next step's MMAs wait for
-        if (tl) g_tc_timeline[t * 8 + 4] = clock64();
         mbar_acquire(&bars[kBarC], par);
-        if (tl) g_tc_timeline[t * 8 + 5] = clock64();
         const bool live = t < len;
         // (last layer: 8 units per pass -- with the lo halves of h' the 16-unit pass does not fit the 112 registers, and a
         // spilled loop scalar costs an L2 round trip here: the L1 is 28 KB next to 227 KB of shared memory)
@@ -662,11 +633,7 @@ gru_tc_kernel(const GruTcParams p) {
             const __half2 p01 = __floats2half2_rn(n01.x, n01.y), p23 = __floats2half2_rn(n23.x, n23.y);
             packed[i / 2] = *reinterpret_cast<const uint32_t*>(&p01);
             packed[i / 2 + 1] = *reinterpret_cast<const uint32_t*>(&p23);
-#ifdef KWS_ABL_NOLO
-            if (false) {
-#else
             if (kLast) {                                           // what the rounding lost: the FC's second operand
-#endif
               const float2 b01 = __half22float2(p01), b23 = __half22float2(p23);
               packed_lo[kLast ? i / 2 : 0] = tc::pack_half2(n01.x - b01.x, n01.y - b01.y);
               packed_lo[kLast ? i / 2 + 1 : 0] = tc::pack_half2(n23.x - b23.x, n23.y - b23.y);
@@ -686,7 +653,6 @@ gru_tc_kernel(const GruTcParams p) {
           }
         }
         if (kLast || more) tmem_publish(&bars[kBarAH]);            // releases the next step's r/u MMAs (last layer: and this step's FC)
-        if (tl) g_tc_timeline[t * 8 + 6] = clock64();
         // ---- outputs of this step, in the shadow of the next step's r-gate MMAs.  dynamic_rnn: zero output past the length
         const bool emit = all_live || live;
         if (!kLast) {
@@ -714,7 +680,6 @@ gru_tc_kernel(const GruTcParams p) {
         }
         ++nf;
       }
-      if (p.timeline && blockIdx.x == 0 && tid == 0 && tile == blockIdx.x) g_tc_timeline[7] = clock64();
       if (ok) {
         float4* dst = reinterpret_cast<float4*>(p.h_out + s * kHidden + u0);
 #pragma unroll
@@ -814,39 +779,19 @@ tc_pack_x_kernel(const float* __restrict__ x, long S, int n, int in_dim, int nc,
   }
 }
 
-int launch_gru_tc(kws_model* m, const GruArgs& a, cudaStream_t st) {
-  if (a.S <= 0) return KWS_OK;
-  if (m->cfg.num_classes > kTcMaxClasses)
-    return fail(KWS_ERR_UNSUPPORTED, "the tensor-core recurrent kernel keeps %d classes, the model has %d", kTcMaxClasses,
-                m->cfg.num_classes);
+int launch_gru_tc(kws_model* m, const GruArgs& a, float* hand_off, cudaStream_t st) {
   const int L = m->cfg.num_layers;
-  if (a.n <= 0) {
-    if (a.state_out != a.state_in)
-      KWS_CUDA_OK(cudaMemcpyAsync(a.state_out, a.state_in, sizeof(float) * L * a.S * kHidden, cudaMemcpyDeviceToDevice, st));
-    return KWS_OK;
-  }
-  if (L > 1 && !a.seq_scratch) {
-    const int rc = kws_model_reserve(m, a.S, a.n);
-    if (rc != KWS_OK) return rc;
-  }
   const long ntiles = ceil_div(a.S, kTcTile);
   const size_t per_buf = static_cast<size_t>(ntiles) * kTcTile * a.n * kHidden;     // halves (whole tiles)
-  __half* seq = reinterpret_cast<__half*>(a.seq_scratch ? a.seq_scratch : m->scratch_seq);
+  __half* seq = reinterpret_cast<__half*>(hand_off);
   // layer 0's operand: written by the front end (x_tiled), or packed here from the caller's row-major fp32 x
   const unsigned char* x0 = reinterpret_cast<const unsigned char*>(a.x);
   if (!a.x_tiled) {
     const int nc = m->layer[0].tc_kx / 8;
     const bool split = m->layer[0].tc_kxw != m->layer[0].tc_kx;
     const size_t need = static_cast<size_t>(ntiles) * a.n * (m->layer[0].tc_kxw / 8) * tc::kTileChunkBytes;
-    if (need > m->tc_xt_bytes) {
-      KWS_CUDA_OK(cudaStreamSynchronize(st));                          // the old buffer may still be read
-      cudaFree(m->tc_xt);
-      m->tc_xt = nullptr;
-      m->tc_xt_bytes = 0;
-      if (cudaMalloc(&m->tc_xt, need) != cudaSuccess)
-        return fail(KWS_ERR_ALLOC, "x operand scratch of %zu bytes: allocation failed", need);
-      m->tc_xt_bytes = need;
-    }
+    const int rc = grow_scratch(&m->tc_xt, &m->tc_xt_bytes, need, "x operand scratch");
+    if (rc != KWS_OK) return rc;
     const long total = ntiles * a.n * nc * kTcTile;
     const long blocks = std::min<long>(ceil_div(total, 256), static_cast<long>(sm_count()) * 16);
     tc_pack_x_kernel<<<static_cast<unsigned>(blocks), 256, 0, st>>>(a.x, a.S, a.n, m->layer[0].in_dim, nc, split ? 1 : 0,
@@ -880,7 +825,6 @@ int launch_gru_tc(kws_model* m, const GruArgs& a, cudaStream_t st) {
     p.C = m->cfg.num_classes;
     p.probs = a.probs;
     p.logits = a.logits;
-    p.timeline = (g_tc_timeline_on == 1 || g_tc_timeline_on == 2 + l) ? 1 : 0;      // 1: every layer (the last one stays), 2 + l: layer l only
     for (int j = 0; j < kHidden; ++j)
       for (int c = 0; c < kTcMaxClasses; ++c) p.fcw[j * kTcMaxClasses + c] = c < m->cfg.num_classes ? m->fc_w_host[j * m->cfg.num_classes + c] : 0.0f;
     for (int c = 0; c < kTcMaxClasses; ++c) p.fcb[c] = c < m->cfg.num_classes ? m->fc_b_host[c] : 0.0f;
@@ -906,7 +850,7 @@ int launch_gru_tc(kws_model* m, const GruArgs& a, cudaStream_t st) {
   // layers are pipelined in time chunks on two streams -- layer 1 runs chunk c while layer 0 runs chunk c + 1 -- so
   // twice as many SMs work.  The recurrence itself is sequential; large batches fill the GPU without this.
   constexpr int kChunk = 64;                                   // multiple of 4: the batched probability stores stay aligned
-  const bool pipelined = L == 2 && 2 * ntiles <= sm_count() && a.n >= 2 * kChunk && !g_tc_timeline_on;
+  const bool pipelined = L == 2 && 2 * ntiles <= sm_count() && a.n >= 2 * kChunk;
   if (!pipelined) {
     for (int l = 0; l < L; ++l) {
       const int rc = launch_layer(l, 0, a.n, true, st);
@@ -937,17 +881,3 @@ int launch_gru_tc(kws_model* m, const GruArgs& a, cudaStream_t st) {
 }
 
 }  // namespace kws
-
-// Debug: phase timeline (SM clock ticks) of the first tile of CTA 0 of the LAST tensor-core GRU launch:
-// per step t, [t*8 + k] = clock at {0 wait R, 1 got R, 2 r done, 3 r*h published, 4 u done, 5 got C, 6 h' published};
-// slot [7] = end of the tile.
-extern "C" int kws_debug_tc_timeline(int enable, long long* host_out, int count) {
-  using namespace kws;
-  clear_error();
-  g_tc_timeline_on = enable;
-  if (host_out && count > 0) {
-    if (count > 64 * 8) count = 64 * 8;
-    KWS_CUDA_OK(cudaMemcpyFromSymbol(host_out, g_tc_timeline, sizeof(long long) * count));
-  }
-  return KWS_OK;
-}

@@ -121,7 +121,6 @@ octbit_gemm_exact_kernel(const unsigned char* __restrict__ q, const signed char*
 }
 
 // ---------------------------------------------------------------- tensor-core back end
-// Saturation candidates: pairs of one weight row that can overflow int16 for some q.
 __global__ void __launch_bounds__(256)
 octbit_find_candidates_kernel(const signed char* __restrict__ w, int B, int K,
                               int* __restrict__ cand_count, unsigned short* __restrict__ cand) {
@@ -139,14 +138,6 @@ octbit_find_candidates_kernel(const signed char* __restrict__ w, int B, int K,
       cand[static_cast<long>(n) * half + slot] = static_cast<unsigned short>(kp);
     }
   }
-}
-
-__device__ __forceinline__ void mma_u8s8(int (&c)[4], const unsigned (&a)[4], unsigned b0, unsigned b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k32.row.col.s32.u8.s8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
-      "{%0,%1,%2,%3};\n"
-      : "+r"(c[0]), "+r"(c[1]), "+r"(c[2]), "+r"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
 
 __device__ __forceinline__ int sat_correction(const unsigned char* __restrict__ qrow,

@@ -27,20 +27,21 @@ struct QuantParams {
   int is_signed;
 };
 
-__device__ __forceinline__ QuantParams quant_params(const OctbitHeader* h) {
-  const float mn = dec_float(h->enc_min);
-  const float mx = dec_float(h->enc_max);
+// the quantiser of a tensor whose elements span [mn, mx]   (:90-124)
+__device__ __forceinline__ QuantParams quant_from_range(float mn, float mx) {
   QuantParams p;
   p.is_signed = mn < 0.0f;
   if (p.is_signed) {
-    const float m = fmaxf(-mn, mx);
-    p.bscale = __fdiv_rn(m, 127.0f);
+    p.bscale = __fdiv_rn(fmaxf(-mn, mx), 127.0f);
     p.offset = 127.0f;
   } else {
     p.bscale = __fdiv_rn(mx, 254.0f);
     p.offset = 0.0f;
   }
   return p;
+}
+__device__ __forceinline__ QuantParams quant_params(const OctbitHeader* h) {
+  return quant_from_range(dec_float(h->enc_min), dec_float(h->enc_max));
 }
 
 __device__ __forceinline__ unsigned quant_one(float x, const QuantParams& p) {
@@ -62,6 +63,19 @@ __device__ __forceinline__ float octbit_epilogue(int l0, int l1, int l2, int l3,
   return __fmul_rn(o, scale);                       // *= scale                     (:179)
 }
 
+__device__ __forceinline__ void mma_u8s8(int (&c)[4], const unsigned (&a)[4], unsigned b0, unsigned b1) {
+  asm volatile(
+      "mma.sync.aligned.m16n8k32.row.col.s32.u8.s8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
+      "{%0,%1,%2,%3};\n"
+      : "+r"(c[0]), "+r"(c[1]), "+r"(c[2]), "+r"(c[3])
+      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
+
+// Saturation candidates (octbit.cu): the pairs of weight row n that can overflow int16 for some u8 row, appended to
+// cand[n * K/2 ..] in any order; cand_count[n] counts them and must be zero before the launch.
+__global__ void __launch_bounds__(256)
+octbit_find_candidates_kernel(const signed char* __restrict__ w, int B, int K, int* __restrict__ cand_count,
+                              unsigned short* __restrict__ cand);
 
 // tensor-core (tcgen05 kind::i8) back end with the quantiser fused in, octbit_tc.cu
 bool octbit_tc_supported(int64_t A, int64_t B, int64_t K);

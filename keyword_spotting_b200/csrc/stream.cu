@@ -166,15 +166,6 @@ stream_labels_kernel(long S, int W, int fpad, dec::Keyword kw, const signed char
   if (counts) counts[s] = sink.count();
 }
 
-// zero the carried state of silent streams when a chunk produces no frame at all
-__global__ void zero_silent_state_kernel(float* state, long S, int layers, const unsigned char* silence) {
-  const long idx = blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x;
-  const long total = static_cast<long>(layers) * S * kHidden;
-  if (idx >= total) return;
-  const long s = (idx / kHidden) % S;
-  if (silence[s]) state[idx] = 0.0f;
-}
-
 // ---- per-stream records (layout in include/kws_b200.h).  Every section starts and ends on a 16-byte boundary, so
 // both kernels move whole 16-byte pieces: one warp per record, lane-strided over its pieces.
 constexpr uint32_t kRecMagic = 0x5253574bu;   // "KWSR" as little-endian bytes
@@ -612,34 +603,27 @@ extern "C" int kws_stream_step(kws_stream* st, const int16_t* pcm, int32_t chunk
     KWS_LAUNCH_OK("stream_pre_kernel");
   }
 
-  if (n_step > 0) {
-    if (!fused) {
-      int rc = launch_frontend(m, src, S, n_step, st->mel, cs, nullptr, tiled);
-      if (rc != KWS_OK) return rc;
-    }
-    if (tev[1]) KWS_CUDA_OK(cudaEventRecord(tev[1], cs));
-    int rc = KWS_OK;
-    GruArgs a;
-    a.x = st->mel;
-    a.x_tiled = tiled;
-    a.seq_scratch = st->seq;
-    a.y_rows_scratch = st->y_rows;
-    a.S = S;
-    a.n = n_step;
-    a.seq_len = st->nframes;
-    a.zero_state = st->silence;
-    a.state_in = st->state;
-    a.state_out = st->state;
-    a.probs = st->probs;
-    a.logits = nullptr;
-    rc = launch_gru(m, a, cs);
+  if (n_step > 0 && !fused) {
+    int rc = launch_frontend(m, src, S, n_step, st->mel, cs, nullptr, tiled);
     if (rc != KWS_OK) return rc;
-  } else {
-    const long total = static_cast<long>(m->cfg.num_layers) * S * kHidden;
-    zero_silent_state_kernel<<<static_cast<unsigned>(ceil_div(total, 256)), 256, 0, cs>>>(
-        st->state, S, m->cfg.num_layers, st->silence);
-    KWS_LAUNCH_OK("zero_silent_state_kernel");
   }
+  if (tev[1]) KWS_CUDA_OK(cudaEventRecord(tev[1], cs));
+  // silent streams restart from a zero state; a chunk without frames does only that
+  GruArgs a;
+  a.x = st->mel;
+  a.x_tiled = tiled;
+  a.seq_scratch = st->seq;
+  a.y_rows_scratch = st->y_rows;
+  a.S = S;
+  a.n = n_step;
+  a.seq_len = st->nframes;
+  a.zero_state = st->silence;
+  a.state_in = st->state;
+  a.state_out = st->state;
+  a.probs = st->probs;
+  a.logits = nullptr;
+  int rc = launch_gru(m, a, cs);
+  if (rc != KWS_OK) return rc;
   if (tev[2]) KWS_CUDA_OK(cudaEventRecord(tev[2], cs));
   stream_post_kernel<<<static_cast<unsigned>(ceil_div(S, 128)), 128, 0, cs>>>(
       st->probs, n_step, C, S, st->cfg.window_chunks, st->fpad, st->cfg.decode_thres, st->kw, st->silence,

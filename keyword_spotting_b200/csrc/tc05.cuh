@@ -81,11 +81,6 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gsrc, uint3
                : "memory");
 }
 
-// `bytes` contiguous bytes of global memory -> L2 (no destination, no completion): one instruction per tile-step
-__device__ __forceinline__ void bulk_prefetch_l2(const void* gsrc, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(gsrc), "r"(bytes) : "memory");
-}
-
 // ---- descriptors
 // shared-memory matrix descriptor, K-major, SWIZZLE_NONE (cute::UMMA::SmemDescriptor)
 __device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {

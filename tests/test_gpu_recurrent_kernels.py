@@ -345,6 +345,22 @@ def test_octbit_second_pass_per_cta():
     _batch_independence(dm, 3 * 148 * 32 + 1500, 3, seed=6)
 
 
+# ================================================================ calls without frames
+@pytest.mark.parametrize("backend", ["tc", "fp32", "octbit"])
+def test_zero_frame_call_passes_the_state_through(backend):
+    """kws_gru_forward with n = 0 and state_out != state_in: state_out is state_in, bit for bit."""
+    L, M = 2, 40
+    ow = _weights(L, M, 6, seed=23)
+    dm = _model(ow, L, M, 6, "tc" if backend == "tc" else "fp32")
+    if backend == "octbit":
+        dm.set_octbit(_octw(dm, [1], True))
+    rng = np.random.default_rng(24)
+    for S in (1, 65, 300):
+        st = _states(rng, L, S)
+        _, so, _ = _call(dm, np.zeros((S, 0, M), np.float32), st)
+        assert np.array_equal(so.view(np.uint32), st.view(np.uint32)), S
+
+
 def test_report_worst_ratios(capsys):
     """Worst error / bound of every back end and step quantity seen by the tests above (run after them)."""
     with capsys.disabled():
